@@ -10,6 +10,7 @@ no collective on the hot path) and the finished samples are all-gathered over NC
 (configs[3] uses the same code with --games-per-gpu 32768).
 
   python bench.py [--gpus N] [--steps K] [--warmup W]          engine arm
+  python bench.py ... --dump-outputs DIR                       + the last timed step's samples as .npy
   python bench.py --impl reference ...                         reference CPU arm
 Under torchrun (N > 1) every rank runs; rank 0 prints the single JSON line.
 """
@@ -37,6 +38,7 @@ FLOP_PER_EVAL = 253400.0         # SURVEY.md 8(d): unpadded dense FLOPs per leaf
 # 1.36 MB for k_mlp_tc
 NCU_DRAM_BYTES_PER_DENSE_LAUNCH = {"game_step": 149.888000e6 + 59.357440e6, "network": 1.356032e6 + 0.000256e6}
 NCU_SOURCE = "profiles/r02_ncu_k_iterate_6ctas.txt, k_iterate<1, 32, 6>"
+DUMP_BUDGET_BYTES = 64 * 10**6
 
 
 def peaks():
@@ -287,6 +289,47 @@ def samples_digest(tr):
     return h.hexdigest()
 
 
+def dump_outputs(out_dir, tr, dist=None):
+    """Write what a caller of the timed path receives after its last step: Trainer.write_samples()
+    (game states [rows, 70], value labels [rows], move probabilities [rows, 96]; 8 symmetry rows per
+    move) as float32, and the step's work counters (simulations, moves, leaf evaluations) as float64.
+    When the rows exceed the 64 MB budget, a fixed seeded sample of them is written, in row order,
+    with their indices in sample_rows.npy (float64), so that two builds can be compared row by row.
+    With several GPUs each rank holds the rows of its contiguous shard of the games: rows are numbered
+    in global game order (rank 0's first), the sample is drawn over all of them and rank 0 gathers and
+    writes it, so the files are those of one trainer running every game. Returns None on other ranks."""
+    gs, ev, pr = tr.write_samples()
+    c = tr.counters()
+    mine = np.array([gs.shape[0], c["simulations"], c["moves"], c["leaf_evals"]], np.int64)
+    rank, world = (0, 1) if dist is None else (dist.get_rank(), dist.get_world_size())
+    every = [mine]
+    if dist is not None:
+        every = [None] * world
+        dist.all_gather_object(every, mine)
+    every = np.stack(every)
+    first, rows = int(every[:rank, 0].sum()), int(every[:, 0].sum())
+    row_bytes = 4 * (gs.shape[1] + 1 + pr.shape[1]) + 8
+    keep = min(rows, (DUMP_BUDGET_BYTES - (1 << 16)) // row_bytes)
+    idx = np.arange(rows) if keep == rows else np.sort(np.random.default_rng(0).choice(rows, keep, replace=False))
+    loc = idx[(idx >= first) & (idx < first + gs.shape[0])] - first
+    parts = [(gs[loc], ev[loc], pr[loc])]
+    if dist is not None:
+        gathered = [None] * world if rank == 0 else None
+        dist.gather_object(parts[0], gathered, dst=0)
+        parts = gathered
+    if rank != 0:
+        return None
+    arrays = {"game_states": np.concatenate([p[0] for p in parts]),
+              "eval_samples": np.concatenate([p[1] for p in parts]),
+              "prob_samples": np.concatenate([p[2] for p in parts]),
+              "sample_rows": idx.astype(np.float64),
+              "counters": every[:, 1:].sum(0).astype(np.float64)}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    return {"dir": out_dir, "rows": rows, "rows_written": int(keep), "files": sorted(arrays)}
+
+
 def run_engine_arm(args, rank, world, local_rank):
     import torch
     import corintho_ai_b200 as cb
@@ -366,6 +409,7 @@ def run_engine_arm(args, rank, world, local_rank):
     launches = L.cb200_launch_count() - launches0
     phase_ms = tr.phase_times()  # of the timed (un-profiled) pass
     digest_timed = samples_digest(tr)
+    dumped = dump_outputs(args.dump_outputs, tr, dist) if args.dump_outputs else None
 
     # ---- (2) the SAME steps on the SAME schedule (stream groups, parking, persistent tail) with a
     # CUDA-event pair around every kernel launch, recorded on the stream the kernel is launched on:
@@ -540,6 +584,8 @@ def run_engine_arm(args, rank, world, local_rank):
         "cpu_baseline": cpu,
         "clocks": clocks,
     }
+    if dumped is not None:
+        line["dumped_outputs"] = dumped
     print(json.dumps(line), flush=True)
     if dist is not None:
         dist.destroy_process_group()
@@ -620,7 +666,14 @@ def main():
     ap.add_argument("--precision", default=os.environ.get("CB200_PRECISION", "bf16"), choices=["bf16", "fp32"])
     ap.add_argument("--ref-games", type=int, default=256, help="games in one CPU-reference sample")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the samples of the last timed step, of all ranks, as DIR/<name>.npy "
+                         "(engine arm, at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "engine":
+        ap.error("--dump-outputs writes the engine's outputs: it needs --impl engine")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

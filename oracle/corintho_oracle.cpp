@@ -1060,6 +1060,38 @@ void orc_game_step_batch(int64_t n, const uint64_t *states, const uint32_t *rnd,
   }
 }
 
+// Reachable states from uniformly random legal play-outs, the generator of ref_gen_states
+// (ref_harness.cpp) restated on the oracle's rules: every position of every play-out (start and
+// terminal positions included) is emitted until n states exist. Returns the number of play-outs.
+int64_t orc_gen_states(uint64_t seed, int64_t n, uint64_t *out) {
+  uint64_t s = seed;
+  int64_t count = 0, games = 0;
+  while (count < n) {
+    State g = start_state();
+    ++games;
+    for (;;) {
+      out[2 * count] = g.w0, out[2 * count + 1] = g.w1;
+      if (++count >= n) break;
+      Mask m;
+      legal_moves(g, m);
+      int nl = m.count();
+      if (nl == 0) break;
+      uint64_t z = (s += 0x9E3779B97F4A7C15ull);  // splitmix64
+      z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ull;
+      z = (z ^ (z >> 27)) * 0x94D049BB133111EBull;
+      int k = (int)((z ^ (z >> 31)) % (uint64_t)nl);
+      int chosen = 0;
+      for (int mv = 0; mv < kNumMoves; ++mv)
+        if (m.get(mv) && k-- == 0) {
+          chosen = mv;
+          break;
+        }
+      g = do_move(g, chosen);
+    }
+  }
+  return games;
+}
+
 // ---- Trainer (trainer.cpp:18-256) --------------------------------------------------------
 // Shard of a larger run (the engine's multi-GPU partitioning, not in the reference): global games
 // [first_game, first_game + num_games) of the seed stream of mt19937(seed), parity = global index

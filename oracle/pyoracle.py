@@ -63,6 +63,7 @@ class _Lib:
         self._t_wsamp = fn("trainer_write_samples", None, [C.c_void_p, _f32p, _f32p, _f32p])
         self._t_score = fn("trainer_score", C.c_float, [C.c_void_p])
         self._t_mate = fn("trainer_avg_mate_length", C.c_float, [C.c_void_p])
+        self._gen = fn("gen_states", C.c_int64, [C.c_uint64, C.c_int64, _u64p])
 
     # ---- tables
     def line_breaker(self, idx):
@@ -97,6 +98,12 @@ class _Lib:
     def encode(self, st):
         out = np.zeros(70, np.float32)
         self._encode(np.ascontiguousarray(st, np.uint64), out)
+        return out
+
+    def gen_states(self, seed, n):
+        """n reachable states: every position of uniformly random legal play-outs (splitmix64)."""
+        out = np.zeros((n, 2), np.uint64)
+        self._gen(seed, n, out)
         return out
 
     def step_batch(self, states, rnd, want_enc=True, threads=1):
@@ -255,15 +262,6 @@ class _Tourney:
 class RefLib(_Lib):
     def __init__(self):
         super().__init__(REF_SO, "ref_")
-        f = self.lib.ref_gen_states
-        f.restype = C.c_int64
-        f.argtypes = [C.c_uint64, C.c_int64, _u64p]
-        self._gen = f
-
-    def gen_states(self, seed, n):
-        out = np.zeros((n, 2), np.uint64)
-        self._gen(seed, n, out)
-        return out
 
     def space_symmetry(self, k, j):
         return self.lib.ref_space_symmetry(k, j)

@@ -29,5 +29,5 @@ def oracle():
 def ref():
     from oracle.pyoracle import RefLib, have_ref
     if not have_ref():
-        pytest.skip("oracle/_ref not built (reference tree absent and no prebuilt library)")
+        pytest.skip("oracle/_ref not built: set CORINTHO_AI_REFERENCE to a checkout of the original project")
     return RefLib()

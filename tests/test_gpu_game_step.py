@@ -1,5 +1,8 @@
 """K1 game-logic kernel through the C ABI vs golden vectors (from the compiled reference), vs
-the oracle at 1M states, and size-independent properties at the BASELINE configs[1] size."""
+the oracle at 1M states, and size-independent properties at the BASELINE configs[1] size.
+The large tests take their positions from the oracle's generator, the same code they compare
+with; the golden vectors (test_game_step_matches_golden, and the generator pinned to the
+reference's play-outs in test_oracle_rules.py) keep both tied to the reference."""
 import os
 
 import numpy as np
@@ -52,7 +55,7 @@ def test_game_step_ragged_sizes_without_encoding(oracle, n):
                          ids=["paired", "paired-one-wave", "paired-branchy-finish", "paired-branchy-finish-prefetch",
                               "paired-cta-queue", "paired-7-ctas", "paired-prefetch-6-ctas", "paired-joint-finish-no-prefetch",
                               "split", "select-only"])
-def test_game_step_kernel_forms_vs_oracle(oracle, ref, monkeypatch, env):
+def test_game_step_kernel_forms_vs_oracle(oracle, monkeypatch, env):
     """Every form of the game-logic kernel (paired with a queue per warp, prefetch and the joint
     branch-free finish = default; without either; with a queue per CTA; register-capped builds;
     split; select-only) and the default with a single
@@ -63,17 +66,17 @@ def test_game_step_kernel_forms_vs_oracle(oracle, ref, monkeypatch, env):
     for k, v in env.items():
         monkeypatch.setenv(k, v)
     n = 1 << 18
-    states = ref.gen_states(4711, n)
+    states = oracle.gen_states(4711, n)
     mf, nx, _ = cb.game_step(cb.planes_from_reference_order(states), 5)
     masks, flags, nxt, _ = oracle.step_batch(states, step_rnd(5, n), want_enc=False, threads=8)
     assert (mf[:, :3] == masks).all() and (mf[:, 3] == flags).all()
     assert (cb.reference_order_from_planes(nx) == nxt).all()
 
 
-def test_game_step_1m_states_vs_oracle(oracle, ref):
+def test_game_step_1m_states_vs_oracle(oracle):
     """BASELINE.json configs[1] size: 1M reachable states, bit-exact against the oracle."""
     n = 1 << 20
-    states = ref.gen_states(20261018, n)
+    states = oracle.gen_states(20261018, n)
     mf, nx, _ = cb.game_step(cb.planes_from_reference_order(states), 77)
     masks, flags, nxt, _ = oracle.step_batch(states, step_rnd(77, n), want_enc=False, threads=8)
     assert (mf[:, :3] == masks).all() and (mf[:, 3] == flags).all()

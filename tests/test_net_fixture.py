@@ -8,6 +8,7 @@ import os
 import numpy as np
 
 from netref import forward_folded
+from util import NO_REFERENCE, reference_file
 
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
@@ -41,10 +42,10 @@ def test_network_restatement_and_importer_match_the_hand_evaluated_graph():
 
 
 def test_importer_reproduces_the_committed_weights():
-    src = "/root/reference/corintho_ai/docker/tflite_model.tflite"
-    if not os.path.exists(src):
+    src = reference_file("corintho_ai/docker/tflite_model.tflite")
+    if src is None:
         import pytest
-        pytest.skip("reference tree not present")
+        pytest.skip(NO_REFERENCE)
     from corintho_ai_b200.tflite_import import load_tflite_weights
     flat = np.load(os.path.join(GOLD, "trained_net.npz"))["flat"]
     assert load_tflite_weights(src).tobytes() == flat.tobytes()

@@ -98,6 +98,13 @@ def test_oracle_matches_golden_rules(oracle):
     assert ((fl & 3) == 1).sum() > 100 and ((fl >> 2) & 1).sum() > 1000  # losses and lines covered
 
 
+def test_oracle_state_generator_reproduces_the_golden_states(oracle):
+    """The golden states are the reference harness's play-outs for seed 777 (make_golden.py); the
+    oracle's generator, which the larger tests draw their positions from, replays them exactly."""
+    states = GOLD["states"]
+    assert oracle.gen_states(777, len(states)).tobytes() == states.tobytes()
+
+
 def test_oracle_matches_compiled_reference_rules(oracle, ref):
     states = ref.gen_states(31337, 300000)
     rnd = step_rnd(5, len(states))
@@ -137,27 +144,27 @@ def test_swar_rules_header_matches_golden():
     assert [lib.shim_step_rnd(C.c_uint64(seed), C.c_uint64(i)) for i in range(64)] == list(r)
 
 
-def test_basic_moves_is_the_legal_mask_when_no_line_exists(ref):
+def test_basic_moves_is_the_legal_mask_when_no_line_exists(oracle):
     """The split game-logic kernel (game_step.cuh) finishes positions without a line from
     basic_moves() alone and queues the others: its line flag must equal legal_moves_t's and, when
     no line exists, its mask must be the legal mask. 300 k reachable positions + the golden set."""
     from corintho_ai_b200 import planes_from_reference_order
     lib = _shim()
     lib.shim_basic_moves_check.restype = C.c_int64
-    for states in (GOLD["states"], ref.gen_states(4242, 300000)):
+    for states in (GOLD["states"], oracle.gen_states(4242, 300000)):
         pl = planes_from_reference_order(states)
         bad = lib.shim_basic_moves_check(C.c_int64(len(pl)), pl.ctypes.data_as(C.c_void_p))
         assert bad == 0
 
 
-def test_paired_fast_path_forms_equal_the_plain_ones(ref):
+def test_paired_fast_path_forms_equal_the_plain_ones(oracle):
     """k_game_step_pair (game_step.cuh) runs basic_moves_pair / nth_move_lut / do_move_lut; on the
     host they must agree with basic_moves / nth_move / do_move for every position, every legal move
     and every rank. 300 k reachable positions + the golden set, paired first-with-last."""
     from corintho_ai_b200 import planes_from_reference_order
     lib = _shim()
     lib.shim_fast_path_check.restype = C.c_int64
-    for states in (GOLD["states"], ref.gen_states(777, 300000)):
+    for states in (GOLD["states"], oracle.gen_states(777, 300000)):
         pl = planes_from_reference_order(states)
         bad = lib.shim_fast_path_check(C.c_int64(len(pl)), pl.ctypes.data_as(C.c_void_p))
         assert bad == 0

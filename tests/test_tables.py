@@ -1,5 +1,5 @@
 """Rule DATA tables: product header == oracle copy == compiled reference == a fresh parse of
-the reference header (when /root/reference is present)."""
+the reference header (when CORINTHO_AI_REFERENCE names a checkout of the original project)."""
 import os
 import re
 import sys
@@ -9,6 +9,10 @@ import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, os.path.join(ROOT, "tools"))
+
+from util import NO_REFERENCE, reference_file  # noqa: E402
+
+UTIL_H = reference_file("corintho_ai/cpp/include/util.h")
 
 
 def parse_generated(path, prefix):
@@ -48,12 +52,10 @@ def test_tables_against_compiled_reference(ref, oracle):
         assert [ref.move_symmetry(k, j) for j in range(96)] == list(msym[k])
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/corintho_ai/cpp/include/util.h"),
-                    reason="reference tree not present")
+@pytest.mark.skipif(UTIL_H is None, reason=NO_REFERENCE)
 def test_tables_against_reference_header():
     import gen_tables
-    masks, gam_bits, space, move = gen_tables.parse_util_h(
-        "/root/reference/corintho_ai/cpp/include/util.h")
+    masks, gam_bits, space, move = gen_tables.parse_util_h(UTIL_H)
     lb, gam, ssym, msym = parse_generated(PRODUCT, "kC")
     assert (np.array(masks, np.uint32) == lb).all()
     assert (np.array(gam_bits, np.uint32) == gam).all()

@@ -6,10 +6,11 @@ import numpy as np
 import pytest
 
 from netref import forward_folded
+from util import NO_REFERENCE, REFERENCE, reference_file
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 FLAT = np.load(os.path.join(ROOT, "tests", "golden", "trained_net.npz"))["flat"]
-REF_TFLITE = "/root/reference/corintho_ai/docker/tflite_model.tflite"
+REF_TFLITE = reference_file("corintho_ai/docker/tflite_model.tflite")
 
 
 def _positions(oracle, n, seed=0):
@@ -41,7 +42,7 @@ def test_trained_network_prefers_legal_moves(oracle):
     assert mass[0] > 0.999  # the start position
 
 
-@pytest.mark.skipif(not os.path.exists(REF_TFLITE), reason="reference tree not present")
+@pytest.mark.skipif(REF_TFLITE is None, reason=NO_REFERENCE)
 def test_fixture_equals_fresh_import_and_all_checkpoints_load():
     import glob
     from corintho_ai_b200.tflite_import import load_tflite_weights, parse_tflite
@@ -50,7 +51,7 @@ def test_fixture_equals_fresh_import_and_all_checkpoints_load():
     assert tensors[inputs[0]]["shape"] == [1, 70]
     # rating/tourney.pyx:153-154: TFLite outputs are (policy, value), the reverse of Keras
     assert tensors[outputs[0]]["shape"] == [1, 96] and tensors[outputs[1]]["shape"] == [1, 1]
-    files = glob.glob("/root/reference/corintho_ai/rating/tflite_models/*.tflite")
+    files = glob.glob(os.path.join(REFERENCE, "corintho_ai", "rating", "tflite_models", "*.tflite"))
     assert len(files) == 95
     for f in files[::12]:
         assert load_tflite_weights(f).size == 127997

@@ -1,9 +1,27 @@
 """Shared helpers for the test-suite (numpy only)."""
 import hashlib
+import os
+import subprocess
 
 import numpy as np
 
 M64 = np.uint64(0xFFFFFFFFFFFFFFFF)
+
+# A checkout of the original corintho-ai project (the directory that holds corintho_ai/), where
+# oracle/Makefile builds the compiled reference from: the tests that compare with its sources or
+# shipped models directly skip without one.
+_ORACLE = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "oracle")
+_r = subprocess.run(["make", "-s", "--no-print-directory", "-C", _ORACLE, "print-ref"],
+                    capture_output=True, text=True)
+REFERENCE = _r.stdout.strip() if _r.returncode == 0 else ""
+NO_REFERENCE = ("no checkout of the original project at %r (oracle/Makefile REF; set CORINTHO_AI_REFERENCE)"
+                % REFERENCE)
+
+
+def reference_file(rel):
+    """Path of `rel` inside the original project's checkout, or None when it is not available."""
+    p = os.path.join(REFERENCE, rel) if REFERENCE else ""
+    return p if p and os.path.exists(p) else None
 
 
 def step_rnd(seed, n):
