@@ -13,8 +13,8 @@ import os
 
 import numpy as np
 
-__all__ = ["Trainer", "Corintho200Error", "game_step", "lib", "build", "NUM_MOVES", "STATE_SIZE",
-           "WEIGHT_FLOATS", "planes_from_reference_order", "reference_order_from_planes",
+__all__ = ["Trainer", "Tourney", "Analysis", "check_states", "Corintho200Error", "game_step", "lib",
+           "build", "NUM_MOVES", "STATE_SIZE", "WEIGHT_FLOATS", "planes_from_reference_order", "reference_order_from_planes",
            "random_weights", "fold_batchnorm"]
 
 NUM_MOVES = 96      # util.h:43
@@ -108,6 +108,12 @@ def lib():
         "cb200_tourney_counters": (i32, [vp, vp]),
         "cb200_tourney_set_weights": (i32, [vp, i32, vp, C.c_size_t, i32]),
         "cb200_tourney_run": (i32, [vp, i32]),
+        "cb200_analysis_create": (vp, [i32, i32, i32, f32, f32]),
+        "cb200_analysis_destroy": (None, [vp]),
+        "cb200_analysis_set_weights": (i32, [vp, vp, C.c_size_t, i32]),
+        "cb200_analysis_run": (i32, [vp, i32, vp, i32, vp, vp, vp, vp, vp]),
+        "cb200_analysis_counters": (i32, [vp, vp]),
+        "cb200_check_states": (i64, [i64, vp, vp]),
     }
     for name, (res, args) in sig.items():
         f = getattr(L, name)
@@ -549,3 +555,90 @@ class Tourney:
             self.writeScores(f.name)
             rows = [ln.split() for ln in open(f.name).read().splitlines() if ln.strip()]
         return [(int(a), int(b), float(c)) for a, b, c in rows]
+
+
+def _out_buf(a, dtype, min_size, what):
+    """Output buffer of a given dtype with the checks of _out_f32."""
+    if not isinstance(a, np.ndarray) or a.dtype != dtype or not a.flags.c_contiguous \
+            or not a.flags.writeable:
+        raise Corintho200Error(f"{what}: need a writable C-contiguous {np.dtype(dtype).name} numpy array")
+    if a.size < min_size:
+        raise Corintho200Error(f"{what}: {a.size} elements given, {min_size} needed")
+    return a
+
+
+def check_states(states):
+    """Structural check of cstates [n,2] u64 (see cb200_check_states): bool array, True = valid.
+    Needs no GPU."""
+    st = np.ascontiguousarray(states, np.uint64).reshape(-1, 2)
+    ok = np.zeros(st.shape[0], np.uint8)
+    _check(lib().cb200_check_states(st.shape[0], _ptr(st), _ptr(ok)))
+    return ok.astype(bool)
+
+
+class Analysis:
+    """The engine's move and search statistics for given positions: the batched form of the
+    reference's DockerMC (corintho_ai/cpp/src/dockermc.cpp) that docker/choose_move.pyx serves.
+    Every position is searched by one testing-mode TrainMC with the device-resident network, which
+    then chooses its move; see cb200_analysis_run in include/corintho_b200.h for the exact meaning
+    of every output."""
+
+    def __init__(self, max_positions, max_searches=1600, searches_per_eval=16, c_puct=1.0,
+                 epsilon=0.25):
+        L = lib()
+        h = L.cb200_analysis_create(int(max_positions), int(max_searches), int(searches_per_eval),
+                                    float(c_puct), float(epsilon))
+        if not h:
+            raise Corintho200Error("Analysis: " + L.cb200_last_error().decode())
+        self._h = C.c_void_p(h)
+        self.max_positions = int(max_positions)
+
+    def close(self):
+        if getattr(self, "_h", None):
+            lib().cb200_analysis_destroy(self._h)
+            self._h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def set_weights(self, flat_weights, precision="fp32"):
+        w = _in_f32(flat_weights, WEIGHT_FLOATS, "set_weights: weights")
+        prec = {"fp32": 0, "bf16": 1, "fp16": 2, "bf16x3": 3}[precision]
+        _check(lib().cb200_analysis_set_weights(self._h, _ptr(w), w.size, prec))
+
+    setWeights = set_weights
+
+    def run(self, states, seed=0, evals=True):
+        """states: [n,2] u64 cstates. Returns {"moves" [n] i32, "results" [n] i32, "values" [n]
+        f32, "visits" [n,96] i32, "evals" [n,96] f32 (only with evals=True)}."""
+        st = np.ascontiguousarray(states, np.uint64)
+        if st.ndim != 2 or st.shape[1] != 2:
+            raise Corintho200Error("run: states must be an [n, 2] array of cstate words")
+        n = st.shape[0]
+        out = {"moves": np.zeros(n, np.int32), "results": np.zeros(n, np.int32),
+               "values": np.zeros(n, np.float32), "visits": np.zeros((n, NUM_MOVES), np.int32)}
+        if evals:
+            out["evals"] = np.zeros((n, NUM_MOVES), np.float32)
+        self.run_into(st, seed, **out)
+        return out
+
+    def run_into(self, states, seed, moves, results, values, visits, evals=None):
+        """run() into caller-owned buffers (checked like the Trainer's output buffers)."""
+        st = np.ascontiguousarray(states, np.uint64).reshape(-1, 2)
+        n = st.shape[0]
+        _out_buf(moves, np.int32, n, "run: moves")
+        _out_buf(results, np.int32, n, "run: results")
+        _out_f32(values, n, "run: values")
+        _out_buf(visits, np.int32, n * NUM_MOVES, "run: visits")
+        if evals is not None:
+            _out_f32(evals, n * NUM_MOVES, "run: evals")
+        _check(lib().cb200_analysis_run(self._h, n, _ptr(st), int(seed), _ptr(moves), _ptr(results),
+                                        _ptr(values), _ptr(visits), _ptr(evals)))
+
+    def counters(self):
+        out = np.zeros(2, np.int64)
+        _check(lib().cb200_analysis_counters(self._h, _ptr(out)))
+        return {"simulations": int(out[0]), "leaf_evals": int(out[1])}

@@ -23,6 +23,7 @@
 #include "tree.cuh"
 #include "persistent.cuh"
 #include "match.cuh"
+#include "analysis.cuh"
 #include "gather.cuh"
 
 using namespace cb200;
@@ -1862,6 +1863,53 @@ int cb200_trainer_dump_tree(cb200_trainer *t, int game, int player, int64_t out[
 
 
 // ==============================================================================================
+// A device-resident network of the fused tourney (one per model id) and of the analysis. The
+// weights stay on the host until the first run that needs them uploads them (the device state may
+// not exist when they are set). Same weight layout and precision codes as cb200_trainer_set_weights.
+struct ResidentNet {
+  std::vector<float> host;
+  int precision = -1;  // -1 = no weights set
+  bool uploaded = false;
+  NetF32 f32;
+  NetTC tc;
+};
+
+static void resident_net_set(ResidentNet &n, const float *weights, int precision) {
+  n.host.assign(weights, weights + kNetWeightFloats);
+  n.precision = precision;
+  n.uploaded = false;
+}
+
+static int resident_net_upload(ResidentNet &n) {
+  if (n.uploaded) return CB200_OK;
+  // tensor-core operand modes: precision 1 -> bf16, 2 -> fp16, 3 -> bf16x3 (hi + lo operands)
+  const int rc = n.precision == 0 ? net_f32_upload(n.f32, n.host.data())
+                                  : net_tc_upload(n.tc, n.host.data(), n.precision == 1 ? 0 : (n.precision == 2 ? 1 : 2));
+  if (rc == CB200_OK) n.uploaded = true;
+  return rc;
+}
+
+static void resident_net_free(ResidentNet &n) {
+  cudaFree(n.f32.w);
+  n.f32.w = nullptr;
+  net_tc_free(n.tc);
+}
+
+// Evaluate the leaf cstates packed[0 .. t->d_summary[0]) into t's answer buffers on the current
+// stream. The answer of row k for move m is then at d_probs[k * prs + m * pcs]: row-major from the
+// fp32 kernel, move-major (leading dimension cap + kAnswerSlack) from the tensor-core kernel.
+static int resident_net_launch(const ResidentNet &n, cb200_trainer *t, const ulonglong2 *packed, long &prs,
+                               long &pcs) {
+  if (n.precision == 0) {
+    prs = CB200_NUM_MOVES, pcs = 1;
+    return launch_mlp_f32(n.f32, packed, t->d_summary, 0, (int)t->cap, t->d_eval, t->d_probs);
+  }
+  prs = 1, pcs = (long)(t->cap + kAnswerSlack);
+  return launch_mlp_tc(n.tc, packed, t->d_summary, 0, (int)t->cap, t->d_eval, t->d_probs,
+                       (int)(t->cap + kAnswerSlack));
+}
+
+// ==============================================================================================
 // Tourney (corintho_ai/cpp/include/tourney.h:12-46) over Match (match.h:33-101); device side in
 // match.cuh. The matches share the per-game storage of a trainer created when the first call
 // needs the device (all players and matches must have been added by then).
@@ -1879,14 +1927,7 @@ struct cb200_tourney {
   // fused mode (cb200_tourney_set_weights / cb200_tourney_run): one device-resident network per
   // model id, evaluated in the first-seen order of the ids like rating/tourney.pyx:112-173
   std::vector<int> model_order;
-  struct Net {
-    std::vector<float> host;  // kept until the device exists
-    int precision = -1;
-    bool uploaded = false;
-    NetF32 f32;
-    NetTC tc;
-  };
-  std::map<int, Net> nets;
+  std::map<int, ResidentNet> nets;
 };
 
 static int tourney_ready_build(cb200_tourney *T, cb200_trainer *t, const std::vector<MatchSide> &sides,
@@ -2011,10 +2052,7 @@ cb200_tourney *cb200_tourney_create(int num_threads, const char *log_folder) {
 void cb200_tourney_destroy(cb200_tourney *T) {
   if (!T) return;
   cudaFree(T->d_sides), cudaFree(T->d_pack_offs), cudaFree(T->d_iter_offs);
-  for (auto &kv : T->nets) {
-    cudaFree(kv.second.f32.w);
-    net_tc_free(kv.second.tc);
-  }
+  for (auto &kv : T->nets) resident_net_free(kv.second);
   if (T->t) cb200_trainer_destroy(T->t);
   delete T;
 }
@@ -2116,10 +2154,7 @@ int cb200_tourney_set_weights(cb200_tourney *T, int model_id, const float *weigh
   if (model_id < 0 || !weights || n_floats != kNetWeightFloats || precision < 0 || precision > 3)
     return set_error(CB200_ERR_ARG, "cb200_tourney_set_weights: bad arguments (model id >= 0, 127997 floats, "
                                     "precision 0|1|2|3)");
-  cb200_tourney::Net &n = T->nets[model_id];
-  n.host.assign(weights, weights + n_floats);
-  n.precision = precision;
-  n.uploaded = false;
+  resident_net_set(T->nets[model_id], weights, precision);
   return CB200_OK;
 }
 
@@ -2133,13 +2168,7 @@ int cb200_tourney_run(cb200_tourney *T, int max_rounds) {
     auto it = T->nets.find(id);
     if (it == T->nets.end() || it->second.precision < 0)
       return set_error(CB200_ERR_STATE, "cb200_tourney_run: no weights set for model " + std::to_string(id));
-    cb200_tourney::Net &n = it->second;
-    if (!n.uploaded) {
-      rc = n.precision == 0 ? net_f32_upload(n.f32, n.host.data())
-                            : net_tc_upload(n.tc, n.host.data(), n.precision == 1 ? 0 : (n.precision == 2 ? 1 : 2));
-      if (rc != CB200_OK) return rc;
-      n.uploaded = true;
-    }
+    if ((rc = resident_net_upload(it->second)) != CB200_OK) return rc;
   }
   cudaStream_t st = cur_stream();
   const int grid = (t->P.num_games + kTreeWarps - 1) / kTreeWarps;
@@ -2161,18 +2190,10 @@ int cb200_tourney_run(cb200_tourney *T, int max_rounds) {
         CB_LAUNCHED();
         long prs = CB200_NUM_MOVES, pcs = 1;
         if (id >= 0) {
-          cb200_tourney::Net &n = T->nets[id];
           k_match_pack<<<(t->P.num_games + 7) / 8, 256, 0, st>>>(t->P, T->d_sides, id, T->d_pack_offs, nullptr,
                                                                  t->d_packed);
           CB_LAUNCHED();
-          if (n.precision == 0) {
-            rc = launch_mlp_f32(n.f32, t->d_packed, t->d_summary, 0, (int)t->cap, t->d_eval, t->d_probs);
-          } else {
-            rc = launch_mlp_tc(n.tc, t->d_packed, t->d_summary, 0, (int)t->cap, t->d_eval, t->d_probs,
-                               (int)(t->cap + kAnswerSlack));
-            prs = 1, pcs = (long)(t->cap + kAnswerSlack);
-          }
-          if (rc != CB200_OK) return rc;
+          if ((rc = resident_net_launch(T->nets[id], t, t->d_packed, prs, pcs)) != CB200_OK) return rc;
         }
         k_match_iterate<<<grid, kTreeWarps * 32, 0, st>>>(t->P, T->d_sides, t->d_eval, t->d_probs, T->d_iter_offs,
                                                           id, prs, pcs);
@@ -2208,6 +2229,163 @@ int cb200_tourney_counters(cb200_tourney *T, int64_t out[4]) {
   int rc = tourney_ready(T);
   if (rc) return rc;
   return cb200_trainer_counters(T->t, out);
+}
+
+// ==============================================================================================
+// Analysis (the reference's DockerMC, dockermc.cpp, for a batch of given positions); device side
+// in analysis.cuh. The positions use the per-game storage of an internal testing-mode trainer, one
+// "game" per position, created with the analysis object; every run re-seeds and resets it.
+
+// The structural invariants of a cstate that the engine accepts from a caller (checked over the
+// reachable positions of 1 000 000 random play-outs by tests/test_oracle_analysis.py): side to move
+// 0 or 1, byte 7 zero, at most 4 pieces of a kind in a hand, frozen squares occupied, and every
+// piece of a kind either on the board or in a hand (8 of each kind).
+static bool valid_state(uint64_t w0, uint64_t w1) {
+  if (((w1 >> 48) & 0xff) > 1 || (w1 >> 56) != 0) return false;
+  const uint32_t base = (uint32_t)(w0 & 0xffff), column = (uint32_t)((w0 >> 16) & 0xffff);
+  const uint32_t capital = (uint32_t)((w0 >> 32) & 0xffff), frozen = (uint32_t)(w0 >> 48);
+  if (frozen & ~(base | column | capital)) return false;
+  const uint32_t plane[3] = {base, column, capital};
+  for (int t = 0; t < 3; ++t) {
+    const int h0 = (int)((w1 >> (8 * t)) & 0xff), h1 = (int)((w1 >> (8 * (3 + t))) & 0xff);
+    if (h0 > 4 || h1 > 4 || __builtin_popcount(plane[t]) != 8 - h0 - h1) return false;
+  }
+  return true;
+}
+
+int64_t cb200_check_states(int64_t n, const uint64_t *states, uint8_t *valid) {
+  if (n < 0 || (n > 0 && !states)) return set_error(CB200_ERR_ARG, "cb200_check_states: bad arguments");
+  int64_t bad = 0;
+  for (int64_t i = 0; i < n; ++i) {
+    const bool ok = valid_state(states[2 * i], states[2 * i + 1]);
+    if (valid) valid[i] = ok ? 1 : 0;
+    bad += ok ? 0 : 1;
+  }
+  return bad;
+}
+
+struct cb200_analysis {
+  int max_positions = 0, max_searches = 0;
+  cb200_trainer *t = nullptr;  // trainer max_searches = max(max_searches, spe): it sizes the arenas only
+  ulonglong2 *d_roots = nullptr;   // [max_positions] the positions of the current run
+  int32_t *d_moves = nullptr, *d_results = nullptr, *d_visits = nullptr;
+  float *d_values = nullptr, *d_evals = nullptr;
+  ResidentNet net;
+  int64_t counters[2] = {0, 0};    // {simulations, leaf evaluations} of the last run
+};
+
+cb200_analysis *cb200_analysis_create(int max_positions, int max_searches, int searches_per_eval, float c_puct,
+                                      float epsilon) {
+  last_error_ref().clear();
+  // the validation of cb200_tourney_add_player
+  if (max_positions <= 0 || max_searches <= 0 || searches_per_eval <= 0 || searches_per_eval > 64 ||
+      !(c_puct > 0.0f) || !(epsilon >= 0.0f) || !(epsilon <= 1.0f)) {
+    set_error(CB200_ERR_ARG, "cb200_analysis_create: invalid argument");
+    return nullptr;
+  }
+  cb200_trainer *t = cb200_trainer_create_shard(max_positions, 0, max_positions, "", 0,
+                                                std::max(max_searches, searches_per_eval), searches_per_eval,
+                                                c_puct, epsilon, 0, 1);
+  if (!t) return nullptr;
+  cb200_analysis *A = new cb200_analysis();
+  A->max_positions = max_positions, A->max_searches = max_searches, A->t = t;
+  const size_t n = (size_t)max_positions;
+  if (dmalloc(&A->d_roots, n) != CB200_OK || dmalloc(&A->d_moves, n) != CB200_OK ||
+      dmalloc(&A->d_results, n) != CB200_OK || dmalloc(&A->d_values, n) != CB200_OK ||
+      dmalloc(&A->d_visits, n * CB200_NUM_MOVES) != CB200_OK ||
+      dmalloc(&A->d_evals, n * CB200_NUM_MOVES) != CB200_OK) {
+    const std::string msg = last_error_ref();
+    cb200_analysis_destroy(A);
+    last_error_ref() = msg;
+    return nullptr;
+  }
+  return A;
+}
+
+void cb200_analysis_destroy(cb200_analysis *A) {
+  if (!A) return;
+  if (A->t) cudaSetDevice(A->t->device);
+  cudaFree(A->d_roots), cudaFree(A->d_moves), cudaFree(A->d_results), cudaFree(A->d_values);
+  cudaFree(A->d_visits), cudaFree(A->d_evals);
+  resident_net_free(A->net);
+  if (A->t) cb200_trainer_destroy(A->t);
+  delete A;
+}
+
+int cb200_analysis_set_weights(cb200_analysis *A, const float *weights, size_t n_floats, int precision) {
+  last_error_ref().clear();
+  if (!A) return set_error(CB200_ERR_ARG, "null analysis");
+  if (!weights || n_floats != kNetWeightFloats || precision < 0 || precision > 3)
+    return set_error(CB200_ERR_ARG, "cb200_analysis_set_weights: bad arguments (127997 floats, precision 0|1|2|3)");
+  resident_net_set(A->net, weights, precision);
+  return CB200_OK;
+}
+
+int cb200_analysis_run(cb200_analysis *A, int n, const uint64_t *states, int seed, int32_t *moves,
+                       int32_t *results, float *values, int32_t *visits, float *evals) {
+  last_error_ref().clear();
+  if (!A) return set_error(CB200_ERR_ARG, "null analysis");
+  if (n <= 0 || n > A->max_positions)
+    return set_error(CB200_ERR_ARG, "cb200_analysis_run: n must be in [1, max_positions]");
+  if (!states || !moves || !results || !values || !visits)
+    return set_error(CB200_ERR_ARG, "cb200_analysis_run: null states / moves / results / values / visits");
+  for (int i = 0; i < n; ++i)
+    if (!valid_state(states[2 * i], states[2 * i + 1]))
+      return set_error(CB200_ERR_ARG, "cb200_analysis_run: state " + std::to_string(i) + " is not a valid cstate");
+  if (A->net.precision < 0) return set_error(CB200_ERR_STATE, "cb200_analysis_run: no weights set");
+  cb200_trainer *t = A->t;
+  int rc = guard(t);
+  if (rc != CB200_OK) return rc;
+  if ((rc = resident_net_upload(A->net)) != CB200_OK) return rc;
+  A->counters[0] = A->counters[1] = 0;
+  // positions [0, n) become games [0, n) of the trainer: seeds = outputs 0 .. n-1 of mt19937(seed),
+  // fresh control blocks and trees (the kernel builds each root on its first round)
+  t->P.num_games = n;
+  if ((rc = cb200_trainer_reset(t, seed)) != CB200_OK) return rc;
+  cudaStream_t st = cur_stream();
+  CB_CUDA(cudaMemcpyAsync(A->d_roots, states, (size_t)n * sizeof(ulonglong2), cudaMemcpyHostToDevice, st));
+  const AnalysisOut out{A->d_moves, A->d_results, A->d_values, A->d_visits, evals ? A->d_evals : nullptr};
+  const int grid = (n + kTreeWarps - 1) / kTreeWarps;
+  // every round completes at least one search or the turn of each live position
+  const int max_rounds = A->max_searches + 8;
+  for (int round = 0;; ++round) {
+    // request offsets of every live position (contiguous packing) and the live count
+    k_scan_requests<<<1, 1024, 0, st>>>(t->P, -1, t->d_offs, t->d_summary);
+    CB_LAUNCHED();
+    if (round % 8 == 0) {  // one small read-back every few rounds
+      if ((rc = fetch_summary(t)) != CB200_OK) return rc;
+      if (t->h_summary[1] == 0) break;
+      if (round > max_rounds) return set_error(CB200_ERR_STATE, "cb200_analysis_run: the searches did not finish");
+    }
+    k_pack_requests<<<(n + 7) / 8, 256, 0, st>>>(t->P, -1, t->d_offs, nullptr, t->d_packed);
+    CB_LAUNCHED();
+    long prs = 0, pcs = 0;
+    if ((rc = resident_net_launch(A->net, t, t->d_packed, prs, pcs)) != CB200_OK) return rc;
+    k_analysis_iterate<<<grid, kTreeWarps * 32, 0, st>>>(t->P, A->max_searches, A->d_roots, t->d_eval,
+                                                          t->d_probs, prs, pcs, t->d_offs, out);
+    CB_LAUNCHED();
+    CB_CUDA(cudaGetLastError());
+    ++t->iterations_done;
+  }
+  CB_CUDA(cudaMemcpyAsync(moves, A->d_moves, (size_t)n * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+  CB_CUDA(cudaMemcpyAsync(results, A->d_results, (size_t)n * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+  CB_CUDA(cudaMemcpyAsync(values, A->d_values, (size_t)n * sizeof(float), cudaMemcpyDeviceToHost, st));
+  CB_CUDA(cudaMemcpyAsync(visits, A->d_visits, (size_t)n * CB200_NUM_MOVES * sizeof(int32_t),
+                          cudaMemcpyDeviceToHost, st));
+  if (evals)
+    CB_CUDA(cudaMemcpyAsync(evals, A->d_evals, (size_t)n * CB200_NUM_MOVES * sizeof(float),
+                            cudaMemcpyDeviceToHost, st));
+  int64_t c4[4];
+  if ((rc = cb200_trainer_counters(t, c4)) != CB200_OK) return rc;  // synchronises the stream
+  A->counters[0] = c4[0], A->counters[1] = c4[2];
+  return CB200_OK;
+}
+
+int cb200_analysis_counters(cb200_analysis *A, int64_t out[2]) {
+  last_error_ref().clear();
+  if (!A || !out) return set_error(CB200_ERR_ARG, "null analysis / out");
+  out[0] = A->counters[0], out[1] = A->counters[1];
+  return CB200_OK;
 }
 
 }  // extern "C"

@@ -257,6 +257,55 @@ int cb200_tourney_run(cb200_tourney *t, int max_rounds);
 /* out = {simulations, moves, leaf evaluations, do_iteration calls} over all matches */
 int cb200_tourney_counters(cb200_tourney *t, int64_t out[4]);
 
+/* ---- Analysis: the engine's move and search statistics for given positions ------------------
+ * The batched form of the reference's DockerMC (corintho_ai/cpp/src/dockermc.cpp, served by
+ * docker/choose_move.pyx): every position is searched by one testing-mode TrainMC with the
+ * resident network, which then chooses its move exactly as TrainMC::chooseMove does in testing
+ * mode (trainmc.cpp:110-137, 438-473; no opening randomisation). Parameters max_searches,
+ * searches_per_eval, c_puct, epsilon: meaning and validation as in cb200_tourney_add_player
+ * (searches_per_eval <= 64). The object holds device storage for max_positions positions, sized
+ * once and reused by every run. */
+typedef struct cb200_analysis cb200_analysis;
+cb200_analysis *cb200_analysis_create(int max_positions, int max_searches, int searches_per_eval,
+                                      float c_puct, float epsilon);  /* NULL on error */
+void cb200_analysis_destroy(cb200_analysis *a);
+/* Same weight layout and precision codes as cb200_trainer_set_weights. */
+int cb200_analysis_set_weights(cb200_analysis *a, const float *weights, size_t n_floats, int precision);
+/* Search every position of states[n][2] (cstates, layout at the top of this file).
+ *   Random stream: position i's mt19937 is seeded with the i-th output of mt19937(seed), the rule of
+ *     the Trainer's game seeds (trainer.cpp:238-256), so a position's outputs depend only on its
+ *     index, the seed, the parameters and the network -- not on n or the rest of the batch.
+ *   Side to move: byte 6 of the cstate; that side's tree is searched. Depth is not an input (in
+ *     testing mode only the logs read it).
+ *   Outputs, read from the root before the move is applied:
+ *     moves[i]     the move id chosen (-1 for a position without a legal move);
+ *     results[i]   the root's result code, from the view of the side to move:
+ *                  0 unknown, 1 lost (no legal move, a line on the board), 2 drawn (no legal move,
+ *                  no line), 4 proven lost, 5 proven drawn, 6 proven won (util.h:58-61 kResult*,
+ *                  kDeduced*); 3 never occurs;
+ *     values[i]    the root's evaluation_: the running sum the search keeps over the root's
+ *                  visits, from the view of the side to move (higher is better for it);
+ *     visits[i][m] the visits_ of the child reached by move id m (0 for an illegal or unexpanded
+ *                  move);
+ *     evals[i][m]  that child's evaluation_, from the view of the side to move in the child (the
+ *                  opponent): -evals / visits is the move's mean value for the side to move, the
+ *                  exploitation term of PUCT selection (trainmc.cpp:540-600). May be NULL.
+ *   A position without a legal move is not searched: move -1, result 1 or 2, visits and value 0.
+ * Errors: CB200_ERR_ARG for n <= 0, n > max_positions, a null required pointer or a state that
+ * cb200_check_states rejects; CB200_ERR_STATE without weights; CB200_ERR_OVERFLOW when a search
+ * overflowed its node arena; CB200_ERR_CUDA without a usable device. The object stays usable after
+ * an error. */
+int cb200_analysis_run(cb200_analysis *a, int n, const uint64_t *states, int seed,
+                       int32_t *moves /* [n] */, int32_t *results /* [n] */, float *values /* [n] */,
+                       int32_t *visits /* [n][96] */, float *evals /* [n][96] or NULL */);
+/* out = {simulations, leaf evaluations} of the last run */
+int cb200_analysis_counters(cb200_analysis *a, int64_t out[2]);
+/* Structural check of cstates given by a caller (no device needed): byte 6 (side to move) 0 or 1,
+ * byte 7 zero, at most 4 pieces of a kind in either hand, frozen squares occupied, and for every
+ * kind, pieces on the board = 8 - both hands' count. valid[i] (may be NULL) = 1 / 0. Returns the
+ * number of rejected states, < 0 on bad arguments. */
+int64_t cb200_check_states(int64_t n, const uint64_t *states /* [n][2] */, uint8_t *valid);
+
 #ifdef __cplusplus
 }
 #endif

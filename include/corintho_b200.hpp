@@ -123,9 +123,36 @@ class Tourney {
   int rows_ = 0;
 };
 
+/* Beyond the reference: the batched DockerMC (dockermc.cpp) -- a searched move choice and the root
+ * statistics for every given position (cb200_analysis_run in corintho_b200.h; INTEGRATION.md 7). */
+class Analysis {
+ public:
+  Analysis(int max_positions, int max_searches = 1600, int searches_per_eval = 16, float c_puct = 1.0f,
+           float epsilon = 0.25f)
+      : h_{cb200_analysis_create(max_positions, max_searches, searches_per_eval, c_puct, epsilon)} {
+    if (!h_) throw std::runtime_error(cb200_last_error());
+  }
+  ~Analysis() { cb200_analysis_destroy(h_); }
+  Analysis(const Analysis &) = delete;
+  Analysis &operator=(const Analysis &) = delete;
+
+  void setWeights(const float *weights, size_t n_floats, int precision) {
+    check(cb200_analysis_set_weights(h_, weights, n_floats, precision));
+  }
+  void run(int n, const uint64_t *states, int seed, int32_t *moves, int32_t *results, float *values,
+           int32_t *visits, float *evals = nullptr) {
+    check(cb200_analysis_run(h_, n, states, seed, moves, results, values, visits, evals));
+  }
+  cb200_analysis *handle() { return h_; }
+
+ private:
+  cb200_analysis *h_;
+};
+
 }  // namespace cb200_host
 
 #ifndef CB200_HPP_NO_GLOBAL_NAMES
+using cb200_host::Analysis;
 using cb200_host::Tourney;
 using cb200_host::Trainer;
 #endif
