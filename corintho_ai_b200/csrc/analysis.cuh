@@ -65,7 +65,6 @@ __global__ void __launch_bounds__(kTreeWarps * 32, 4)
   const ulonglong2 rv = roots[g];
   const CState root{rv.x, rv.y};
   Ctx c;
-  c.bind_lanes();
   c.to_play = (int)((root.w1 >> 48) & 0xffu), c.parity = 0, c.result = ctl[CW_RESULT];
   c.mate_turn = 0, c.n_samples = 0;
   c.n_pending = ctl[CW_N_PENDING], c.error = ctl[CW_ERROR], c.spare = ctl[CW_SPARE];

@@ -151,10 +151,6 @@ struct cb200_trainer {
   int seed = 0;
   // fused mode: games are split into independent stream groups (no lock-step across groups)
   int n_groups = 1;
-  int lanes = kGameLanes;     // lanes per game in the lock-step kernels (CB200_LANES overrides)
-  int ps_lanes = 32;          // ... and in the persistent kernels (CB200_PS_LANES)
-  int min_blocks = 6;         // resident CTAs per SM the fused game step is compiled for (CB200_MINBLOCKS):
-                              // 24 warps per SM at 85 registers; +1 % at 4 096 games, +10 % at 32 768 over 4
   int32_t *d_live_list = nullptr;   // [num_games] live games per stream group (TreeParams::live_list)
   int32_t *d_live_count = nullptr;  // [n_groups]
   std::vector<cudaStream_t> g_stream;
@@ -345,16 +341,8 @@ int iterate(cb200_trainer *t, const float *d_eval, const float *d_probs, int to_
   const long prs = probs_move_major ? 1 : CB200_NUM_MOVES;
   const long pcs = probs_move_major ? (long)t->cap : 1;
   ProfScope ps(t, 3);
-  // lanes per game: 16 (two games per warp; the default) or 32 (CB200_LANES=32, for comparison)
-  if (t->lanes == 32) {
-    const int per_cta = kTreeWarps;
-    k_iterate<false, 32, 4><<<(t->P.num_games + per_cta - 1) / per_cta, kTreeWarps * 32, 0, cur_stream()>>>(
-        t->P, d_eval, d_probs, prs, pcs, t->d_offs, to_play, t->iterations_done, t->stagger_div);
-  } else {
-    const int per_cta = kTreeWarps * 2;
-    k_iterate<false, 16, 4><<<(t->P.num_games + per_cta - 1) / per_cta, kTreeWarps * 32, 0, cur_stream()>>>(
-        t->P, d_eval, d_probs, prs, pcs, t->d_offs, to_play, t->iterations_done, t->stagger_div);
-  }
+  k_iterate<false, 4><<<(t->P.num_games + kTreeWarps - 1) / kTreeWarps, kTreeWarps * 32, 0, cur_stream()>>>(
+      t->P, d_eval, d_probs, prs, pcs, t->d_offs, to_play, t->iterations_done, t->stagger_div);
   CB_LAUNCHED();
   CB_CUDA(cudaGetLastError());
   if (to_play != 0 && to_play != 1) ++t->iterations_done;
@@ -796,11 +784,8 @@ cb200_trainer *cb200_trainer_create_shard(int total_games, int first_game, int n
   if (ng < 1) ng = 1;
   while (ng > 1 && num_games / ng < 64) ng /= 2;
   t->n_groups = ng;
-  if (const char *env = getenv("CB200_LANES")) t->lanes = atoi(env) == 32 ? 32 : 16;
-  if (const char *env = getenv("CB200_MINBLOCKS")) t->min_blocks = atoi(env);
-  if (const char *env = getenv("CB200_PS_LANES")) t->ps_lanes = atoi(env) == 16 ? 16 : 32;
-  const int per_cta = kTreeWarps * (32 / t->lanes);  // games per CTA of the lock-step kernel
-  int per = ((num_games + ng - 1) / ng + per_cta - 1) / per_cta * per_cta;
+  // group boundaries fall on whole CTAs of the lock-step kernel (kTreeWarps games)
+  int per = ((num_games + ng - 1) / ng + kTreeWarps - 1) / kTreeWarps * kTreeWarps;
   for (int g = 0; g < ng; ++g) {
     int b = g * per, e = b + per < num_games ? b + per : num_games;
     if (b >= num_games) {
@@ -1440,11 +1425,11 @@ static int ps_list_games(cb200_trainer *t) {
 }
 
 extern "C++" {
-template <int kMode, int kGames, int kL>
+template <int kMode, int kGames>
 static int ps_launch(cb200_trainer *t, const TreeParams &P, int rounds, int exit_done) {
   static bool attr_set[16] = {false};
   if (t->device < 16 && !attr_set[t->device]) {
-    CB_CUDA(cudaFuncSetAttribute(k_selfplay_persistent<kMode, kGames, kL>,
+    CB_CUDA(cudaFuncSetAttribute(k_selfplay_persistent<kMode, kGames>,
                                  cudaFuncAttributeMaxDynamicSharedMemorySize,
                                  (int)ps_smem_bytes<kMode, kGames>()));
     attr_set[t->device] = true;
@@ -1457,7 +1442,7 @@ static int ps_launch(cb200_trainer *t, const TreeParams &P, int rounds, int exit
   const int grid = t->ps_n < t->ps_ctas ? t->ps_n : t->ps_ctas;
   // two-model (gating match) runs: model 1 answers the other side's requests
   const uint8_t *w1 = P.testing ? (const uint8_t *)t->nettc[1].w : nullptr;
-  k_selfplay_persistent<kMode, kGames, kL><<<grid, kGames * kL, ps_smem_bytes<kMode, kGames>(), t->g_stream[0]>>>(
+  k_selfplay_persistent<kMode, kGames><<<grid, kGames * 32, ps_smem_bytes<kMode, kGames>(), t->g_stream[0]>>>(
       P, (const uint8_t *)t->nettc[0].w, w1, t->d_ps_list, t->ps_n, ev0, pr0, pcs0, t->d_ps_eval[nxt],
       t->d_ps_probs[nxt], t->ps_ld, t->d_ps_packed, rounds, exit_done, t->iterations_done,
       t->d_ps_out);
@@ -1544,21 +1529,12 @@ static int run_persistent(cb200_trainer *t, int max_rounds, int *rounds_done, bo
     int rc;
     {
       ProfScope ps(t, wide ? 5 : 4, st);
-      // lanes per game: one warp (the default: the tail is bound by the serial chain of a game,
-      // which is shortest with 32 lanes) or 16 (CB200_PS_LANES=16)
-      const bool half = t->ps_lanes == 16;
       if (mode == 2)
-        rc = half ? ps_launch<2, 8, 16>(t, P, rounds, exit_done) : ps_launch<2, 8, 32>(t, P, rounds, exit_done);
+        rc = ps_launch<2, 8>(t, P, rounds, exit_done);
       else if (mode == 1)
-        rc = wide ? (half ? ps_launch<1, 16, 16>(t, P, rounds, exit_done)
-                          : ps_launch<1, 16, 32>(t, P, rounds, exit_done))
-                  : (half ? ps_launch<1, 8, 16>(t, P, rounds, exit_done)
-                          : ps_launch<1, 8, 32>(t, P, rounds, exit_done));
+        rc = wide ? ps_launch<1, 16>(t, P, rounds, exit_done) : ps_launch<1, 8>(t, P, rounds, exit_done);
       else
-        rc = wide ? (half ? ps_launch<0, 16, 16>(t, P, rounds, exit_done)
-                          : ps_launch<0, 16, 32>(t, P, rounds, exit_done))
-                  : (half ? ps_launch<0, 8, 16>(t, P, rounds, exit_done)
-                          : ps_launch<0, 8, 32>(t, P, rounds, exit_done));
+        rc = wide ? ps_launch<0, 16>(t, P, rounds, exit_done) : ps_launch<0, 8>(t, P, rounds, exit_done);
     }
     if (rc != CB200_OK) return rc;
     CB_CUDA(cudaMemcpyAsync(t->h_ps_out, t->d_ps_out, 4 * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
@@ -1622,9 +1598,9 @@ static int run_selfplay_groups(cb200_trainer *t, int max_iterations) {
   if (ps_capacity > ps_max) ps_capacity = ps_max;
   const int stagger_span =
       t->stagger_div > 0 ? (t->P.first_game + t->P.num_games - 1) / t->stagger_div : 0;
-  // With several stream groups the game step runs in its 96-register build (four CTAs leave
-  // 16 K registers per SM) and the network in single-tile CTAs of 128 threads that fit beside
-  // them, so that one group's network overlaps the other groups' tree work (2-3 % per run).
+  // With several stream groups the network runs in single-tile CTAs of 128 threads (13 K
+  // registers) that fit beside five 80-register game-step CTAs, so that one group's network
+  // overlaps the other groups' tree work (2-3 % per run).
   const bool overlap = tc && ng > 1 && getenv("CB200_NO_OVERLAP") == nullptr;
   const bool use_lists = getenv("CB200_NO_LIVE_LIST") == nullptr;
   std::vector<int> group_live(ng, -1);  // live games per group at the last host sync (-1 = unknown)
@@ -1666,9 +1642,8 @@ static int run_selfplay_groups(cb200_trainer *t, int max_iterations) {
     const int yb = live_games >= yield_min_live ? yield_budget : 0;
     int batch = 32;
     if (max_iterations > 0 && max_iterations - done_iters < batch) batch = max_iterations - done_iters;
-    // the games of each group that are still live (finished games would leave idle lane groups
+    // the games of each group that are still live (finished games would leave idle warps
     // behind): rebuilt once per batch on the group's own stream
-    const int per_cta = kTreeWarps * (32 / t->lanes);
     for (int g = 0; g < ng && use_lists; ++g) {
       if (!active[g]) continue;
       TreeParams P = t->P;
@@ -1699,29 +1674,19 @@ static int run_selfplay_groups(cb200_trainer *t, int max_iterations) {
         TreeParams P = t->P;
         P.game_begin = gb, P.game_end = ge, P.group_row0 = row0, P.group_ctr = ctr;
         P.yield_budget = yb;
-        int width = ge - gb;  // lane groups to launch: the group's games, or its live games
+        int width = ge - gb;  // warps to launch: the group's games, or its live games
         if (use_lists) {
           P.live_list = t->d_live_list, P.live_count = t->d_live_count + g;
           if (group_live[g] >= 0 && group_live[g] < width) width = group_live[g];
         }
         {
           ProfScope ps(t, 3, st);
-          const dim3 grid((width + per_cta - 1) / per_cta), block(kTreeWarps * 32);
+          const dim3 grid((width + kTreeWarps - 1) / kTreeWarps), block(kTreeWarps * 32);
           if (grid.x > 0) {
-#define CB_ITER(L, MB) \
-  k_iterate<true, L, MB><<<grid, block, 0, st>>>(P, t->d_eval, t->d_probs, prs, pcs, nullptr, -1, it, t->stagger_div)
-            // lanes per game x resident CTAs per SM (register budget 65536 / (128 * MB))
-            if (t->lanes == 32) {
-              if (t->min_blocks >= 8) CB_ITER(32, 8);
-              else if (t->min_blocks == 7) CB_ITER(32, 7);
-              else if (t->min_blocks == 6) CB_ITER(32, 6);
-              else if (t->min_blocks == 5) CB_ITER(32, 5);
-              else CB_ITER(32, 4);
-            } else {
-              if (t->min_blocks <= 3) CB_ITER(16, 3);
-              else CB_ITER(16, 4);
-            }
-#undef CB_ITER
+            // built for 6 resident CTAs per SM (80 registers): faster than 4, 5, 7 or 8 at 4 096,
+            // 8 192 and 32 768 games (profiles/r02_register_budget_final.txt)
+            k_iterate<true, 6><<<grid, block, 0, st>>>(P, t->d_eval, t->d_probs, prs, pcs, nullptr, -1, it,
+                                                       t->stagger_div);
             CB_LAUNCHED();
           }
         }

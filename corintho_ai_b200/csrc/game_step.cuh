@@ -1,7 +1,9 @@
-// K1: game-logic kernel (BASELINE.json configs[1]) -- one thread per state.
+// K1: game-logic kernel (BASELINE.json configs[1]).
 // Per state: 16 B read (cstate), 16 B written (legal mask + flags), 16 B written (next state);
 // the optional 70-float NN encoding is written warp-cooperatively so stores stay coalesced.
-// HBM-bound by construction; see DESIGN.md "K1" for the roofline arithmetic.
+// HBM-bound by construction; see DESIGN.md "K1" for the roofline arithmetic. Two kernels:
+// k_game_step_encode when the encoding is requested, k_game_step_pairw otherwise. The forms
+// measured against the latter in round 2 are in profiles/r02_k1_paired_variants.txt.
 #ifndef CORINTHO_B200_GAME_STEP_CUH
 #define CORINTHO_B200_GAME_STEP_CUH
 
@@ -11,12 +13,12 @@ namespace cb200 {
 
 constexpr int kStepThreads = 256;
 
-template <bool kEncode>
+// Encoding form (the 70-float NN encoding is requested): one thread per state.
 __global__ void __launch_bounds__(kStepThreads)
-    k_game_step(int64_t n, const ulonglong2 *__restrict__ states, uint64_t seed,
-                uint4 *__restrict__ mask_flags, ulonglong2 *__restrict__ next,
-                float *__restrict__ enc) {
-  __shared__ ulonglong2 sm_states[kEncode ? kStepThreads : 1];
+    k_game_step_encode(int64_t n, const ulonglong2 *__restrict__ states, uint64_t seed,
+                       uint4 *__restrict__ mask_flags, ulonglong2 *__restrict__ next,
+                       float *__restrict__ enc) {
+  __shared__ ulonglong2 sm_states[kStepThreads];
   // 32-bit indices: the launcher refuses more than 2^31 - 2^20 states per call; the loop counter
   // is unsigned so that the last `+= stride` cannot wrap
   const unsigned stride = gridDim.x * kStepThreads;
@@ -33,7 +35,7 @@ __global__ void __launch_bounds__(kStepThreads)
       const bool lines = legal_moves_t<true>(s, m, DeviceLB());
       const int nl = __popc(m[0]) + __popc(m[1]) + __popc(m[2]);
       const int result = terminal_result(nl, lines);
-      // select-only: compute the move for every state, keep it only where one exists
+      // compute the move for every state, keep it only where one exists
       // r % nl with nl <= 96: quotient estimate from floor(2^32 / nl) (one below at most), fix-up
       const uint32_t rnd = step_rnd(seed, (uint64_t)i), dv = (uint32_t)max(nl, 1);
       uint32_t rem = rnd - __umulhi(rnd, __ldg(d_inv32 + dv)) * dv;
@@ -48,113 +50,34 @@ __global__ void __launch_bounds__(kStepThreads)
                                      ((uint32_t)chosen << 16));
       next[i] = make_ulonglong2(o.w0, o.w1);
     }
-    if (kEncode) {
-      // warp-cooperative write of 32 x 70 contiguous floats (game.cpp:45-58 layout)
-      const int lane = threadIdx.x & 31;
-      ulonglong2 *ws = sm_states + (threadIdx.x & ~31);
-      ws[lane] = make_ulonglong2(s.w0, s.w1);
-      __syncwarp();
-      const int64_t base = i - lane;
-      const int64_t left = n - base;
-      const int cnt = left >= 32 ? 32 : (left > 0 ? (int)left : 0);
-      float *out = enc + base * CB200_STATE_SIZE;
-      for (int f = lane; f < cnt * CB200_STATE_SIZE; f += 32) {
-        const int si = f / CB200_STATE_SIZE, j = f - si * CB200_STATE_SIZE;
-        const ulonglong2 v = ws[si];
-        out[f] = encode_elem(CState{v.x, v.y}, j);
-      }
-      __syncwarp();
+    // warp-cooperative write of 32 x 70 contiguous floats (game.cpp:45-58 layout)
+    const int lane = threadIdx.x & 31;
+    ulonglong2 *ws = sm_states + (threadIdx.x & ~31);
+    ws[lane] = make_ulonglong2(s.w0, s.w1);
+    __syncwarp();
+    const int64_t base = i - lane;
+    const int64_t left = n - base;
+    const int cnt = left >= 32 ? 32 : (left > 0 ? (int)left : 0);
+    float *out = enc + base * CB200_STATE_SIZE;
+    for (int f = lane; f < cnt * CB200_STATE_SIZE; f += 32) {
+      const int si = f / CB200_STATE_SIZE, j = f - si * CB200_STATE_SIZE;
+      const ulonglong2 v = ws[si];
+      out[f] = encode_elem(CState{v.x, v.y}, j);
     }
+    __syncwarp();
   }
 }
 
-// K1, split form (no encoding requested). 85 % of reachable positions contain no line, and for
-// them the legal mask is the basic-rule mask; the line rules (category search, four table masks,
-// capital fix-ups) are ~60 % of the select-only instruction stream above. A CTA therefore runs
-//   phase A  every thread: basic mask + "any line?" test; positions without a line are finished
-//            at once, the others are queued in shared memory (state + index);
-//   phase B  whenever 256 positions are queued, every thread takes one and runs the full
-//            legal_moves_t on it -- dense warps on the expensive path instead of 5 live lanes.
-// Same outputs as k_game_step<false> (tests compare both with the oracle); stores of queued
-// positions are scattered 16-byte writes (15 % of the states).
-__device__ __forceinline__ void game_step_finish(int i, const CState &s, const uint32_t m[3], bool lines,
-                                                 uint64_t seed, uint4 *__restrict__ mask_flags,
-                                                 ulonglong2 *__restrict__ next) {
-  const int nl = __popc(m[0]) + __popc(m[1]) + __popc(m[2]);
-  const int result = terminal_result(nl, lines);
-  const uint32_t rnd = step_rnd(seed, (uint64_t)i), dv = (uint32_t)max(nl, 1);
-  uint32_t rem = rnd - __umulhi(rnd, __ldg(d_inv32 + dv)) * dv;
-  rem -= rem >= dv ? dv : 0u;
-  const int pick = nth_move(m, (int)rem);
-  const CState moved = do_move(s, pick & 127);
-  const int chosen = nl > 0 ? pick : 0x7f;
-  CState o;
-  o.w0 = nl > 0 ? moved.w0 : s.w0, o.w1 = nl > 0 ? moved.w1 : s.w1;
-  mask_flags[i] = make_uint4(m[0], m[1], m[2],
-                             (uint32_t)result | (lines ? 4u : 0u) | ((uint32_t)nl << 8) | ((uint32_t)chosen << 16));
-  next[i] = make_ulonglong2(o.w0, o.w1);
-}
-
-__global__ void __launch_bounds__(kStepThreads)
-    k_game_step_split(int64_t n, const ulonglong2 *__restrict__ states, uint64_t seed,
-                      uint4 *__restrict__ mask_flags, ulonglong2 *__restrict__ next) {
-  constexpr int kQueue = 2 * kStepThreads;  // fewer than 256 entries before a trip, at most 256 more
-  __shared__ ulonglong2 q_state[kQueue];
-  __shared__ int q_idx[kQueue];
-  __shared__ int q_n;
-  const int tid = threadIdx.x;
-  if (tid == 0) q_n = 0;
-  __syncthreads();
-  const unsigned stride = gridDim.x * kStepThreads;  // unsigned: the last `+= stride` cannot wrap
-  const unsigned n_round = (unsigned)(((n + kStepThreads - 1) / kStepThreads) * kStepThreads);  // uniform trip count per CTA
-  for (unsigned base = blockIdx.x * kStepThreads; base < n_round; base += stride) {
-    const int i = (int)(base + tid);
-    if (i < n) {
-      const ulonglong2 v = __ldg(states + i);
-      const CState s{v.x, v.y};
-      uint32_t m[3];
-      if (!basic_moves(s, m)) {
-        game_step_finish(i, s, m, false, seed, mask_flags, next);
-      } else {
-        // (a warp-aggregated append -- ballot + one atomic per warp -- measured 4 % slower: the
-        // ballot makes the whole warp wait for its slowest lane before the next trip's load)
-        const int slot = atomicAdd(&q_n, 1);
-        q_state[slot] = v, q_idx[slot] = i;
-      }
-    }
-    __syncthreads();
-    const int qn = q_n;
-    __syncthreads();  // every thread has read the count before the next trip's appends change it
-    if (qn >= kStepThreads) {  // CTA-uniform: one queued position per thread
-      const int e = qn - kStepThreads + tid;
-      const ulonglong2 v = q_state[e];
-      const CState s{v.x, v.y};
-      uint32_t m[3];
-      const bool lines = legal_moves_t<false>(s, m, DeviceLB());
-      game_step_finish(q_idx[e], s, m, lines, seed, mask_flags, next);
-      __syncthreads();
-      if (tid == 0) q_n = qn - kStepThreads;
-      __syncthreads();
-    }
-  }
-  for (int e = tid; e < q_n; e += kStepThreads) {  // drain
-    const ulonglong2 v = q_state[e];
-    const CState s{v.x, v.y};
-    uint32_t m[3];
-    const bool lines = legal_moves_t<false>(s, m, DeviceLB());
-    game_step_finish(q_idx[e], s, m, lines, seed, mask_flags, next);
-  }
-}
-
-// K1, paired form with one queue per CTA (CB200_K1_PAIR=2). The split idea above, with the integer-ALU
-// work per position cut further (the ALU pipe is what bounds K1, DESIGN.md section 4):
+// Paired form helpers. 85 % of reachable positions contain no line, and for them the legal mask
+// is the basic-rule mask; the line rules (category search, four table masks, capital fix-ups) are
+// ~60 % of the instruction stream of one position per thread without the encoding. The paired kernel cuts the
+// integer-ALU work per position (the ALU pipe is what bounds K1, DESIGN.md section 4):
 //   * a thread takes TWO positions per trip (i and i + 256: both loads and all stores stay
 //     coalesced) and runs the basic-rule mask and the "any line?" test on both at once, one
 //     position in each 16-bit half of every plane register (basic_moves_pair);
 //   * nth_move's last three levels and do_move's move decode are shared-memory tables
 //     (nth_move_lut / do_move_lut, 4.3 KB per CTA);
-//   * terminal positions (no legal move) skip the move instead of computing and discarding it.
-// Positions with a line are queued as in the split kernel and processed 256 at a time.
+//   * positions with a line are queued and finished later by full warps.
 struct SmemLB {
   const uint32_t *p;
   __device__ __forceinline__ const uint32_t *operator()(int idx) const { return p + 4 * idx; }
@@ -172,7 +95,7 @@ __device__ __forceinline__ void game_step_finish_lut(int i, const CState &s, con
                                                      const uint32_t *inv32) {
   const int nl = __popc(m[0]) + __popc(m[1]) + __popc(m[2]);
   const uint32_t rnd = step_rnd_mix(seed_c + (uint64_t)(uint32_t)i * 0x9E3779B97F4A7C15ull);
-  // rnd % nl as in game_step_finish; inv32[0] = 0 leaves a meaningless rem that nl == 0 never uses
+  // rnd % nl as in k_game_step_encode; inv32[0] = 0 leaves a meaningless rem that nl == 0 never uses
   const uint32_t dv = (uint32_t)nl;
   uint32_t rem = rnd - __umulhi(rnd, inv32[dv]) * dv;
   rem -= rem >= dv ? dv : 0u;
@@ -185,84 +108,6 @@ __device__ __forceinline__ void game_step_finish_lut(int i, const CState &s, con
   }
   mask_flags[i] = make_uint4(m[0], m[1], m[2], tail);
   next[i] = make_ulonglong2(o.w0, o.w1);
-}
-
-__global__ void __launch_bounds__(kStepThreads)
-    k_game_step_pair(int64_t n, const ulonglong2 *__restrict__ states, uint64_t seed,
-                     uint4 *__restrict__ mask_flags, ulonglong2 *__restrict__ next) {
-  constexpr int kQueue = 3 * kStepThreads;  // fewer than 256 entries before a trip, at most 512 more
-  __shared__ ulonglong2 q_state[kQueue];
-  __shared__ uint4 q_mask[kQueue];  // basic-rule mask (x, y, z) and the position's index (w)
-  __shared__ int q_n;
-  __shared__ __align__(16) uint32_t s_move[96 * kMoveLutWords];
-  __shared__ __align__(16) uint8_t s_nth[256 * 8];
-  __shared__ uint32_t s_inv[128];
-  const int tid = threadIdx.x;
-  reinterpret_cast<uint2 *>(s_nth)[tid] = reinterpret_cast<const uint2 *>(d_nth_lut)[tid];
-  if (tid < 128) s_inv[tid] = d_inv32[tid];
-  if (tid < 96 * kMoveLutWords / 4)
-    reinterpret_cast<uint4 *>(s_move)[tid] = reinterpret_cast<const uint4 *>(d_move_lut)[tid];
-  if (tid == 0) q_n = 0;
-  __syncthreads();
-  const uint32_t *ML = s_move;
-  const SmemNthLut NL{s_nth};
-  const uint64_t seed_c = seed + 0x9E3779B97F4A7C15ull;
-  constexpr int kTrip = 2 * kStepThreads;
-  const unsigned stride = gridDim.x * kTrip;  // unsigned: the last `+= stride` cannot wrap
-  const unsigned n_round = (unsigned)(((n + kTrip - 1) / kTrip) * kTrip);  // uniform trip count per CTA
-  for (unsigned base = blockIdx.x * kTrip; base < n_round; base += stride) {
-    const unsigned ua = base + tid, ub = ua + kStepThreads;
-    if (ua < (unsigned)n) {
-      const bool hb = ub < (unsigned)n;
-      const int ia = (int)ua, ib = (int)ub;
-      const ulonglong2 va = __ldg(states + ia);
-      const ulonglong2 vb = hb ? __ldg(states + ib) : va;
-      const CState a{va.x, va.y}, b{vb.x, vb.y};
-      uint32_t ma[3], mb[3];
-      bool la, lb;
-      basic_moves_pair(a, b, ma, mb, la, lb);
-      if (!la) {
-        game_step_finish_lut(ia, a, ma, false, seed_c, mask_flags, next, ML, NL, s_inv);
-      } else {
-        const int slot = atomicAdd(&q_n, 1);
-        q_state[slot] = va, q_mask[slot] = make_uint4(ma[0], ma[1], ma[2], (uint32_t)ia);
-      }
-      if (hb) {
-        if (!lb) {
-          game_step_finish_lut(ib, b, mb, false, seed_c, mask_flags, next, ML, NL, s_inv);
-        } else {
-          const int slot = atomicAdd(&q_n, 1);
-          q_state[slot] = vb, q_mask[slot] = make_uint4(mb[0], mb[1], mb[2], (uint32_t)ib);
-        }
-      }
-    }
-    __syncthreads();
-    int qn = q_n;
-    __syncthreads();  // every thread has read the count before the next appends change it
-    if (qn >= kStepThreads) {  // CTA-uniform
-      do {
-        const int e = qn - kStepThreads + tid;
-        const ulonglong2 v = q_state[e];
-        const uint4 qm = q_mask[e];
-        const CState s{v.x, v.y};
-        uint32_t m[3] = {qm.x, qm.y, qm.z};
-        const bool lines = line_rules_on_basic(s, m, DeviceLB());
-        game_step_finish_lut((int)qm.w, s, m, lines, seed_c, mask_flags, next, ML, NL, s_inv);
-        qn -= kStepThreads;
-      } while (qn >= kStepThreads);
-      __syncthreads();
-      if (tid == 0) q_n = qn;
-      __syncthreads();
-    }
-  }
-  for (int e = tid; e < q_n; e += kStepThreads) {  // drain
-    const ulonglong2 v = q_state[e];
-    const uint4 qm = q_mask[e];
-    const CState s{v.x, v.y};
-    uint32_t m[3] = {qm.x, qm.y, qm.z};
-    const bool lines = line_rules_on_basic(s, m, DeviceLB());
-    game_step_finish_lut((int)qm.w, s, m, lines, seed_c, mask_flags, next, ML, NL, s_inv);
-  }
 }
 
 // Both positions of a thread finished together, without a branch: the two dependent chains
@@ -286,17 +131,17 @@ __device__ __forceinline__ void game_step_finish_one_sel(const CState &s, const 
   tail = any ? (((uint32_t)nl << 8) | ((uint32_t)pick << 16)) : ((uint32_t)kResultDraw | (0x7fu << 16));
 }
 
-// K1, paired form with one queue per WARP (the default, with kPrefetch and kJoint). k_game_step_pair above synchronises the
-// CTA twice per trip: its ncu capture shows the warps of a CTA waiting together for their loads
-// right after the barrier (long-scoreboard 7.2, barrier 2.5 stall cycles per issue, issue slots
-// 66 % busy). Here every warp owns a queue of 96 entries and a warp-uniform count in a register:
+// K1, paired form with one queue per WARP. A single queue per CTA synchronises the CTA twice per
+// trip: its ncu capture showed the warps of a CTA waiting together for their loads right after the
+// barrier (long-scoreboard 7.2, barrier 2.5 stall cycles per issue, issue slots 66 % busy). Here
+// every warp owns a queue of 96 entries and a warp-uniform count in a register:
 //   * appending is two ballots and predicated stores (no atomics, no branch: the warp is still
 //     converged right after basic_moves_pair);
 //   * a warp flushes 32 queued positions whenever it has them -- __syncwarp only, no __syncthreads
 //     inside the loop, so the 56 warps of an SM drift apart and cover each other's load latency;
-//   * kPrefetch: the next trip's two positions are requested before the current ones are processed.
-template <bool kPrefetch, int kMinBlocks, bool kJoint = false>
-__global__ void __launch_bounds__(kStepThreads, kMinBlocks)
+//   * the next trip's two positions are requested before the current ones are processed;
+//   * the positions without a line are finished by game_step_finish_one_sel, both at once.
+__global__ void __launch_bounds__(kStepThreads, 1)
     k_game_step_pairw(int64_t n, const ulonglong2 *__restrict__ states, uint64_t seed,
                       uint4 *__restrict__ mask_flags, ulonglong2 *__restrict__ next) {
   constexpr int kWarps = kStepThreads / 32;
@@ -329,23 +174,17 @@ __global__ void __launch_bounds__(kStepThreads, kMinBlocks)
   const ulonglong2 none = make_ulonglong2(0ull, 0ull);  // empty board, no pieces: no move, no line
   unsigned base = blockIdx.x * kTrip;
   ulonglong2 pa = none, pb = none;
-  if (kPrefetch && base < n_round) {
+  if (base < n_round) {
     if (base + tid < un) pa = __ldg(states + base + tid);
     if (base + tid + kStepThreads < un) pb = __ldg(states + base + tid + kStepThreads);
   }
   for (; base < n_round; base += stride) {
     const unsigned ua = base + tid, ub = ua + kStepThreads;
     const bool ha = ua < un, hb = ub < un;
-    ulonglong2 va, vb;
-    if (kPrefetch) {
-      va = pa, vb = pb;
-      const unsigned na = ua + stride, nb = ub + stride;  // past n_round means past n
-      pa = na < un ? __ldg(states + na) : none;
-      pb = nb < un ? __ldg(states + nb) : none;
-    } else {
-      va = ha ? __ldg(states + ua) : none;
-      vb = hb ? __ldg(states + ub) : none;
-    }
+    const ulonglong2 va = pa, vb = pb;
+    const unsigned na = ua + stride, nb = ub + stride;  // past n_round means past n
+    pa = na < un ? __ldg(states + na) : none;
+    pb = nb < un ? __ldg(states + nb) : none;
     const CState a{va.x, va.y}, b{vb.x, vb.y};
     uint32_t ma[3], mb[3];
     bool la, lb;
@@ -362,22 +201,17 @@ __global__ void __launch_bounds__(kStepThreads, kMinBlocks)
       qs[slot] = vb, qm[slot] = make_uint4(mb[0], mb[1], mb[2], ub);
     }
     qn += __popc(bb);
-    if (kJoint) {
-      uint32_t ta, tb;
-      CState oa, ob;
-      game_step_finish_one_sel(a, ma, ua, seed_c, ML, NL, s_inv, ta, oa);
-      game_step_finish_one_sel(b, mb, ub, seed_c, ML, NL, s_inv, tb, ob);
-      if (ha && !la) {
-        mask_flags[ua] = make_uint4(ma[0], ma[1], ma[2], ta);
-        next[ua] = make_ulonglong2(oa.w0, oa.w1);
-      }
-      if (hb && !lb) {
-        mask_flags[ub] = make_uint4(mb[0], mb[1], mb[2], tb);
-        next[ub] = make_ulonglong2(ob.w0, ob.w1);
-      }
-    } else {
-      if (ha && !la) game_step_finish_lut((int)ua, a, ma, false, seed_c, mask_flags, next, ML, NL, s_inv);
-      if (hb && !lb) game_step_finish_lut((int)ub, b, mb, false, seed_c, mask_flags, next, ML, NL, s_inv);
+    uint32_t ta, tb;
+    CState oa, ob;
+    game_step_finish_one_sel(a, ma, ua, seed_c, ML, NL, s_inv, ta, oa);
+    game_step_finish_one_sel(b, mb, ub, seed_c, ML, NL, s_inv, tb, ob);
+    if (ha && !la) {
+      mask_flags[ua] = make_uint4(ma[0], ma[1], ma[2], ta);
+      next[ua] = make_ulonglong2(oa.w0, oa.w1);
+    }
+    if (hb && !lb) {
+      mask_flags[ub] = make_uint4(mb[0], mb[1], mb[2], tb);
+      next[ub] = make_ulonglong2(ob.w0, ob.w1);
     }
     __syncwarp();  // the appended entries are visible to the whole warp
     while (qn >= 32) {  // warp-uniform
@@ -413,27 +247,15 @@ __global__ void __launch_bounds__(kStepThreads, kMinBlocks)
   }
 }
 
-// resident CTAs of a paired kernel per SM (register- and shared-memory-limited), asked once per form
-typedef void (*K1PairFn)(int64_t, const ulonglong2 *, uint64_t, uint4 *, ulonglong2 *);
-inline K1PairFn k1_pair_kernel(int form) {
-  switch (form) {
-    case 1: return k_game_step_pairw<true, 1>;
-    case 2: return k_game_step_pair;
-    case 3: return k_game_step_pairw<false, 7>;
-    case 4: return k_game_step_pairw<true, 6>;
-    case 5: return k_game_step_pairw<false, 1, true>;
-    case 6: return k_game_step_pairw<true, 1, true>;
-    default: return k_game_step_pairw<false, 1>;
-  }
-}
-inline int k1_pair_ctas_per_sm(int form) {
-  static int ctas[7] = {0, 0, 0, 0, 0, 0, 0};
-  if (ctas[form] == 0) {
+// resident CTAs of the paired kernel per SM (register- and shared-memory-limited), asked once
+inline int k1_pair_ctas_per_sm() {
+  static int ctas = 0;
+  if (ctas == 0) {
     int v = 0;
-    const cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&v, k1_pair_kernel(form), kStepThreads, 0);
-    ctas[form] = e == cudaSuccess && v >= 1 ? v : 4;
+    const cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&v, k_game_step_pairw, kStepThreads, 0);
+    ctas = e == cudaSuccess && v >= 1 ? v : 4;
   }
-  return ctas[form];
+  return ctas;
 }
 
 inline int launch_game_step(int64_t n, const void *d_states, uint64_t seed, void *d_mask_flags,
@@ -445,33 +267,20 @@ inline int launch_game_step(int64_t n, const void *d_states, uint64_t seed, void
   int dev = 0, sms = 148;
   cudaGetDevice(&dev);
   cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-  // persistent-style grid: a multiple of the SM count, 8 resident CTAs of 256 threads per SM
-  int64_t want = (n + kStepThreads - 1) / kStepThreads;
-  int64_t cap = (int64_t)sms * 8 * 4;
-  int grid = (int)(want < cap ? want : cap);
-  if (d_enc)
-    k_game_step<true><<<grid, kStepThreads, 0, cur_stream()>>>(
+  if (d_enc) {
+    // persistent-style grid: a multiple of the SM count, 8 resident CTAs of 256 threads per SM
+    const int64_t want = (n + kStepThreads - 1) / kStepThreads;
+    const int64_t cap = (int64_t)sms * 8 * 4;
+    const int grid = (int)(want < cap ? want : cap);
+    k_game_step_encode<<<grid, kStepThreads, 0, cur_stream()>>>(
         n, (const ulonglong2 *)d_states, seed, (uint4 *)d_mask_flags, (ulonglong2 *)d_next,
         (float *)d_enc);
-  else if (getenv("CB200_K1_SELECT_ONLY"))  // the round-1 kernel, kept for comparison
-    k_game_step<false><<<grid, kStepThreads, 0, cur_stream()>>>(
-        n, (const ulonglong2 *)d_states, seed, (uint4 *)d_mask_flags, (ulonglong2 *)d_next,
-        nullptr);
-  else if (getenv("CB200_K1_SPLIT"))  // one position per thread (the form before the paired kernel)
-    k_game_step_split<<<grid, kStepThreads, 0, cur_stream()>>>(
-        n, (const ulonglong2 *)d_states, seed, (uint4 *)d_mask_flags, (ulonglong2 *)d_next);
-  else {
-    // a few waves of CTAs, each looping over its share (CB200_K1_WAVES: sweep knob, default 8).
-    // CB200_K1_PAIR: 0 = queue per warp, 1 = the same with prefetch, 2 = queue per CTA,
-    // 3 / 4 = forms 0 / 1 compiled for 7 / 6 resident CTAs per SM, 5 / 6 = forms 0 / 1 with both positions of a
-    // thread finished together, branch-free (6 is the default)
-    const char *wv = getenv("CB200_K1_WAVES"), *fv = getenv("CB200_K1_PAIR");
-    const int waves = wv && atoi(wv) > 0 ? atoi(wv) : 8;
-    const int form = fv && atoi(fv) >= 0 && atoi(fv) <= 6 ? atoi(fv) : 6;
-    const int64_t want2 = (n + 2 * kStepThreads - 1) / (2 * kStepThreads);
-    const int64_t cap2 = (int64_t)sms * k1_pair_ctas_per_sm(form) * waves;
-    const int grid2 = (int)(want2 < cap2 ? want2 : cap2);
-    k1_pair_kernel(form)<<<grid2, kStepThreads, 0, cur_stream()>>>(
+  } else {
+    // 8 waves of CTAs, each looping over its share
+    const int64_t want = (n + 2 * kStepThreads - 1) / (2 * kStepThreads);
+    const int64_t cap = (int64_t)sms * k1_pair_ctas_per_sm() * 8;
+    const int grid = (int)(want < cap ? want : cap);
+    k_game_step_pairw<<<grid, kStepThreads, 0, cur_stream()>>>(
         n, (const ulonglong2 *)d_states, seed, (uint4 *)d_mask_flags, (ulonglong2 *)d_next);
   }
   CB_LAUNCHED();

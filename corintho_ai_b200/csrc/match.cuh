@@ -67,7 +67,6 @@ __global__ void __launch_bounds__(kTreeWarps * 32, 4)
   if (!match_selected(ctl, sides, model_id)) return;
   WarpSm &sm = sm_all[warp];
   Ctx c;
-  c.bind_lanes();
   c.to_play = ctl[CW_TO_PLAY], c.parity = 0, c.result = ctl[CW_RESULT];
   c.mate_turn = 0, c.n_samples = 0;
   c.n_pending = ctl[CW_N_PENDING], c.error = ctl[CW_ERROR], c.spare = ctl[CW_SPARE];

@@ -4,7 +4,7 @@
 // busy, but each launch lasts as long as its slowest game and every iteration pays two kernel
 // boundaries. Once all live games fit on the GPU at 16 games per SM, one CTA per SM takes 8 or 16
 // games and loops by itself:
-//     game step of its games (kGameLanes lanes each: run_game = SelfPlayer::doIteration)
+//     game step of its games (one warp each: run_game = SelfPlayer::doIteration)
 //  -> the tensor-core network on the <= 128 / 256 leaf positions they queued (tc_forward)
 // without leaving the SM, so a CTA only ever waits for its own games. Requests and answers
 // travel through CTA-private rows of small global buffers (L2 resident). Per-game order of
@@ -44,16 +44,15 @@ __global__ void k_live_list(TreeParams P, int32_t *__restrict__ list, int32_t *_
   if (lane == 0) *count = n;
 }
 
-// kGames = 8 (one network tile) or 16 (two tiles) games per CTA, each run by kL lanes (kL = 32:
-// 256 / 512 threads, the network is run by the first 256 or -- a single tile -- 128 of them;
-// kL = 16: 128 / 256 threads). Games are dealt
+// kGames = 8 (one network tile) or 16 (two tiles) games per CTA, one warp each (256 / 512
+// threads; the network is run by the first 256 or -- a single tile -- 128 of them). Games are dealt
 // round-robin over the CTAs (slot = group * gridDim.x + blockIdx.x) so that every SM gets its share
 // however few games are left. All CTAs stop at their next round boundary once `exit_done` games of
 // this launch have finished (the host then deals the remaining games again). out[0] += games still
 // live when the CTA stopped, out[1] = min error code, out[2] = max rounds executed by a CTA,
 // out[3] = games finished during the launch.
-template <int kMode, int kGames, int kL>
-__global__ void __launch_bounds__(kGames * kL, 1)
+template <int kMode, int kGames>
+__global__ void __launch_bounds__(kGames * 32, 1)
     k_selfplay_persistent(TreeParams P, const uint8_t *__restrict__ W,
                           const uint8_t *__restrict__ W1, const int32_t *__restrict__ game_list,
                           int n_list, const float *eval0, const float *probs0, long pcs0,
@@ -62,7 +61,7 @@ __global__ void __launch_bounds__(kGames * kL, 1)
   static_assert(kGames == 8 || kGames == 16, "one or two network tiles per CTA");
   static_assert(ps_smem_bytes<kMode, kGames>() <= 227 * 1024, "bf16x3 fits with 8 games per CTA only");
   constexpr int kNetThreads = kGames == 8 ? 128 : kTcThreads;  // one tile or two
-  static_assert(kGames * kL >= kNetThreads, "too few threads for the network");
+  static_assert(kGames * 32 >= kNetThreads, "too few threads for the network");
   const bool net_thread = threadIdx.x < kNetThreads;
   constexpr int kRows = kGames * kPsRowsPerGame;
   extern __shared__ __align__(128) uint8_t smem[];
@@ -73,7 +72,7 @@ __global__ void __launch_bounds__(kGames * kL, 1)
   TcState S;
   if (net_thread) tc_setup(S, smem, kNetThreads, kMode == 2 ? 2 : 1);
   WarpSm *sm_all = reinterpret_cast<WarpSm *>(smem + ps_tree_smem_off<kMode, kGames>());
-  const int grp = threadIdx.x / kL;
+  const int grp = threadIdx.x / 32;
   const int slot = grp * gridDim.x + blockIdx.x;
   const int g = slot < n_list ? game_list[slot] : -1;
   const int row0 = blockIdx.x * kRows * (two ? 2 : 1);
@@ -88,9 +87,9 @@ __global__ void __launch_bounds__(kGames * kL, 1)
     __syncthreads();
     if (g >= 0) {
       const bool ext = round == 0;  // answers of the requests queued before this launch
-      run_game<true, kL>(P, g, sm_all[grp], ext ? eval0 : eval, ext ? probs0 : probs, 1,
-                         ext ? pcs0 : (long)ld, nullptr, -1, iteration0 + round, 0, &s_ctr[0],
-                         &s_ctr[1], &s_ctr[2], row0, packed, two ? kRows : 0);
+      run_game<true>(P, g, sm_all[grp], ext ? eval0 : eval, ext ? probs0 : probs, 1,
+                     ext ? pcs0 : (long)ld, nullptr, -1, iteration0 + round, 0, &s_ctr[0],
+                     &s_ctr[1], &s_ctr[2], row0, packed, two ? kRows : 0);
     }
     __syncthreads();
     const int n = s_ctr[0], n1 = s_ctr[4];

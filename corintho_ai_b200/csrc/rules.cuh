@@ -242,7 +242,7 @@ CB_HD int nth_move(const uint32_t m[3], int k) {
   return base;
 }
 
-// ---- K1 fast-path forms (game_step.cuh, k_game_step_pair). Same results as basic_moves /
+// ---- K1 fast-path forms (game_step.cuh, k_game_step_pairw). Same results as basic_moves /
 // nth_move / do_move above (tests/host_shim checks them against each other on the host and the
 // GPU tests against the oracle); written for the integer-ALU pipe, which bounds K1:
 //   * two positions per thread share every plane operation (16-bit planes of position a in the

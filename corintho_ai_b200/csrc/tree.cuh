@@ -1,5 +1,4 @@
-// K2-K6: the self-play game step -- a group of kL lanes (kL = 32: one warp per game, the
-// default; kL = 16: two games per warp, CB200_LANES=16) owns one game and executes
+// K2-K6: the self-play game step -- one warp per game executes
 // SelfPlayer::doIteration (corintho_ai/cpp/src/selfplayer.cpp:115-122) for it:
 //   eval ingest + backup   TrainMC::receiveEval      trainmc.cpp:269-296 (212-267)
 //   PUCT select / expand   TrainMC::search           trainmc.cpp:602-696 (chooseNext 540-600)
@@ -15,14 +14,10 @@
 //                 move | prior<<7 | result<<16 | all_visited<<19 | has_child<<20 |
 //                 child_n_legal<<21 | child_has_children<<28}
 // A node's statistics live in its parent's slot, so PUCT selection at a node is ONE coalesced
-// read of header+slots (lane e loads slots e, e + kL, ... as uint4) and virtual loss is a plain store.
-// With kL = 16 the two games of a warp run the same code under their own lane masks (every
-// collective below takes the group mask): scalar work (rules, control flow) is replicated 16x
-// instead of 32x and the code is shaped so that both halves stay converged (expansion after the
-// select loop, MT19937 words regenerated where they are drawn instead of in a 624-word twist at
-// data-dependent times). Measured on B200 (DESIGN.md section 8): 19 % fewer warp instructions per
-// game step but a 1.6x longer dependent chain per warp, and the step is bound by that chain, not
-// by issue slots -- so one warp per game stays the default.
+// read of header+slots (lane e loads slots e, e + 32, ... as uint4) and virtual loss is a plain store.
+// Two games per warp (16 lanes each) were measured on a B200 and were slower: fewer warp
+// instructions per game step, but a longer dependent chain per game, and the step is bound by
+// that chain (DESIGN.md section 8).
 // The root record is at word root_off (re-rooting is in place; the kept subtree is compacted
 // into the spare arena only when room runs out); root statistics are in the per-tree control
 // block. The per-game context (Ctx) lives in registers: every device function below is
@@ -53,8 +48,7 @@ constexpr int kMaxPath = 64;
 constexpr int kPendWords = 2 + kMaxPath;  // leaf_off, path_len, path[kMaxPath]
 constexpr int kMaxSamples = 64;
 constexpr int kVsqrtCap = 2048;  // entries of the c_puct*sqrt(visits) table
-constexpr int kTreeWarps = 4;    // warps per CTA of the lock-step kernels: 4 * (32 / kL) games
-constexpr int kGameLanes = 32;   // default lanes per self-play game (16 = two games per warp)
+constexpr int kTreeWarps = 4;    // warps (= games) per CTA of the lock-step kernels
 constexpr int kCtlWords = 20;  // CW_* below; words 12-16 belong to Match (match.cuh)
 constexpr int kTreeCtlWords = 12;
 
@@ -109,7 +103,7 @@ struct TreeParams {
 };
 
 constexpr int kFlatCap = 448;  // legal-move slots processed per flat ingest chunk
-// per-game scratch in shared memory (one per lane group)
+// per-game scratch in shared memory (one per warp)
 struct WarpSm {
   __align__(16) float f[100];
   uint32_t node[kMaxPath + 1];
@@ -163,13 +157,9 @@ __device__ __forceinline__ double fast_rcp(double x) {
   return r;
 }
 
-// Per-group view of one game. Every member is uniform over the group's kL lanes.
-template <int kL>
-struct CtxT {
-  static constexpr int L = kL;
-  int lane;        // lane within the group, 0 .. kL-1
-  unsigned gmask;  // the group's lanes within the warp (all 32 for kL = 32)
-  int lshift;      // warp lane of the group's lane 0
+// Per-warp view of one game. Every member except lane is uniform over the warp.
+struct Ctx {
+  int lane = threadIdx.x & 31;
   // game control (selfplayer.h:88-111)
   int to_play, parity, result, mate_turn, n_samples, n_pending, error, spare, mt_idx;
   int d_sims, d_evals, d_moves, d_searches;  // work done in this launch (< 2^31 by far)
@@ -190,63 +180,34 @@ struct CtxT {
   int32_t *tree_ctl;
   ulonglong2 *leaf_state, *sample_state;
   float *sample_probs;
-
-  __device__ __forceinline__ void bind_lanes() {
-    const int wl = threadIdx.x & 31;
-    lane = wl & (kL - 1);
-    lshift = wl & ~(kL - 1);
-    gmask = kL == 32 ? kFull : (((1u << (kL & 31)) - 1u) << lshift);
-  }
 };
-using Ctx = CtxT<32>;  // one warp per game / match (match.cuh)
 
-// ---- collectives over the lanes of one game --------------------------------------------------
-// Lane indices, ballot bits and shuffle sources are relative to the group.
-template <class C> __device__ __forceinline__ unsigned g_mask(const C &c) {
-  if constexpr (C::L == 32) return kFull;
-  else return c.gmask;
+// ---- collectives over the warp of one game ---------------------------------------------------
+__device__ __forceinline__ void g_sync(const Ctx &) { __syncwarp(kFull); }
+__device__ __forceinline__ unsigned g_ballot(const Ctx &, bool p) { return __ballot_sync(kFull, p); }
+__device__ __forceinline__ bool g_all(const Ctx &, bool p) { return __all_sync(kFull, p); }
+template <class T> __device__ __forceinline__ T g_shfl(const Ctx &, T v, int src) {
+  return __shfl_sync(kFull, v, src);
 }
-template <class C> __device__ __forceinline__ void g_sync(const C &c) { __syncwarp(g_mask(c)); }
-template <class C> __device__ __forceinline__ unsigned g_ballot(const C &c, bool p) {
-  if constexpr (C::L == 32) return __ballot_sync(kFull, p);
-  else return (__ballot_sync(c.gmask, p) >> c.lshift) & ((1u << C::L) - 1u);
+template <class T> __device__ __forceinline__ T g_shfl_up(const Ctx &, T v, int d) {
+  return __shfl_up_sync(kFull, v, d);
 }
-template <class C> __device__ __forceinline__ bool g_all(const C &c, bool p) {
-  return __all_sync(g_mask(c), p);
-}
-template <class C, class T> __device__ __forceinline__ T g_shfl(const C &c, T v, int src) {
-  return __shfl_sync(g_mask(c), v, src, C::L);
-}
-template <class C, class T> __device__ __forceinline__ T g_shfl_up(const C &c, T v, int d) {
-  return __shfl_up_sync(g_mask(c), v, d, C::L);
-}
-template <class C> __device__ __forceinline__ int g_max(const C &c, int v) {
-  return __reduce_max_sync(g_mask(c), v);
-}
-template <class C> __device__ __forceinline__ uint32_t g_max(const C &c, uint32_t v) {
-  return __reduce_max_sync(g_mask(c), v);
-}
-template <class C> __device__ __forceinline__ int g_min(const C &c, int v) {
-  return __reduce_min_sync(g_mask(c), v);
-}
-template <class C> __device__ __forceinline__ int g_add(const C &c, int v) {
-  return __reduce_add_sync(g_mask(c), v);
-}
-template <class C> __device__ __forceinline__ unsigned g_match(const C &c, uint32_t v) {
-  if constexpr (C::L == 32) return __match_any_sync(kFull, v);
-  else return (__match_any_sync(c.gmask, v) >> c.lshift) & ((1u << C::L) - 1u);
-}
+__device__ __forceinline__ int g_max(const Ctx &, int v) { return __reduce_max_sync(kFull, v); }
+__device__ __forceinline__ uint32_t g_max(const Ctx &, uint32_t v) { return __reduce_max_sync(kFull, v); }
+__device__ __forceinline__ int g_min(const Ctx &, int v) { return __reduce_min_sync(kFull, v); }
+__device__ __forceinline__ int g_add(const Ctx &, int v) { return __reduce_add_sync(kFull, v); }
+__device__ __forceinline__ unsigned g_match(const Ctx &, uint32_t v) { return __match_any_sync(kFull, v); }
 
-template <class C> __device__ __forceinline__ uint32_t g_incl_scan(const C &c, uint32_t v) {
+__device__ __forceinline__ uint32_t g_incl_scan(const Ctx &c, uint32_t v) {
 #pragma unroll
-  for (int d = 1; d < C::L; d <<= 1) {
+  for (int d = 1; d < 32; d <<= 1) {
     const uint32_t o = g_shfl_up(c, v, d);
     if (c.lane >= d) v += o;
   }
   return v;
 }
 
-template <class C> __device__ __forceinline__ void load_tree(C &c, const TreeParams &P, int p) {
+__device__ __forceinline__ void load_tree(Ctx &c, const TreeParams &P, int p) {
   const int32_t *t = c.tree_ctl + p * kTreeCtlWords;
   const int4 a = *reinterpret_cast<const int4 *>(t);
   const int4 b = *reinterpret_cast<const int4 *>(t + 4);
@@ -256,7 +217,7 @@ template <class C> __device__ __forceinline__ void load_tree(C &c, const TreePar
   c.root_off = (uint32_t)t[TW_ROOT_OFF];
   c.base = c.arenas + (size_t)c.arena * P.arena_words;
 }
-template <class C> __device__ __forceinline__ void store_tree(C &c) {
+__device__ __forceinline__ void store_tree(Ctx &c) {
   if (c.lane == 0) {
     int32_t *t = c.tree_ctl + c.cur_p * kTreeCtlWords;
     *reinterpret_cast<int4 *>(t) =
@@ -274,8 +235,9 @@ template <class C> __device__ __forceinline__ void store_tree(C &c) {
 // computed right before it is drawn. Going through the ring in order this is exactly
 // std::mt19937's block twist (positions below p already hold the new generation, which is what
 // new[p] needs for p >= 227 and for p = 623), but the work is spread evenly over the draws
-// instead of arriving as one 624-word twist at a data-dependent time -- the two games of a warp
-// then draw in step. mt_idx = position of the next word (624 = wrap to 0 first).
+// instead of arriving as one 624-word twist at a data-dependent time (1 670 -> 570 warp
+// instructions per game iteration, DESIGN.md section 8). mt_idx = position of the next word
+// (624 = wrap to 0 first).
 __device__ __forceinline__ uint32_t mt_temper(uint32_t y) {
   y ^= y >> 11;
   y ^= (y << 7) & 0x9d2c5680u;
@@ -289,7 +251,7 @@ __device__ __forceinline__ uint32_t mt_next_word(const uint32_t *mt, int p) {
   const uint32_t y = (a & 0x80000000u) | (b & 0x7fffffffu);
   return m ^ (y >> 1) ^ ((y & 1u) ? 0x9908b0dfu : 0u);
 }
-template <class C> __device__ __forceinline__ uint32_t rng_one(C &c) {
+__device__ __forceinline__ uint32_t rng_one(Ctx &c) {
   if (c.mt_idx >= 624) c.mt_idx = 0;
   const uint32_t w = mt_next_word(c.mt, c.mt_idx);  // every lane reads the same three words
   g_sync(c);
@@ -300,15 +262,14 @@ template <class C> __device__ __forceinline__ uint32_t rng_one(C &c) {
 }
 
 __device__ __forceinline__ void copy_words(uint32_t *dst, const uint32_t *src, uint32_t nwords,
-                                           int lane, int lanes) {
+                                           int lane) {
   const uint4 *s = reinterpret_cast<const uint4 *>(src);
   uint4 *d = reinterpret_cast<uint4 *>(dst);
-  for (uint32_t i = lane; i < (nwords >> 2); i += lanes) d[i] = s[i];
+  for (uint32_t i = lane; i < (nwords >> 2); i += 32) d[i] = s[i];
 }
 
 // ---- node construction (Node ctor + initializeEdges, node.cpp:31-39, 256-283) ---------------
-template <class C>
-__device__ __forceinline__ int make_record(C &c, const TreeParams &P, const CState &st,
+__device__ __forceinline__ int make_record(Ctx &c, const TreeParams &P, const CState &st,
                                            int depth, int &result) {
   uint32_t m[3];
   const bool lines = legal_moves(st, m, DeviceLB());
@@ -326,17 +287,14 @@ __device__ __forceinline__ int make_record(C &c, const TreeParams &P, const CSta
                       (uint32_t)(st.w1 >> 32)));
     st4(r + 4, make_uint4((uint32_t)n | ((uint32_t)depth << 8), 0u, 0u, 0u));
   }
-  // slot of move id b = rank of bit b among the legal moves; lane l writes ids l, l + kL, ...
+  // slot of move id b = rank of bit b among the legal moves; lane l writes ids l, l + 32, l + 64
 #pragma unroll
   for (int w = 0; w < 3; ++w) {
     const int pre = w == 0 ? 0 : (w == 1 ? n0 : n0 + n1);
-#pragma unroll
-    for (int h = 0; h < 32 / C::L; ++h) {
-      const int b = c.lane + C::L * h;
-      if ((m[w] >> b) & 1u)
-        st4(r + 8 + 4 * (pre + __popc(m[w] & ((1u << b) - 1u))),
-            make_uint4(0u, 0u, 0u, (uint32_t)(32 * w + b)));
-    }
+    const int b = c.lane;
+    if ((m[w] >> b) & 1u)
+      st4(r + 8 + 4 * (pre + __popc(m[w] & ((1u << b) - 1u))),
+          make_uint4(0u, 0u, 0u, (uint32_t)(32 * w + b)));
   }
   c.used = off + 8u + 4u * (uint32_t)n;
   result = terminal_result(n, lines);
@@ -353,8 +311,7 @@ __device__ __forceinline__ CState rec_state(const uint32_t *r) {
 }
 
 // Single-node tree (Node(game, depth) node.cpp:25-29; reset paths trainmc.cpp:397-404,461-468)
-template <class C>
-__device__ __forceinline__ void fresh_tree(C &c, const TreeParams &P, const CState &st,
+__device__ __forceinline__ void fresh_tree(Ctx &c, const TreeParams &P, const CState &st,
                                            int depth) {
   c.used = 0;
   c.root_off = 0;
@@ -368,7 +325,7 @@ __device__ __forceinline__ void fresh_tree(C &c, const TreeParams &P, const CSta
 }
 
 // queue the root for evaluation (trainmc.cpp:150-152, 160-162, 198-200)
-template <class C> __device__ __forceinline__ void request_root(C &c) {
+__device__ __forceinline__ void request_root(Ctx &c) {
   if (c.lane == 0) {
     uint32_t *pd = c.pending + c.n_pending * kPendWords;
     const uint4 h = ld4(c.base + c.root_off);
@@ -383,9 +340,7 @@ template <class C> __device__ __forceinline__ void request_root(C &c) {
 // ---- TrainMC::moveDown (trainmc.cpp:475-495): child behind root slot e becomes the root -----
 // Breadth-first copy of the kept subtree into the spare arena; only records that have
 // children are queued for scanning (queue grows down from the top of the target arena).
-template <class C>
-__device__ __forceinline__ void move_down(C &c, const TreeParams &P, int e) {
-  constexpr int kL = C::L;
+__device__ __forceinline__ void move_down(Ctx &c, const TreeParams &P, int e) {
   const uint32_t *src = c.base;
   uint32_t *dst = c.arenas + (size_t)c.spare * P.arena_words;
   const uint4 s = ld4(src + c.root_off + 8 + 4 * e);
@@ -403,7 +358,7 @@ __device__ __forceinline__ void move_down(C &c, const TreeParams &P, int e) {
     return;
   }
   const uint32_t sz = 8u + 4u * (uint32_t)s3_cnl(s.w);
-  copy_words(dst, src + s.z, sz, c.lane, kL);
+  copy_words(dst, src + s.z, sz, c.lane);
   uint32_t alloc = sz;
   int q_head = 0, q_tail = 0;
   uint32_t *q = dst + (P.arena_words - 1);
@@ -418,7 +373,7 @@ __device__ __forceinline__ void move_down(C &c, const TreeParams &P, int e) {
     ++q_head;
     uint32_t *r = dst + roff;
     const int rn = (int)(r[4] & 0xffu);
-    for (int e0 = 0; e0 < rn; e0 += kL) {
+    for (int e0 = 0; e0 < rn; e0 += 32) {
       const int ee = e0 + c.lane;
       bool has = false, gc = false;
       uint32_t coff = 0, csz = 0;
@@ -429,7 +384,7 @@ __device__ __forceinline__ void move_down(C &c, const TreeParams &P, int e) {
       }
       const uint32_t incl = g_incl_scan(c, csz);
       const uint32_t excl = incl - csz;
-      const uint32_t total = g_shfl(c, incl, kL - 1);
+      const uint32_t total = g_shfl(c, incl, 31);
       const unsigned gm = g_ballot(c, gc);
       const int ngc = __popc(gm);
       if (alloc + total + (uint32_t)(q_tail + ngc) > P.arena_words) {
@@ -446,7 +401,7 @@ __device__ __forceinline__ void move_down(C &c, const TreeParams &P, int e) {
         const uint32_t so = g_shfl(c, coff, sl);
         const uint32_t sw = g_shfl(c, csz, sl);
         const uint32_t dof = alloc + g_shfl(c, excl, sl);
-        copy_words(dst + dof, src + so, sw, c.lane, kL);
+        copy_words(dst + dof, src + so, sw, c.lane);
       }
       alloc += total;
     }
@@ -466,25 +421,23 @@ __device__ __forceinline__ void move_down(C &c, const TreeParams &P, int e) {
 // probs element (answer row k, move m) = probs[k * prs + m * pcs]: row-major [n][96] from the
 // host API (prs 96, pcs 1), move-major [96][ld] from the tensor-core network (prs 1, pcs ld).
 // Same arithmetic, in the same order per leaf, as the reference loop, but organised so that the
-// loads of all pending leaves (processed kL at a time) are in flight together:
+// loads of all pending leaves (processed 32 at a time) are in flight together:
 //   "flat" phases  : one lane per legal-move slot over the concatenation of all leaves
 //                    (the MT19937 draw of flat element i is simply draw number i); the leaf an
 //                    element belongs to comes from a byte array filled once per chunk;
 //   "leaf" phases  : one lane per leaf for the order-dependent float sums / max / integer sum;
 //   backup         : per tree level, the lanes whose paths meet in the same slot are grouped with
 //                    __match_any_sync and the lowest lane applies the adds in leaf order.
-template <class C>
-__device__ __forceinline__ void receive_eval(C &c, const TreeParams &P, WarpSm &sm,
+__device__ __forceinline__ void receive_eval(Ctx &c, const TreeParams &P, WarpSm &sm,
                                              const float *eval, const float *probs, long prs,
                                              long pcs) {
-  constexpr int kL = C::L;
-  constexpr int kE = 128 / kL;    // flat elements per lane per trip (4 or 8)
-  constexpr int kTrip = kE * kL;  // = 128 flat elements per trip
+  constexpr int kE = 4;       // flat elements per lane per trip
+  constexpr int kTrip = 128;  // flat elements per trip
   const int np_all = c.n_pending;
   const int lane = c.lane;
   const int prs32 = (int)prs, pcs32 = (int)pcs;  // element offsets fit 31 bits (<= 96 * rows)
-  for (int b0 = 0; b0 < np_all; b0 += kL) {
-  const int np = min(kL, np_all - b0);
+  for (int b0 = 0; b0 < np_all; b0 += 32) {
+  const int np = min(32, np_all - b0);
   const float *eval_b = eval + b0;
   const float *probs_b = probs + (long)b0 * prs;
   // ---- leaf phase 0: pending records (leaf offset, path length | n_legal << 8)
@@ -505,7 +458,7 @@ __device__ __forceinline__ void receive_eval(C &c, const TreeParams &P, WarpSm &
   for (int u = 0; u < 4; ++u) path4[u] = (lane < np && my_plen > u) ? my_pd[2 + u] : 0u;
   const int incl = (int)g_incl_scan(c, (uint32_t)my_n);
   sm.l_pre[lane] = incl - my_n;
-  if (lane == kL - 1) sm.l_pre[kL] = incl;
+  if (lane == 31) sm.l_pre[32] = incl;
   sm.l_off[lane] = my_off;
   g_sync(c);
   for (int k0 = 0; k0 < np;) {
@@ -535,7 +488,7 @@ __device__ __forceinline__ void receive_eval(C &c, const TreeParams &P, WarpSm &
     uint32_t w3n[kE];
 #pragma unroll
     for (int u = 0; u < kE; ++u) {
-      const int i = lane + kL * u;
+      const int i = lane + 32 * u;
       w3n[u] = 0;
       if (i < T) {
         const int k = sm.own[i];
@@ -547,7 +500,7 @@ __device__ __forceinline__ void receive_eval(C &c, const TreeParams &P, WarpSm &
       float pv4[kE];
 #pragma unroll
       for (int u = 0; u < kE; ++u) {
-        const int i = i0 + lane + kL * u;
+        const int i = i0 + lane + 32 * u;
         w3[u] = w3n[u];
         pv4[u] = 0.0f;
         if (i < T) pv4[u] = probs_b[(int)sm.own[i] * prs32 + s3_move(w3[u]) * pcs32];
@@ -555,7 +508,7 @@ __device__ __forceinline__ void receive_eval(C &c, const TreeParams &P, WarpSm &
       if (i0 + kTrip < T) {
 #pragma unroll
         for (int u = 0; u < kE; ++u) {
-          const int i = i0 + kTrip + lane + kL * u;
+          const int i = i0 + kTrip + lane + 32 * u;
           w3n[u] = 0;
           if (i < T) {
             const int k = sm.own[i];
@@ -565,7 +518,7 @@ __device__ __forceinline__ void receive_eval(C &c, const TreeParams &P, WarpSm &
       }
 #pragma unroll
       for (int u = 0; u < kE; ++u) {
-        const int i = i0 + lane + kL * u;
+        const int i = i0 + lane + 32 * u;
         if (i < T) sm.mv[i] = (uint8_t)s3_move(w3[u]), sm.fval[i] = pv4[u];
       }
     }
@@ -581,7 +534,7 @@ __device__ __forceinline__ void receive_eval(C &c, const TreeParams &P, WarpSm &
         uint32_t y[kE];
 #pragma unroll
         for (int u = 0; u < kE; ++u) {
-          const int i = i0 + lane + kL * u;
+          const int i = i0 + lane + 32 * u;
           y[u] = i < seg ? mt_next_word(c.mt, c.mt_idx + i) : 0u;
         }
         g_sync(c);
@@ -590,7 +543,7 @@ __device__ __forceinline__ void receive_eval(C &c, const TreeParams &P, WarpSm &
         for (int u = 0; u < kE; ++u) g[u] = d_gamma[mt_temper(y[u]) & 1023u];
 #pragma unroll
         for (int u = 0; u < kE; ++u) {
-          const int i = i0 + lane + kL * u;
+          const int i = i0 + lane + 32 * u;
           if (i < seg) c.mt[c.mt_idx + i] = y[u], sm.dval[done + i] = g[u];
         }
         g_sync(c);
@@ -619,7 +572,7 @@ __device__ __forceinline__ void receive_eval(C &c, const TreeParams &P, WarpSm &
     g_sync(c);
     // ---- flat phase 4: weighted = filtered*scalar + dirichlet*dscalar (setProbs)
 #pragma unroll 2
-    for (int i = lane; i < T; i += kL) {
+    for (int i = lane; i < T; i += 32) {
       const int k = sm.own[i];
       sm.fval[i] = __fadd_rn(__fmul_rn(sm.fval[i], sm.l_a[k]), __fmul_rn(sm.dval[i], sm.l_b[k]));
     }
@@ -636,7 +589,7 @@ __device__ __forceinline__ void receive_eval(C &c, const TreeParams &P, WarpSm &
     // ---- flat phase 6: 9-bit integer priors. A leaf is evaluated before it can get children,
     // so its slot words are still {0, 0, 0, move}: the new word is move | prior << 7.
 #pragma unroll 2
-    for (int i = lane; i < T; i += kL) {
+    for (int i = lane; i < T; i += 32) {
       const int k = sm.own[i];
       const int j = i + base_i - sm.l_pre[k];
       const double x = (double)__fmul_rn(sm.fval[i], sm.l_a[k]);
@@ -712,7 +665,7 @@ __device__ __forceinline__ void receive_eval(C &c, const TreeParams &P, WarpSm &
     c.root_eval = __fadd_rn(c.root_eval, (pl & 1) ? dd : de);
   }
   g_sync(c);
-  }  // batch of <= kL leaves
+  }  // batch of <= 32 leaves
   c.root_allv = 0;
   c.d_evals += np_all;
   c.n_pending = 0;
@@ -803,12 +756,9 @@ __device__ __forceinline__ float skey_inv(int k) {
 
 // ---- TrainMC::search (trainmc.cpp:602-696) --------------------------------------------------
 // The select loop only walks down existing children; a new edge ends it and the expansion
-// (do_move + legal moves + record write, the long scalar part) runs after the loop, where the
-// games that share a warp have converged again.
-template <class C>
-__device__ __forceinline__ void search(C &c, const TreeParams &P, WarpSm &sm) {
-  constexpr int kL = C::L;
-  constexpr int kS = kL == 32 ? 2 : 3;  // slot registers per lane: 64 / 48 slots screened
+// (do_move + legal moves + record write, the long scalar part) runs after the loop.
+__device__ __forceinline__ void search(Ctx &c, const TreeParams &P, WarpSm &sm) {
+  constexpr int kS = 2;  // slot registers per lane: 64 slots screened
   ++c.searches_done;
   c.work += 1;
   int level = 0;
@@ -840,7 +790,7 @@ __device__ __forceinline__ void search(C &c, const TreeParams &P, WarpSm &sm) {
     uint4 s[kS];
 #pragma unroll
     for (int j = 0; j < kS; ++j)
-      s[j] = c.lane + kL * j < n ? ld4(r + 8 + 4 * (c.lane + kL * j)) : zero4;
+      s[j] = c.lane + 32 * j < n ? ld4(r + 8 + 4 * (c.lane + 32 * j)) : zero4;
     const uint4 h1 = ld4(r + 4);
     const int depth = (int)((h1.x >> 8) & 0xffu);
     const float denominator = __uint_as_float(h1.y);
@@ -853,7 +803,7 @@ __device__ __forceinline__ void search(C &c, const TreeParams &P, WarpSm &sm) {
       v_sqrt = __double2float_rn(__dmul_rn((double)P.c_puct, sqrt((double)(float)cur_visits)));
     int emin = -1;
     bool none = false;
-    if (n <= kS * kL) {
+    if (n <= kS * 32) {
       // screening pass: interval per slot, decide when a single slot (or only exact ones) can
       // hold the maximum
       float lo[kS], hi[kS];
@@ -862,7 +812,7 @@ __device__ __forceinline__ void search(C &c, const TreeParams &P, WarpSm &sm) {
 #pragma unroll
       for (int j = 0; j < kS; ++j) {
         lo[j] = hi[j] = -INFINITY, in[j] = false;
-        if (j == 0 || n > kL * j) in[j] = puct_bounds(s[j], denominator, v_sqrt, lo[j], hi[j]);  // group-uniform
+        if (j == 0 || n > 32 * j) in[j] = puct_bounds(s[j], denominator, v_sqrt, lo[j], hi[j]);  // warp-uniform
         lmx = fmaxf(lmx, lo[j]);
       }
       const float lmax = skey_inv(g_max(c, skey(lmx)));
@@ -870,7 +820,7 @@ __device__ __forceinline__ void search(C &c, const TreeParams &P, WarpSm &sm) {
         none = true;
       } else {
         // candidates = slots whose interval reaches lmax; per lane: how many, the first one, and
-        // whether any of them is inexact -- then three group collectives whatever kS is
+        // whether any of them is inexact -- then three warp collectives whatever kS is
         int cnt_l = 0, first_l = 0x7fffffff;
         bool cin = false;
 #pragma unroll
@@ -878,7 +828,7 @@ __device__ __forceinline__ void search(C &c, const TreeParams &P, WarpSm &sm) {
           const bool cj = hi[j] >= lmax;
           cin = cin || (cj && in[j]);
           cnt_l += cj ? 1 : 0;
-          first_l = cj ? c.lane + kL * j : first_l;
+          first_l = cj ? c.lane + 32 * j : first_l;
         }
         const int cnt = g_add(c, cnt_l);
         const bool any_in = g_ballot(c, cin) != 0u;
@@ -890,7 +840,7 @@ __device__ __forceinline__ void search(C &c, const TreeParams &P, WarpSm &sm) {
       CB_PROF(c.n_exact += 1;)
       float best_u = -INFINITY;
       int best_e = 0x7fffffff;
-      for (int e = c.lane, j = 0; e < n; e += kL, ++j) {
+      for (int e = c.lane, j = 0; e < n; e += 32, ++j) {
         uint4 sx;
         if (j < kS) {
           sx = s[0];
@@ -937,7 +887,7 @@ __device__ __forceinline__ void search(C &c, const TreeParams &P, WarpSm &sm) {
       g_sync(c);
       return;
     }
-    const int owner = emin & (kL - 1), oj = emin / kL;
+    const int owner = emin & 31, oj = emin / 32;
     const uint32_t so = node + 8u + 4u * (uint32_t)emin;
     uint4 best_s = s[0];
 #pragma unroll
@@ -1013,7 +963,7 @@ __device__ __forceinline__ void search(C &c, const TreeParams &P, WarpSm &sm) {
         const uint32_t *pr = c.base + sm.node[l];
         const int pn = (int)(pr[4] & 0xffu);
         bool ok = true;
-        for (int e = c.lane; e < pn; e += kL) {
+        for (int e = c.lane; e < pn; e += 32) {
           const uint32_t w = pr[8 + 4 * e + 3];
           if (!s3_has(w) || !r_known(s3_result(w))) ok = false;
         }
@@ -1056,8 +1006,7 @@ __device__ __forceinline__ void search(C &c, const TreeParams &P, WarpSm &sm) {
 }
 
 // ---- TrainMC::doIteration (trainmc.cpp:139-178) ---------------------------------------------
-template <class C>
-__device__ __forceinline__ bool tree_do_iteration(C &c, const TreeParams &P, WarpSm &sm,
+__device__ __forceinline__ bool tree_do_iteration(Ctx &c, const TreeParams &P, WarpSm &sm,
                                                   const float *eval, const float *probs,
                                                   long prs = 0, long pcs = 0,
                                                   bool resume = false) {
@@ -1093,11 +1042,11 @@ __device__ __forceinline__ bool tree_do_iteration(C &c, const TreeParams &P, War
 }
 
 // TrainMC::chooseHighProbMove (trainmc.cpp:298-308) incl. the int32 max_prob quirk (Q3)
-template <class C> __device__ __forceinline__ int choose_high_prob(C &c, WarpSm &sm) {
+__device__ __forceinline__ int choose_high_prob(Ctx &c, WarpSm &sm) {
   const uint32_t *r = c.base + c.root_off;
   const int n = (int)(r[4] & 0xffu);
   const float denominator = __uint_as_float(r[5]);
-  for (int e = c.lane; e < n; e += C::L)
+  for (int e = c.lane; e < n; e += 32)
     sm.f[e] = __fmul_rn((float)s3_prior(r[8 + 4 * e + 3]), denominator);
   g_sync(c);
   int max_prob = 0, idx = -1;
@@ -1110,8 +1059,7 @@ template <class C> __device__ __forceinline__ int choose_high_prob(C &c, WarpSm 
 }
 
 // "Reset tree" (trainmc.cpp:397-404, 461-468): single node reached by `move` from the root
-template <class C>
-__device__ __forceinline__ void reset_tree_after(C &c, const TreeParams &P, int move) {
+__device__ __forceinline__ void reset_tree_after(Ctx &c, const TreeParams &P, int move) {
   const CState st = do_move(rec_state(c.base + c.root_off), move);
   const int depth = (int)((c.base[c.root_off + 4] >> 8) & 0xffu) + 1;
   g_sync(c);
@@ -1120,12 +1068,10 @@ __device__ __forceinline__ void reset_tree_after(C &c, const TreeParams &P, int 
 }
 
 // ---- TrainMC::chooseMove (trainmc.cpp:110-137, 310-473) -------------------------------------
-// Lane l looks at root slots l, l + kL, ... (ascending); per-lane bests are merged with the
+// Lane l looks at root slots l, l + 32, ... (ascending); per-lane bests are merged with the
 // reference's tie-breaks (first slot wins).
-template <class C>
-__device__ __forceinline__ int choose_move(C &c, const TreeParams &P, WarpSm &sm,
+__device__ __forceinline__ int choose_move(Ctx &c, const TreeParams &P, WarpSm &sm,
                                            float *prob_sample) {
-  constexpr int kL = C::L;
   const uint32_t *r = c.base + c.root_off;
   const int n = (int)(r[4] & 0xffu);
   const int depth = (int)((r[4] >> 8) & 0xffu);
@@ -1135,7 +1081,7 @@ __device__ __forceinline__ int choose_move(C &c, const TreeParams &P, WarpSm &sm
     // skipping won children unless the root is lost.
     const bool won = r_won(c.root_result);
     int best_key = -1, best_e = 0x7fffffff;
-    for (int e = c.lane; e < n; e += kL) {
+    for (int e = c.lane; e < n; e += 32) {
       const uint4 sl = ld4(r + 8 + 4 * e);
       if (s3_has(sl.w)) {
         const int cr = s3_result(sl.w);
@@ -1162,13 +1108,13 @@ __device__ __forceinline__ int choose_move(C &c, const TreeParams &P, WarpSm &sm
   if (depth < 6 && !P.testing) {  // chooseMoveOpening (trainmc.cpp:375-436)
     int choice = choose_high_prob(c, sm);
     int vis = 0;
-    for (int e = c.lane; e < n; e += kL) {
+    for (int e = c.lane; e < n; e += 32) {
       const uint4 sl = ld4(r + 8 + 4 * e);
       if (s3_has(sl.w) && !r_won(s3_result(sl.w))) vis += (int)sl.y;
     }
     const int visits = g_add(c, vis);
     const float denominator = __double2float_rn(__ddiv_rn(1.0, (double)(float)visits));
-    for (int e = c.lane; e < n; e += kL) {
+    for (int e = c.lane; e < n; e += 32) {
       const uint4 sl = ld4(r + 8 + 4 * e);
       if (s3_has(sl.w) && !r_won(s3_result(sl.w)))
         prob_sample[s3_move(sl.w)] = __fmul_rn((float)(int)sl.y, denominator);
@@ -1180,7 +1126,7 @@ __device__ __forceinline__ int choose_move(C &c, const TreeParams &P, WarpSm &sm
     }
     const int target = (int)(rng_one(c) % (uint32_t)visits);
     int carry = 0, found = -1;
-    for (int e0 = 0; e0 < n && found < 0; e0 += kL) {
+    for (int e0 = 0; e0 < n && found < 0; e0 += 32) {
       const int e = e0 + c.lane;
       bool elig = false;
       uint32_t v = 0u;
@@ -1192,7 +1138,7 @@ __device__ __forceinline__ int choose_move(C &c, const TreeParams &P, WarpSm &sm
       const uint32_t incl = g_incl_scan(c, v) + (uint32_t)carry;
       const unsigned hit = g_ballot(c, elig && (int)incl > target);
       if (hit) found = e0 + (__ffs((int)hit) - 1);
-      carry = (int)g_shfl(c, incl, kL - 1);
+      carry = (int)g_shfl(c, incl, 31);
     }
     choice = s3_move(r[8 + 4 * found + 3]);
     move_down(c, P, found);
@@ -1203,7 +1149,7 @@ __device__ __forceinline__ int choose_move(C &c, const TreeParams &P, WarpSm &sm
   int choice = choose_high_prob(c, sm);
   int bv = 0, be = 0x7fffffff;
   float bf = 0.0f;
-  for (int e = c.lane; e < n; e += kL) {
+  for (int e = c.lane; e < n; e += 32) {
     const uint4 sl = ld4(r + 8 + 4 * e);
     if (s3_has(sl.w) && !r_won(s3_result(sl.w))) {
       const int cr = s3_result(sl.w);
@@ -1229,13 +1175,12 @@ __device__ __forceinline__ int choose_move(C &c, const TreeParams &P, WarpSm &sm
 }
 
 // ---- TrainMC::receiveOpponentMove (trainmc.cpp:180-204) -------------------------------------
-template <class C>
-__device__ __forceinline__ bool receive_opponent_move(C &c, const TreeParams &P, int move,
+__device__ __forceinline__ bool receive_opponent_move(Ctx &c, const TreeParams &P, int move,
                                                       const CState &st, int depth) {
   const uint32_t *r = c.base + c.root_off;
   const int n = (int)(r[4] & 0xffu);
   int found = 0x7fffffff;
-  for (int e = c.lane; e < n; e += C::L) {
+  for (int e = c.lane; e < n; e += 32) {
     const uint32_t w = r[8 + 4 * e + 3];
     if (s3_has(w) && s3_move(w) == move) found = e;
   }
@@ -1264,8 +1209,7 @@ constexpr int kLogWords = 1024, kLogMain = 16, kLogMainMax = 64, kLogKids = kLog
 constexpr int kLogMaxMoves = 130;
 static_assert(kLogKids + 5 * CB200_NUM_MOVES <= kLogWords, "log record too small");
 
-template <class C>
-__device__ __forceinline__ uint32_t *log_record(const C &c, const TreeParams &P) {
+__device__ __forceinline__ uint32_t *log_record(const Ctx &c, const TreeParams &P) {
   if (P.log_buf == nullptr) return nullptr;
   const int g = (int)((c.tree_ctl - P.tree) / (2 * kTreeCtlWords));
   if (g >= P.n_logged) return nullptr;
@@ -1335,8 +1279,7 @@ __device__ __noinline__ void log_pre_move(const uint32_t *base, uint32_t root_of
 // finished) or kTurnIterate (the caller must run TrainMC::doIteration for the side now to move,
 // without answers, and come back here if that completes the turn as well).
 enum : int { kTurnWait = 0, kTurnOver = 1, kTurnIterate = 2 };
-template <class C>
-__device__ __forceinline__ int choose_move_and_continue(C &c, const TreeParams &P, WarpSm &sm,
+__device__ __forceinline__ int choose_move_and_continue(Ctx &c, const TreeParams &P, WarpSm &sm,
                                                         bool defer_search) {
   {
     if (r_known(c.root_result) && c.mate_turn == 0) c.mate_turn = c.n_samples + 1;
@@ -1359,7 +1302,7 @@ __device__ __forceinline__ int choose_move_and_continue(C &c, const TreeParams &
         return kTurnOver;
       }
       float *ps = c.sample_probs + (size_t)c.n_samples * CB200_NUM_MOVES;
-      for (int j = c.lane; j < CB200_NUM_MOVES; j += C::L) ps[j] = 0.0f;
+      for (int j = c.lane; j < CB200_NUM_MOVES; j += 32) ps[j] = 0.0f;
       if (c.lane == 0) {
         const uint4 h = ld4(c.base + c.root_off);
         c.sample_state[c.n_samples] = make_ulonglong2((uint64_t)h.x | ((uint64_t)h.y << 32),
@@ -1420,13 +1363,13 @@ __device__ __forceinline__ bool game_selected(const int32_t *ctl, int to_play) {
   return ctl[CW_TO_PLAY] == ((to_play + ctl[CW_PARITY]) & 1);
 }
 
-// One SelfPlayer::doIteration for game g, executed by one group of kL lanes. offs[g] = index of
+// One SelfPlayer::doIteration for game g, executed by one warp. offs[g] = index of
 // game g's first answer row in eval/probs (exclusive prefix sum of the request counts the answers
 // were produced for). kFused: answers are read at the row the game was handed last time
 // (ctl[CW_REQ_BASE]); the new leaf states are appended to `packed` at row0 + (rows handed out
 // by one atomicAdd on *req_ctr per game); *live_ctr counts the games that are not finished and
 // *err_ctr keeps the most negative error code.
-template <bool kFused, int kL>
+template <bool kFused>
 __device__ __forceinline__ void run_game(const TreeParams &P, int g, WarpSm &sm,
                                          const float *__restrict__ eval,
                                          const float *__restrict__ probs, long prs, long pcs,
@@ -1437,8 +1380,7 @@ __device__ __forceinline__ void run_game(const TreeParams &P, int g, WarpSm &sm,
   int32_t *ctl = P.ctl + (size_t)g * kCtlWords;
   if (!game_selected(ctl, to_play)) return;
   const bool training = (to_play != 0 && to_play != 1);
-  CtxT<kL> c;
-  c.bind_lanes();
+  Ctx c;
   // staggered start (trainer.cpp:184-186), on the global game index
   if (training && stagger_div > 0 && (P.first_game + g) / stagger_div > iteration) {
     if (kFused && c.lane == 0) atomicAdd(live_ctr, 1);
@@ -1465,11 +1407,11 @@ __device__ __forceinline__ void run_game(const TreeParams &P, int g, WarpSm &sm,
     // This launch will ingest evaluations: request everything whose address is already known
     // (MT19937 state, pending records, this game's rows of the move-major probability matrix)
     // so that the DRAM/L2 round trips overlap the control-block loads and each other.
-    for (int i = c.lane * 32; i < 624; i += kL * 32) prefetch_l1(c.mt + i);
+    for (int i = c.lane * 32; i < 624; i += 1024) prefetch_l1(c.mt + i);
     const int pw = c.n_pending * kPendWords;
-    for (int i = c.lane * 32; i < pw; i += kL * 32) prefetch_l1(c.pending + i);
+    for (int i = c.lane * 32; i < pw; i += 1024) prefetch_l1(c.pending + i);
     if (pcs > 1)
-      for (int m = c.lane; m < CB200_NUM_MOVES; m += kL) prefetch_l1(probs + (long)m * pcs + off);
+      for (int m = c.lane; m < CB200_NUM_MOVES; m += 32) prefetch_l1(probs + (long)m * pcs + off);
   }
   load_tree(c, P, c.to_play);
   // SelfPlayer::doIteration (selfplayer.cpp:115-122) with chooseMoveAndContinue's loop
@@ -1505,7 +1447,7 @@ __device__ __forceinline__ void run_game(const TreeParams &P, int g, WarpSm &sm,
     }
     base = g_shfl(c, base, 0);
     if (!c.yielded)
-      for (int k = c.lane; k < c.n_pending; k += kL) packed[row0 + base + k] = c.leaf_state[k];
+      for (int k = c.lane; k < c.n_pending; k += 32) packed[row0 + base + k] = c.leaf_state[k];
     if (c.lane == 0) ctl[CW_YIELD] = c.yielded;
   }
   if (c.lane == 0) {
@@ -1546,17 +1488,16 @@ __device__ __forceinline__ void run_game(const TreeParams &P, int g, WarpSm &sm,
   }
 }
 
-// Lock-step game step: one group of kL lanes per game, all games of the trainer (or the live
-// games of one stream group, through the group's live list).
-template <bool kFused, int kL, int kMinBlocks>
+// Lock-step game step: one warp per game, all games of the trainer (or the live games of one
+// stream group, through the group's live list).
+template <bool kFused, int kMinBlocks>
 __global__ void __launch_bounds__(kTreeWarps * 32, kMinBlocks)
     k_iterate(TreeParams P, const float *__restrict__ eval, const float *__restrict__ probs,
               long prs, long pcs, const int32_t *__restrict__ offs, int to_play, int iteration,
               int stagger_div) {
-  constexpr int kGroups = kTreeWarps * (32 / kL);  // games per CTA
-  __shared__ WarpSm sm_all[kGroups];
-  const int grp = threadIdx.x / kL;
-  const int idx = blockIdx.x * kGroups + grp;
+  __shared__ WarpSm sm_all[kTreeWarps];
+  const int grp = threadIdx.x / 32;
+  const int idx = blockIdx.x * kTreeWarps + grp;
   int g;
   if (kFused) {
     if (P.live_list != nullptr) {
@@ -1571,10 +1512,10 @@ __global__ void __launch_bounds__(kTreeWarps * 32, kMinBlocks)
     if (g >= P.num_games) return;
   }
   const int par = (iteration + 1) & 1;
-  run_game<kFused, kL>(P, g, sm_all[grp], eval, probs, prs, pcs, offs, to_play, iteration,
-                       stagger_div, kFused ? P.group_ctr + par : nullptr,
-                       kFused ? P.group_ctr + 2 + par : nullptr, kFused ? P.group_ctr + 4 : nullptr,
-                       P.group_row0, P.packed);
+  run_game<kFused>(P, g, sm_all[grp], eval, probs, prs, pcs, offs, to_play, iteration,
+                   stagger_div, kFused ? P.group_ctr + par : nullptr,
+                   kFused ? P.group_ctr + 2 + par : nullptr, kFused ? P.group_ctr + 4 : nullptr,
+                   P.group_row0, P.packed);
 }
 
 // Live games of one stream group, ascending (one warp per group): list[game_begin + i], i < n.

@@ -30,7 +30,8 @@ extern "C" void shim_step_batch(int64_t n, const uint64_t *states, uint64_t seed
 }
 extern "C" uint32_t shim_step_rnd(uint64_t seed, uint64_t i) { return cb200::step_rnd(seed, i); }
 
-// basic_moves() (the first half of legal_moves_t that the split K1 kernel runs on every position):
+// basic_moves() (the first half of legal_moves_t; the paired K1 kernel runs its paired form,
+// basic_moves_pair, on every position):
 // its "any line" flag must equal legal_moves_t's, and without a line its mask IS the legal mask.
 // Returns the number of positions where that fails.
 extern "C" int64_t shim_basic_moves_check(int64_t n, const uint64_t *states) {

@@ -49,24 +49,16 @@ def test_game_step_ragged_sizes_without_encoding(oracle, n):
     assert (cb.reference_order_from_planes(nx) == nxt).all()
 
 
-@pytest.mark.parametrize("env", [{}, {"CB200_K1_WAVES": "1"}, {"CB200_K1_PAIR": "0"}, {"CB200_K1_PAIR": "1"},
-                                 {"CB200_K1_PAIR": "2"}, {"CB200_K1_PAIR": "3"}, {"CB200_K1_PAIR": "4"},
-                                 {"CB200_K1_PAIR": "5"}, {"CB200_K1_SPLIT": "1"}, {"CB200_K1_SELECT_ONLY": "1"}],
-                         ids=["paired", "paired-one-wave", "paired-branchy-finish", "paired-branchy-finish-prefetch",
-                              "paired-cta-queue", "paired-7-ctas", "paired-prefetch-6-ctas", "paired-joint-finish-no-prefetch",
-                              "split", "select-only"])
-def test_game_step_kernel_forms_vs_oracle(oracle, monkeypatch, env):
-    """Every form of the game-logic kernel (paired with a queue per warp, prefetch and the joint
-    branch-free finish = default; without either; with a queue per CTA; register-capped builds;
-    split; select-only) and the default with a single
-    wave of CTAs (many trips per CTA: the queues wrap through several flushes) against the oracle
-    on 256 k reachable positions."""
-    for k in ("CB200_K1_WAVES", "CB200_K1_PAIR", "CB200_K1_SPLIT", "CB200_K1_SELECT_ONLY"):
-        monkeypatch.delenv(k, raising=False)
-    for k, v in env.items():
-        monkeypatch.setenv(k, v)
-    n = 1 << 18
-    states = oracle.gen_states(4711, n)
+def test_game_step_many_trips_per_cta_vs_oracle(oracle):
+    """The paired kernel with several trips per CTA against the oracle on 2^24 positions (2^22
+    reachable positions tiled 4x, a different random word for every index). The grid is at most
+    8 waves of resident CTAs: 148 SMs x 4 CTAs (64 registers, 256 threads) x 8 = 4 736 CTAs of
+    512 positions per trip = 2.42 M positions per sweep, so every CTA makes about 7 trips. A warp
+    queues about 10 of its 64 positions per trip (the ones with a line), about 66 over its trips,
+    so every warp flushes 32 queued positions inside the loop, the prefetch of the next trip is
+    used, and the drain finishes what is left."""
+    states = np.tile(oracle.gen_states(4711, 1 << 22), (4, 1))
+    n = len(states)
     mf, nx, _ = cb.game_step(cb.planes_from_reference_order(states), 5)
     masks, flags, nxt, _ = oracle.step_batch(states, step_rnd(5, n), want_enc=False, threads=8)
     assert (mf[:, :3] == masks).all() and (mf[:, 3] == flags).all()

@@ -145,9 +145,10 @@ def test_swar_rules_header_matches_golden():
 
 
 def test_basic_moves_is_the_legal_mask_when_no_line_exists(oracle):
-    """The split game-logic kernel (game_step.cuh) finishes positions without a line from
-    basic_moves() alone and queues the others: its line flag must equal legal_moves_t's and, when
-    no line exists, its mask must be the legal mask. 300 k reachable positions + the golden set."""
+    """The paired game-logic kernel (game_step.cuh) finishes positions without a line from the
+    basic-rule mask alone (basic_moves_pair, the paired form of basic_moves()) and queues the
+    others: basic_moves()'s line flag must equal legal_moves_t's and, when no line exists, its mask
+    must be the legal mask. 300 k reachable positions + the golden set."""
     from corintho_ai_b200 import planes_from_reference_order
     lib = _shim()
     lib.shim_basic_moves_check.restype = C.c_int64
@@ -158,7 +159,7 @@ def test_basic_moves_is_the_legal_mask_when_no_line_exists(oracle):
 
 
 def test_paired_fast_path_forms_equal_the_plain_ones(oracle):
-    """k_game_step_pair (game_step.cuh) runs basic_moves_pair / nth_move_lut / do_move_lut; on the
+    """k_game_step_pairw (game_step.cuh) runs basic_moves_pair / nth_move_lut / do_move_lut; on the
     host they must agree with basic_moves / nth_move / do_move for every position, every legal move
     and every rank. 300 k reachable positions + the golden set, paired first-with-last."""
     from corintho_ai_b200 import planes_from_reference_order

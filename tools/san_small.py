@@ -15,12 +15,6 @@ assert t.run_selfplay(0, stagger=True)
 gs, ev, pr, go = t.streamed_samples()
 assert go.shape[0] == t.num_samples()
 t.write_samples(); t.raw_samples_device()
-# 16 lanes per game, lock-step + persistent
-os.environ["CB200_LANES"] = "16"; os.environ["CB200_PS_LANES"] = "16"
-u = cb.Trainer(96, "", 4, 32, 16, 1.0, 0.25)
-u.set_weights(flat, 0, "bf16")
-assert u.run_selfplay(0)
-del os.environ["CB200_LANES"], os.environ["CB200_PS_LANES"]
 # bf16x3 network, two-model testing mode, fused tourney, K1
 v = cb.Trainer(32, "", 5, 32, 8, 1.0, 0.0, 0, 1, True)
 v.set_weights(flat, 0, "bf16x3"); v.set_weights(flat, 1, "bf16x3")
