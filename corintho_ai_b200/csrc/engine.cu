@@ -3,6 +3,7 @@
 // call for call; all game state lives in HBM and every step of the path is a CUDA kernel.
 // There is deliberately no CPU implementation of the path in this library.
 
+#include <limits.h>
 #include <math.h>
 #include <stdlib.h>
 #include <string.h>
@@ -151,6 +152,13 @@ struct cb200_trainer {
   int seed = 0;
   // fused mode: games are split into independent stream groups (no lock-step across groups)
   int n_groups = 1;
+  // the rest of the fused loop's schedule, read from the environment once, at creation
+  struct Schedule {
+    int yield_budget = 96;      // CB200_YIELD: parking work budget (TreeParams::yield_budget)
+    int yield_min_live = 128;   // CB200_YIELD_MIN_LIVE: no parking below that many live games
+    bool persistent = true;     // off with CB200_NO_PERSISTENT
+    long long ps_capacity = LLONG_MAX;  // CB200_PS_CAPACITY: hand-over at most at this many live games
+  } sched;
   int32_t *d_live_list = nullptr;   // [num_games] live games per stream group (TreeParams::live_list)
   int32_t *d_live_count = nullptr;  // [n_groups]
   std::vector<cudaStream_t> g_stream;
@@ -320,6 +328,12 @@ int scan(cb200_trainer *t, int to_play) {
   return CB200_OK;
 }
 
+// error code a game step reported through its summary / counters
+int game_error(int code) {
+  return set_error(code, "a game overflowed its node arena / path / sample buffer (raise "
+                         "CB200_ARENA_NODES) or reached an impossible state");
+}
+
 int fetch_summary(cb200_trainer *t) {
   CB_CUDA(cudaMemcpyAsync(t->h_summary, t->d_summary, 4 * sizeof(int32_t), cudaMemcpyDeviceToHost,
                           cur_stream()));
@@ -328,10 +342,7 @@ int fetch_summary(cb200_trainer *t) {
     int rc = prof_drain(t);
     if (rc != CB200_OK) return rc;
   }
-  if (t->h_summary[2] != 0)
-    return set_error(t->h_summary[2],
-                     "a game overflowed its node arena / path / sample buffer (raise "
-                     "CB200_ARENA_NODES) or reached an impossible state");
+  if (t->h_summary[2] != 0) return game_error(t->h_summary[2]);
   return CB200_OK;
 }
 
@@ -800,6 +811,10 @@ cb200_trainer *cb200_trainer_create_shard(int total_games, int first_game, int n
     }
     t->g_stream.push_back(st), t->g_begin.push_back(b), t->g_end.push_back(e);
   }
+  if (const char *env = getenv("CB200_YIELD")) t->sched.yield_budget = atoi(env);
+  if (const char *env = getenv("CB200_YIELD_MIN_LIVE")) t->sched.yield_min_live = atoi(env);
+  if (const char *env = getenv("CB200_PS_CAPACITY")) t->sched.ps_capacity = atoll(env);
+  t->sched.persistent = getenv("CB200_NO_PERSISTENT") == nullptr;
   {
     int sms = 148;
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
@@ -1408,6 +1423,21 @@ int cb200_trainer_evaluate(cb200_trainer *t, int model, int n, const float *game
   return CB200_OK;
 }
 
+// Games a persistent CTA (one per SM) can hold: bf16x3 networks keep hi and lo operand copies in
+// shared memory and fit with 8 games only.
+static int ps_games_per_sm(int mode) { return mode == 2 ? 8 : 16; }
+
+// The one rule for when the persistent kernel may run the games of a fused run: it takes over at
+// this many live games or fewer; 0 = never. It needs the tensor-core network (in two-model runs
+// both networks, with the same operand mode) and at most kPsRowsPerGame requests per game.
+static int ps_takeover(const cb200_trainer *t) {
+  const NetTC &n0 = t->nettc[0];
+  if (!t->sched.persistent || t->precision[0] != 1 || t->P.spe > kPsRowsPerGame) return 0;
+  if (t->P.testing && (t->precision[1] != 1 || t->nettc[1].mode != n0.mode)) return 0;
+  const long long fit = (long long)t->ps_ctas * ps_games_per_sm(n0.mode);
+  return (int)std::max(0ll, std::min(t->sched.ps_capacity, fit));
+}
+
 // Persistent fused tail (persistent.cuh). Called with every stream idle. Runs the remaining games
 // (or `max_rounds` iterations of them) as a sequence of persistent launches; between launches
 // the live games are listed again so that they spread evenly over the SMs (8 games per CTA
@@ -1502,29 +1532,21 @@ static int run_persistent(cb200_trainer *t, int max_rounds, int *rounds_done, bo
   cudaStream_t st = t->g_stream[0];
   *rounds_done = 0, *all_done = false;
   TreeParams P = t->P;
-  // parking inside the persistent kernels (CB200_PS_YIELD = work budget per round, 0 = off; only
-  // while at least CB200_PS_YIELD_MIN_LIVE games are live)
-  int ps_yield = 0, ps_yield_min = 512;
-  if (const char *e = getenv("CB200_PS_YIELD")) ps_yield = atoi(e);
-  if (const char *e = getenv("CB200_PS_YIELD_MIN_LIVE")) ps_yield_min = atoi(e);
+  P.yield_budget = 0;  // no parking inside the persistent kernels (measured: no gain)
+  // deal the games again once half of them have finished in one launch (not worth it for the
+  // last few; other shares and floors measured within noise)
+  constexpr int kRedealPct = 50, kRedealMinGames = 64;
   while (*rounds_done < max_rounds) {
-    P.yield_budget = t->ps_n >= ps_yield_min ? ps_yield : 0;
     if (t->ps_n == 0) {
       *all_done = true;
       break;
     }
     const int rounds = max_rounds - *rounds_done;
-    // deal the games again once half of them have finished (not worth it for the last few)
-    int redeal_pct = 50, redeal_min = 64;
-    if (const char *e = getenv("CB200_PS_REDEAL_PCT")) redeal_pct = atoi(e);
-    if (const char *e = getenv("CB200_PS_REDEAL_MIN")) redeal_min = atoi(e);
-    int exit_done = t->ps_n > redeal_min ? (int)((long long)t->ps_n * redeal_pct / 100) : 0x7fffffff;
-    if (exit_done < 1) exit_done = 1;
-    if (getenv("CB200_PS_NO_REDEAL")) exit_done = 0x7fffffff;
-    const int mode = t->nettc[0].mode;  // 0 bf16, 1 fp16, 2 bf16x3 (8 games per CTA only: shared memory)
+    const int exit_done = t->ps_n > kRedealMinGames ? t->ps_n * kRedealPct / 100 : INT_MAX;
+    const int mode = t->nettc[0].mode;  // 0 bf16, 1 fp16, 2 bf16x3
     const bool wide = t->ps_n > t->ps_ctas * 8;
-    if (wide && mode == 2)
-      return set_error(CB200_ERR_STATE, "persistent kernel: bf16x3 networks run at most 8 games per SM");
+    if (t->ps_n > t->ps_ctas * ps_games_per_sm(mode))
+      return set_error(CB200_ERR_STATE, "persistent kernel: more live games than fit on the device");
     CB_CUDA(cudaMemsetAsync(t->d_ps_out, 0, 4 * sizeof(int32_t), st));
     int rc;
     {
@@ -1542,9 +1564,7 @@ static int run_persistent(cb200_trainer *t, int max_rounds, int *rounds_done, bo
     if (t->profiling && (rc = prof_drain(t)) != CB200_OK) return rc;
     t->ps_from_lockstep = false;
     t->ps_cur = 1 - t->ps_cur;
-    if (t->h_ps_out[1] != 0)
-      return set_error(t->h_ps_out[1], "a game overflowed its node arena / path / sample buffer (raise "
-                                       "CB200_ARENA_NODES) or reached an impossible state");
+    if (t->h_ps_out[1] != 0) return game_error(t->h_ps_out[1]);
     // CTAs stop at different rounds (all games finished / the re-deal trigger): the launch
     // advanced the run by at most out[2] iterations
     const int ran = t->h_ps_out[2];
@@ -1581,31 +1601,18 @@ static int run_selfplay_groups(cb200_trainer *t, int max_iterations) {
     wall0 = now;
     return ms;
   };
-  // parking budget (TreeParams::yield_budget): a typical doIteration is ~16 searches x ~3 levels
-  // = ~60 units; while many games are live, longer ones (end-game searches that keep hitting
-  // terminal nodes) are cut into several launches. Once few games are left nobody gains from
-  // parking, and it would only stretch the last games.
-  int yield_budget = 96, yield_min_live = 128;
-  if (const char *e = getenv("CB200_YIELD")) yield_budget = atoi(e);
-  if (const char *e = getenv("CB200_YIELD_MIN_LIVE")) yield_min_live = atoi(e);
-  // Persistent tail: once every live game fits on the device at 16 games per SM (and all games
-  // have started), the rest of the run happens inside persistent kernels (persistent.cuh).
-  // (bf16x3 networks hold hi and lo operand copies in shared memory: 8 games per SM, not 16)
-  const bool ps_ok = tc && t->P.spe <= kPsRowsPerGame && !getenv("CB200_NO_PERSISTENT");
-  const long long ps_max = (long long)t->ps_ctas * (t->nettc[model].mode == 2 ? 8 : 16);
-  long long ps_capacity = ps_max;
-  if (const char *e = getenv("CB200_PS_CAPACITY")) ps_capacity = atoll(e);
-  if (ps_capacity > ps_max) ps_capacity = ps_max;
+  // Persistent tail: once few enough games are live (and all games have started), the rest of the
+  // run happens inside persistent kernels (persistent.cuh).
+  const int ps_from = ps_takeover(t);
   const int stagger_span =
       t->stagger_div > 0 ? (t->P.first_game + t->P.num_games - 1) / t->stagger_div : 0;
   // With several stream groups the network runs in single-tile CTAs of 128 threads (13 K
   // registers) that fit beside five 80-register game-step CTAs, so that one group's network
   // overlaps the other groups' tree work (2-3 % per run).
-  const bool overlap = tc && ng > 1 && getenv("CB200_NO_OVERLAP") == nullptr;
-  const bool use_lists = getenv("CB200_NO_LIVE_LIST") == nullptr;
+  const bool overlap = tc && ng > 1;
   std::vector<int> group_live(ng, -1);  // live games per group at the last host sync (-1 = unknown)
   while (max_iterations <= 0 || done_iters < max_iterations) {
-    if (!t->ps_active && ps_ok && live_games <= ps_capacity && t->iterations_done > stagger_span) {
+    if (!t->ps_active && live_games <= ps_from && t->iterations_done > stagger_span) {
       // evaluate the requests queued by the last lock-step game step, then list the live games
       const int it = t->iterations_done;
       for (int g = 0; g < ng; ++g) {
@@ -1639,12 +1646,16 @@ static int run_selfplay_groups(cb200_trainer *t, int max_iterations) {
       if (all_done) result = 1;
       break;
     }
-    const int yb = live_games >= yield_min_live ? yield_budget : 0;
+    // parking budget (TreeParams::yield_budget): a typical doIteration is ~16 searches x ~3 levels
+    // = ~60 units; while many games are live, longer ones (end-game searches that keep hitting
+    // terminal nodes) are cut into several launches. Once few games are left nobody gains from
+    // parking, and it would only stretch the last games.
+    const int yb = live_games >= t->sched.yield_min_live ? t->sched.yield_budget : 0;
     int batch = 32;
     if (max_iterations > 0 && max_iterations - done_iters < batch) batch = max_iterations - done_iters;
     // the games of each group that are still live (finished games would leave idle warps
     // behind): rebuilt once per batch on the group's own stream
-    for (int g = 0; g < ng && use_lists; ++g) {
+    for (int g = 0; g < ng; ++g) {
       if (!active[g]) continue;
       TreeParams P = t->P;
       P.game_begin = t->g_begin[g], P.game_end = t->g_end[g];
@@ -1674,11 +1685,9 @@ static int run_selfplay_groups(cb200_trainer *t, int max_iterations) {
         TreeParams P = t->P;
         P.game_begin = gb, P.game_end = ge, P.group_row0 = row0, P.group_ctr = ctr;
         P.yield_budget = yb;
-        int width = ge - gb;  // warps to launch: the group's games, or its live games
-        if (use_lists) {
-          P.live_list = t->d_live_list, P.live_count = t->d_live_count + g;
-          if (group_live[g] >= 0 && group_live[g] < width) width = group_live[g];
-        }
+        P.live_list = t->d_live_list, P.live_count = t->d_live_count + g;
+        int width = ge - gb;  // warps to launch: the group's games, or its live games once known
+        if (group_live[g] >= 0 && group_live[g] < width) width = group_live[g];
         {
           ProfScope ps(t, 3, st);
           const dim3 grid((width + kTreeWarps - 1) / kTreeWarps), block(kTreeWarps * 32);
@@ -1710,9 +1719,7 @@ static int run_selfplay_groups(cb200_trainer *t, int max_iterations) {
     for (int g = 0; g < ng; ++g) {
       if (!active[g]) continue;
       const int32_t *c = t->h_gctr + g * 8;
-      if (c[4] != 0)
-        return set_error(c[4], "a game overflowed its node arena / path / sample buffer (raise "
-                               "CB200_ARENA_NODES) or reached an impossible state");
+      if (c[4] != 0) return game_error(c[4]);
       if (c[2 + par] == 0 && c[par] == 0) active[g] = 0;
       group_live[g] = c[2 + par];
       live += c[2 + par];
@@ -1755,12 +1762,10 @@ int cb200_trainer_run_selfplay(cb200_trainer *t, int max_iterations, int stagger
     }
     return rc;
   }
-  // two-model (gating match) mode. With both networks on the tensor cores (same operand format)
-  // and every game resident at <= 16 per SM, the whole match runs in the persistent kernel
-  // (persistent.cuh; each game's requests go to the row region of the model that owns its side).
-  if ((t->iterations_done == 0 || t->ps_active) && t->precision[0] == 1 && t->precision[1] == 1 &&
-      t->nettc[0].mode == t->nettc[1].mode && t->P.spe <= kPsRowsPerGame &&
-      t->P.num_games <= t->ps_ctas * (t->nettc[0].mode == 2 ? 8 : 16) && !getenv("CB200_NO_PERSISTENT")) {
+  // two-model (gating match) mode. When the persistent kernel can hold every game, the whole match
+  // runs in it (persistent.cuh; each game's requests go to the row region of the model that owns
+  // its side).
+  if ((t->iterations_done == 0 || t->ps_active) && t->P.num_games <= ps_takeover(t)) {
     CB_CUDA(cudaStreamSynchronize(cur_stream()));
     if (!t->ps_active) {
       if ((rc = ps_list_games(t)) != CB200_OK) return rc;

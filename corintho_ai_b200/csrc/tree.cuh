@@ -85,7 +85,7 @@ struct TreeParams {
   ulonglong2 *packed;        // [num_games*spe] leaf cstates in request-row order
   // fused lock-step mode: live_list[game_begin + i], i < *live_count, are the group's games that
   // were not finished when the list was last rebuilt (k_group_live_list), so that finished games
-  // do not leave half-empty warps behind; null = every game of [game_begin, game_end)
+  // do not leave half-empty warps behind; the lock-step game step launches only these
   const int32_t *live_list;
   const int32_t *live_count;
   // fused mode: a game whose doIteration needs more than this many select levels + searches in
@@ -1500,13 +1500,8 @@ __global__ void __launch_bounds__(kTreeWarps * 32, kMinBlocks)
   const int idx = blockIdx.x * kTreeWarps + grp;
   int g;
   if (kFused) {
-    if (P.live_list != nullptr) {
-      if (idx >= *P.live_count) return;
-      g = P.live_list[P.game_begin + idx];
-    } else {
-      g = P.game_begin + idx;
-      if (g >= P.game_end) return;
-    }
+    if (idx >= *P.live_count) return;
+    g = __ldg(P.live_list + P.game_begin + idx);  // read-only while the game step runs
   } else {
     g = idx;
     if (g >= P.num_games) return;

@@ -234,19 +234,16 @@ def test_fused_selfplay_is_independent_of_parking_and_stream_groups(monkeypatch)
 
 
 KNOB_SETS = [
-    {"CB200_NO_LIVE_LIST": "1"}, {"CB200_NO_OVERLAP": "1", "CB200_GROUPS": "3"},
-    {"CB200_PS_NO_REDEAL": "1"}, {"CB200_PS_REDEAL_PCT": "10", "CB200_PS_REDEAL_MIN": "4"},
-    {"CB200_PS_YIELD": "24", "CB200_PS_YIELD_MIN_LIVE": "1"}, {"CB200_PS_CAPACITY": "40"},
-    {"CB200_PS_CAPACITY": "2368"}, {"CB200_PS_CAPACITY": "2368", "CB200_PS_YIELD": "24", "CB200_PS_YIELD_MIN_LIVE": "1"},
+    {"CB200_GROUPS": "3"}, {"CB200_PS_CAPACITY": "40"}, {"CB200_PS_CAPACITY": "2368"},
     {"CB200_GROUPS": "8", "CB200_YIELD": "30", "CB200_YIELD_MIN_LIVE": "16"},
 ]
 
 
 def test_fused_selfplay_is_independent_of_every_other_knob(monkeypatch):
-    """DESIGN.md section 5's knob table: live lists, network CTA form, persistent re-deal policy,
-    persistent parking, take-over threshold -- none may change a byte of the samples, the score or
-    the exact counters (600 games: several stream groups, both persistent kernel widths after the
-    hand-over)."""
+    """DESIGN.md section 5's knob table: stream group count (with the network overlapped beside the
+    game step), persistent take-over threshold, parking with many groups -- none may change a byte
+    of the samples, the score or the exact counters (600 games: several stream groups, both
+    persistent kernel widths after the hand-over)."""
     flat = cb.fold_batchnorm(cb.random_weights(21))
     knobs = sorted({k for ks in KNOB_SETS for k in ks})
 
