@@ -113,6 +113,13 @@ def lib():
         "cb200_analysis_set_weights": (i32, [vp, vp, C.c_size_t, i32]),
         "cb200_analysis_run": (i32, [vp, i32, vp, i32, vp, vp, vp, vp, vp]),
         "cb200_analysis_counters": (i32, [vp, vp]),
+        "cb200_analysis_begin": (i32, [vp, i32, vp, i32]),
+        "cb200_analysis_num_requests": (i32, [vp]),
+        "cb200_analysis_write_requests": (i32, [vp, vp]),
+        "cb200_analysis_do_iteration": (i32, [vp, vp, vp, i32]),
+        "cb200_analysis_results": (i32, [vp, vp, vp, vp, vp, vp]),
+        "cb200_analysis_write_requests_device": (i32, [vp, vp]),
+        "cb200_analysis_do_iteration_device": (i32, [vp, vp, vp, i32]),
         "cb200_check_states": (i64, [i64, vp, vp]),
     }
     for name, (res, args) in sig.items():
@@ -567,6 +574,23 @@ def _out_buf(a, dtype, min_size, what):
     return a
 
 
+def _dev_f32(t, min_size, what):
+    """Device buffer of the analysis' device forms: a contiguous float32 CUDA tensor with at least
+    `min_size` elements. Duck-typed on torch.Tensor's dtype / device / is_contiguous / numel /
+    data_ptr, so this package does not import torch. Returns the device address."""
+    try:
+        dtype, device = str(t.dtype), t.device
+        contiguous, numel = bool(t.is_contiguous()), int(t.numel())
+    except (AttributeError, TypeError):
+        raise Corintho200Error(f"{what}: need a CUDA tensor, got {type(t).__name__}") from None
+    if dtype != "torch.float32" or getattr(device, "type", None) != "cuda" or not contiguous:
+        raise Corintho200Error(f"{what}: need a contiguous float32 CUDA tensor, got {dtype} on {device}"
+                               f"{'' if contiguous else ' (not contiguous)'}")
+    if numel < min_size:
+        raise Corintho200Error(f"{what}: {numel} elements given, {min_size} needed")
+    return int(t.data_ptr())
+
+
 def check_states(states):
     """Structural check of cstates [n,2] u64 (see cb200_check_states): bool array, True = valid.
     Needs no GPU."""
@@ -614,14 +638,8 @@ class Analysis:
     def run(self, states, seed=0, evals=True):
         """states: [n,2] u64 cstates. Returns {"moves" [n] i32, "results" [n] i32, "values" [n]
         f32, "visits" [n,96] i32, "evals" [n,96] f32 (only with evals=True)}."""
-        st = np.ascontiguousarray(states, np.uint64)
-        if st.ndim != 2 or st.shape[1] != 2:
-            raise Corintho200Error("run: states must be an [n, 2] array of cstate words")
-        n = st.shape[0]
-        out = {"moves": np.zeros(n, np.int32), "results": np.zeros(n, np.int32),
-               "values": np.zeros(n, np.float32), "visits": np.zeros((n, NUM_MOVES), np.int32)}
-        if evals:
-            out["evals"] = np.zeros((n, NUM_MOVES), np.float32)
+        st = _analysis_states(states, "run")
+        out = _analysis_outputs(st.shape[0], evals)
         self.run_into(st, seed, **out)
         return out
 
@@ -639,6 +657,88 @@ class Analysis:
                                         _ptr(values), _ptr(visits), _ptr(evals)))
 
     def counters(self):
+        """{simulations, leaf_evals} of the last run or session (running totals while one is open)."""
         out = np.zeros(2, np.int64)
         _check(lib().cb200_analysis_counters(self._h, _ptr(out)))
         return {"simulations": int(out[0]), "leaf_evals": int(out[1])}
+
+    # ---- external-evaluator protocol: the caller's network answers the requests -----------------
+    # begin; until do_iteration(...) returns True: write_requests, evaluate, do_iteration; results.
+    # See cb200_analysis_begin in include/corintho_b200.h for the protocol's rules.
+    def begin(self, states, seed=0):
+        """Open a session on [n,2] u64 cstates (no weights needed); restarts an open one."""
+        st = _analysis_states(states, "begin")
+        _check(lib().cb200_analysis_begin(self._h, st.shape[0], _ptr(st), int(seed)))
+        self._n = st.shape[0]
+
+    def num_requests(self):
+        return _check(lib().cb200_analysis_num_requests(self._h))
+
+    def write_requests(self, out=None):
+        """The pending request rows: a fresh [num_requests, 70] float32 array, or written into `out`
+        (a writable C-contiguous float32 array of at least num_requests * 70 floats), returned."""
+        n = self.num_requests()
+        if out is None:
+            buf = np.zeros((max(n, 1), STATE_SIZE), np.float32)
+            _check(lib().cb200_analysis_write_requests(self._h, _ptr(buf)))
+            return buf[:n]
+        _out_f32(out, n * STATE_SIZE, "write_requests: out")
+        _check(lib().cb200_analysis_write_requests(self._h, _ptr(out)))
+        return out
+
+    def do_iteration(self, eval=None, probs=None):
+        """One round with the answers to the last write_requests (eval [n], probs [n,96], row-major;
+        None for the first call). True when every position is done."""
+        n = self.num_requests()
+        ev = _in_f32(eval, n, "do_iteration: eval")
+        pr = _in_f32(probs, n * NUM_MOVES, "do_iteration: probs")
+        rows = 0 if ev is None or pr is None else min(ev.size, pr.size // NUM_MOVES)
+        return bool(_check(lib().cb200_analysis_do_iteration(self._h, _ptr(ev), _ptr(pr), rows)))
+
+    def results(self, evals=True):
+        """The outputs of run() for the finished session."""
+        out = _analysis_outputs(getattr(self, "_n", 0), evals)
+        _check(lib().cb200_analysis_results(self._h, _ptr(out["moves"]), _ptr(out["results"]),
+                                            _ptr(out["values"]), _ptr(out["visits"]), _ptr(out.get("evals"))))
+        return out
+
+    def write_requests_device(self, rows):
+        """Pack the pending request rows into a float32 CUDA tensor of at least num_requests * 70
+        elements, on the library's current stream (cb200_set_stream), without waiting."""
+        n = self.num_requests()
+        _check(lib().cb200_analysis_write_requests_device(self._h, _dev_f32(rows, n * STATE_SIZE,
+                                                                            "write_requests_device: rows")))
+        return rows
+
+    def do_iteration_device(self, eval, probs):
+        """do_iteration with float32 CUDA tensors (eval [>= n], probs [>= n, 96] row-major), read in
+        place on the library's current stream; the writes to them must be ordered before it."""
+        n = self.num_requests()
+        ev = _dev_f32(eval, n, "do_iteration_device: eval")
+        pr = _dev_f32(probs, n * NUM_MOVES, "do_iteration_device: probs")
+        rows = min(int(eval.numel()), int(probs.numel()) // NUM_MOVES)
+        return bool(_check(lib().cb200_analysis_do_iteration_device(self._h, ev, pr, rows)))
+
+    def search(self, states, seed, evaluator, evals=True):
+        """run() with the caller's network: evaluator(rows [k,70] float32) -> (eval [k], probs [k,96])
+        answers every round's requests. Returns the dict run() returns."""
+        self.begin(states, seed)
+        answers = (None, None)
+        while not self.do_iteration(*answers):
+            answers = evaluator(self.write_requests())
+        return self.results(evals)
+
+
+def _analysis_states(states, what):
+    st = np.ascontiguousarray(states, np.uint64)
+    if st.ndim != 2 or st.shape[1] != 2:
+        raise Corintho200Error(f"{what}: states must be an [n, 2] array of cstate words")
+    return st
+
+
+def _analysis_outputs(n, evals):
+    out = {"moves": np.zeros(n, np.int32), "results": np.zeros(n, np.int32),
+           "values": np.zeros(n, np.float32), "visits": np.zeros((n, NUM_MOVES), np.int32)}
+    if evals:
+        out["evals"] = np.zeros((n, NUM_MOVES), np.float32)
+    return out

@@ -603,8 +603,13 @@ static int init_state(cb200_trainer *t) {
   CB_CUDA(cudaMemsetAsync(P.counters, 0, Gn * 4 * sizeof(long long), s));
   CB_CUDA(cudaMemsetAsync(t->d_offs, 0, Gn * sizeof(int32_t), s));
   CB_CUDA(cudaMemsetAsync(t->d_summary, 0, 4 * sizeof(int32_t), s));
-  CB_CUDA(cudaMemsetAsync(t->d_eval, 0, t->cap * sizeof(float), s));
-  CB_CUDA(cudaMemsetAsync(t->d_probs, 0, t->cap * CB200_NUM_MOVES * sizeof(float), s));
+  // The whole answer buffers, slack rows included: a fused two-model tourney reads rows that no
+  // evaluation of the run has written yet (the offsets of tourney.cpp:54-62), and they must read as
+  // the zeros of the reference loop's fresh buffers. The tensor-core network's move-major layout
+  // (leading dimension cap + kAnswerSlack) spreads every row over the whole buffer, so zeroing only
+  // cap rows' worth would leave the high move ids of every row to whatever the memory held before.
+  CB_CUDA(cudaMemsetAsync(t->d_eval, 0, (t->cap + kAnswerSlack) * sizeof(float), s));
+  CB_CUDA(cudaMemsetAsync(t->d_probs, 0, (t->cap + kAnswerSlack) * CB200_NUM_MOVES * sizeof(float), s));
   CB_CUDA(cudaMemsetAsync(t->d_gctr, 0, (size_t)t->n_groups * 8 * sizeof(int32_t), s));
   CB_CUDA(cudaStreamSynchronize(s));
   if (P.n_logged > 0) {
@@ -2241,8 +2246,72 @@ struct cb200_analysis {
   int32_t *d_moves = nullptr, *d_results = nullptr, *d_visits = nullptr;
   float *d_values = nullptr, *d_evals = nullptr;
   ResidentNet net;
-  int64_t counters[2] = {0, 0};    // {simulations, leaf evaluations} of the last run
+  int64_t counters[2] = {0, 0};    // {simulations, leaf evaluations} of the last run or session
+  // external-evaluator session (cb200_analysis_begin .. _results): kNoSession, kOpen or kDone;
+  // `requests` = rows the next do_iteration reads, at the offsets the last scan left in t->d_offs
+  enum { kNoSession, kOpen, kDone };
+  int session = kNoSession;
+  int requests = 0;
 };
+
+// The checks of cb200_analysis_run and _begin: n in [1, max_positions], non-null states, every
+// state accepted by cb200_check_states.
+static int analysis_check_states(const cb200_analysis *A, int n, const uint64_t *states, const char *who) {
+  if (n <= 0 || n > A->max_positions) return set_error(CB200_ERR_ARG, std::string(who) + ": n must be in [1, max_positions]");
+  if (!states) return set_error(CB200_ERR_ARG, std::string(who) + ": null states");
+  for (int i = 0; i < n; ++i)
+    if (!valid_state(states[2 * i], states[2 * i + 1]))
+      return set_error(CB200_ERR_ARG, std::string(who) + ": state " + std::to_string(i) + " is not a valid cstate");
+  return CB200_OK;
+}
+
+// positions [0, n) become games [0, n) of the trainer: seeds = outputs 0 .. n-1 of mt19937(seed),
+// fresh control blocks and trees (the kernel builds each root on its first round); the reset leaves
+// zero request offsets and a zero summary behind
+static int analysis_start(cb200_analysis *A, int n, const uint64_t *states, int seed) {
+  cb200_trainer *t = A->t;
+  A->counters[0] = A->counters[1] = 0;
+  t->P.num_games = n;
+  int rc = cb200_trainer_reset(t, seed);
+  if (rc != CB200_OK) return rc;
+  CB_CUDA(cudaMemcpyAsync(A->d_roots, states, (size_t)n * sizeof(ulonglong2), cudaMemcpyHostToDevice, cur_stream()));
+  return CB200_OK;
+}
+
+// One round of k_analysis_iterate; the answers of position g start at row offs[g]:
+// eval[row], probs[row * prs + move * pcs].
+static int analysis_launch(cb200_analysis *A, const float *eval, const float *probs, long prs, long pcs,
+                           bool want_evals) {
+  cb200_trainer *t = A->t;
+  const AnalysisOut out{A->d_moves, A->d_results, A->d_values, A->d_visits, want_evals ? A->d_evals : nullptr};
+  const int grid = (t->P.num_games + kTreeWarps - 1) / kTreeWarps;
+  k_analysis_iterate<<<grid, kTreeWarps * 32, 0, cur_stream()>>>(t->P, A->max_searches, A->d_roots, eval, probs,
+                                                                 prs, pcs, t->d_offs, out);
+  CB_LAUNCHED();
+  CB_CUDA(cudaGetLastError());
+  ++t->iterations_done;
+  return CB200_OK;
+}
+
+// Outputs of the finished positions to the caller's host buffers, then the counters (the counter
+// read-back synchronises the stream).
+static int analysis_copy_out(cb200_analysis *A, int32_t *moves, int32_t *results, float *values, int32_t *visits,
+                             float *evals) {
+  cb200_trainer *t = A->t;
+  const size_t n = (size_t)t->P.num_games;
+  cudaStream_t st = cur_stream();
+  CB_CUDA(cudaMemcpyAsync(moves, A->d_moves, n * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+  CB_CUDA(cudaMemcpyAsync(results, A->d_results, n * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+  CB_CUDA(cudaMemcpyAsync(values, A->d_values, n * sizeof(float), cudaMemcpyDeviceToHost, st));
+  CB_CUDA(cudaMemcpyAsync(visits, A->d_visits, n * CB200_NUM_MOVES * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+  if (evals)
+    CB_CUDA(cudaMemcpyAsync(evals, A->d_evals, n * CB200_NUM_MOVES * sizeof(float), cudaMemcpyDeviceToHost, st));
+  int64_t c4[4];
+  int rc = cb200_trainer_counters(t, c4);
+  if (rc != CB200_OK) return rc;
+  A->counters[0] = c4[0], A->counters[1] = c4[2];
+  return CB200_OK;
+}
 
 cb200_analysis *cb200_analysis_create(int max_positions, int max_searches, int searches_per_eval, float c_puct,
                                       float epsilon) {
@@ -2295,27 +2364,17 @@ int cb200_analysis_run(cb200_analysis *A, int n, const uint64_t *states, int see
                        int32_t *results, float *values, int32_t *visits, float *evals) {
   last_error_ref().clear();
   if (!A) return set_error(CB200_ERR_ARG, "null analysis");
-  if (n <= 0 || n > A->max_positions)
-    return set_error(CB200_ERR_ARG, "cb200_analysis_run: n must be in [1, max_positions]");
-  if (!states || !moves || !results || !values || !visits)
+  A->session = cb200_analysis::kNoSession;  // a run discards an open session
+  if (!moves || !results || !values || !visits)
     return set_error(CB200_ERR_ARG, "cb200_analysis_run: null states / moves / results / values / visits");
-  for (int i = 0; i < n; ++i)
-    if (!valid_state(states[2 * i], states[2 * i + 1]))
-      return set_error(CB200_ERR_ARG, "cb200_analysis_run: state " + std::to_string(i) + " is not a valid cstate");
+  int rc = analysis_check_states(A, n, states, "cb200_analysis_run");
+  if (rc != CB200_OK) return rc;
   if (A->net.precision < 0) return set_error(CB200_ERR_STATE, "cb200_analysis_run: no weights set");
   cb200_trainer *t = A->t;
-  int rc = guard(t);
-  if (rc != CB200_OK) return rc;
+  if ((rc = guard(t)) != CB200_OK) return rc;
   if ((rc = resident_net_upload(A->net)) != CB200_OK) return rc;
-  A->counters[0] = A->counters[1] = 0;
-  // positions [0, n) become games [0, n) of the trainer: seeds = outputs 0 .. n-1 of mt19937(seed),
-  // fresh control blocks and trees (the kernel builds each root on its first round)
-  t->P.num_games = n;
-  if ((rc = cb200_trainer_reset(t, seed)) != CB200_OK) return rc;
+  if ((rc = analysis_start(A, n, states, seed)) != CB200_OK) return rc;
   cudaStream_t st = cur_stream();
-  CB_CUDA(cudaMemcpyAsync(A->d_roots, states, (size_t)n * sizeof(ulonglong2), cudaMemcpyHostToDevice, st));
-  const AnalysisOut out{A->d_moves, A->d_results, A->d_values, A->d_visits, evals ? A->d_evals : nullptr};
-  const int grid = (n + kTreeWarps - 1) / kTreeWarps;
   // every round completes at least one search or the turn of each live position
   const int max_rounds = A->max_searches + 8;
   for (int round = 0;; ++round) {
@@ -2331,29 +2390,170 @@ int cb200_analysis_run(cb200_analysis *A, int n, const uint64_t *states, int see
     CB_LAUNCHED();
     long prs = 0, pcs = 0;
     if ((rc = resident_net_launch(A->net, t, t->d_packed, prs, pcs)) != CB200_OK) return rc;
-    k_analysis_iterate<<<grid, kTreeWarps * 32, 0, st>>>(t->P, A->max_searches, A->d_roots, t->d_eval,
-                                                          t->d_probs, prs, pcs, t->d_offs, out);
-    CB_LAUNCHED();
-    CB_CUDA(cudaGetLastError());
-    ++t->iterations_done;
+    if ((rc = analysis_launch(A, t->d_eval, t->d_probs, prs, pcs, evals != nullptr)) != CB200_OK) return rc;
   }
-  CB_CUDA(cudaMemcpyAsync(moves, A->d_moves, (size_t)n * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-  CB_CUDA(cudaMemcpyAsync(results, A->d_results, (size_t)n * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-  CB_CUDA(cudaMemcpyAsync(values, A->d_values, (size_t)n * sizeof(float), cudaMemcpyDeviceToHost, st));
-  CB_CUDA(cudaMemcpyAsync(visits, A->d_visits, (size_t)n * CB200_NUM_MOVES * sizeof(int32_t),
-                          cudaMemcpyDeviceToHost, st));
-  if (evals)
-    CB_CUDA(cudaMemcpyAsync(evals, A->d_evals, (size_t)n * CB200_NUM_MOVES * sizeof(float),
-                            cudaMemcpyDeviceToHost, st));
-  int64_t c4[4];
-  if ((rc = cb200_trainer_counters(t, c4)) != CB200_OK) return rc;  // synchronises the stream
-  A->counters[0] = c4[0], A->counters[1] = c4[2];
+  return analysis_copy_out(A, moves, results, values, visits, evals);
+}
+
+// ---- external-evaluator protocol: the rounds of cb200_analysis_run with the caller's network ----
+// begin, then until do_iteration returns 1: num_requests, write_requests, evaluate, do_iteration.
+// One summary read-back per do_iteration; write_requests reuses the offsets that read-back left.
+
+// Common entry of the session calls after their argument checks: an open session and the device.
+static int analysis_session(cb200_analysis *A, const char *who) {
+  if (A->session == cb200_analysis::kNoSession)
+    return set_error(CB200_ERR_STATE, std::string(who) + ": no open session (cb200_analysis_begin)");
+  const int rc = guard(A->t);
+  if (rc == CB200_OK) return CB200_OK;
+  A->session = cb200_analysis::kNoSession;
+  return rc;
+}
+
+int cb200_analysis_begin(cb200_analysis *A, int n, const uint64_t *states, int seed) {
+  last_error_ref().clear();
+  if (!A) return set_error(CB200_ERR_ARG, "null analysis");
+  A->session = cb200_analysis::kNoSession;  // a new begin discards an open session, even when it fails
+  int rc = analysis_check_states(A, n, states, "cb200_analysis_begin");
+  if (rc != CB200_OK) return rc;
+  if ((rc = guard(A->t)) != CB200_OK) return rc;
+  if ((rc = analysis_start(A, n, states, seed)) != CB200_OK) return rc;
+  A->requests = 0;  // the first do_iteration queues the roots
+  A->session = cb200_analysis::kOpen;
   return CB200_OK;
+}
+
+int cb200_analysis_num_requests(cb200_analysis *A) {
+  last_error_ref().clear();
+  if (!A) return set_error(CB200_ERR_ARG, "null analysis");
+  const int rc = analysis_session(A, "cb200_analysis_num_requests");
+  return rc != CB200_OK ? rc : A->requests;
+}
+
+// A caller's buffer of the device forms must be device (or managed) memory of the analysis' device:
+// anything else would fault inside the kernel.
+static int check_device_buffer(const cb200_trainer *t, const void *p, const char *who, const char *what) {
+  cudaPointerAttributes at{};
+  const bool ok = cudaPointerGetAttributes(&at, p) == cudaSuccess &&
+                  (at.type == cudaMemoryTypeDevice || at.type == cudaMemoryTypeManaged) && at.device == t->device;
+  cudaGetLastError();  // a failed query leaves nothing behind for the next launch check
+  if (ok) return CB200_OK;
+  return set_error(CB200_ERR_ARG, std::string(who) + ": " + what + " is not device memory of device " +
+                                      std::to_string(t->device));
+}
+
+// Packs the pending requests (position-major, pending order within a position) into rows on the
+// current stream; host_out != nullptr copies them out and waits.
+static int analysis_write_requests(cb200_analysis *A, float *rows, float *host_out, const char *who) {
+  int rc = analysis_session(A, who);
+  if (rc != CB200_OK || A->requests == 0) return rc;
+  cb200_trainer *t = A->t;
+  if (!host_out && (rc = check_device_buffer(t, rows, who, "rows_device")) != CB200_OK) return rc;
+  cudaStream_t st = cur_stream();
+  k_pack_requests<<<(t->P.num_games + 7) / 8, 256, 0, st>>>(t->P, -1, t->d_offs, rows, nullptr);
+  CB_LAUNCHED();
+  CB_CUDA(cudaGetLastError());
+  if (host_out) {
+    CB_CUDA(cudaMemcpyAsync(host_out, rows, (size_t)A->requests * CB200_STATE_SIZE * sizeof(float),
+                            cudaMemcpyDeviceToHost, st));
+    CB_CUDA(cudaStreamSynchronize(st));
+  }
+  return CB200_OK;
+}
+
+int cb200_analysis_write_requests(cb200_analysis *A, float *game_states) {
+  last_error_ref().clear();
+  if (!A || !game_states) return set_error(CB200_ERR_ARG, "cb200_analysis_write_requests: null analysis / game_states");
+  return analysis_write_requests(A, A->t->d_rows, game_states, "cb200_analysis_write_requests");
+}
+
+int cb200_analysis_write_requests_device(cb200_analysis *A, void *rows_device) {
+  last_error_ref().clear();
+  if (!A || !rows_device)
+    return set_error(CB200_ERR_ARG, "cb200_analysis_write_requests_device: null analysis / rows_device");
+  return analysis_write_requests(A, (float *)rows_device, nullptr, "cb200_analysis_write_requests_device");
+}
+
+// One round with the caller's row-major answers (device pointers when on_device, else host pointers
+// staged into the trainer's answer buffers), then the scan for the next round and its read-back.
+static int analysis_do_iteration(cb200_analysis *A, const float *eval, const float *probs, int rows, bool on_device,
+                                 const char *who) {
+  if (!A) return set_error(CB200_ERR_ARG, "null analysis");
+  if (rows < 0 || (rows > 0 && (!eval || !probs)))
+    return set_error(CB200_ERR_ARG, std::string(who) + ": rows < 0, or null eval / probs");
+  int rc = analysis_session(A, who);
+  if (rc != CB200_OK) return rc;
+  if (A->session == cb200_analysis::kDone) return 1;
+  const int need = A->requests;
+  if (rows < need)
+    return set_error(CB200_ERR_ARG, std::string(who) + ": " + std::to_string(rows) + " answer rows given, " +
+                                        std::to_string(need) + " requests pending");
+  cb200_trainer *t = A->t;
+  cudaStream_t st = cur_stream();
+  const float *ev = t->d_eval, *pr = t->d_probs;
+  if (need > 0 && on_device) {
+    if ((rc = check_device_buffer(t, eval, who, "eval_device")) != CB200_OK ||
+        (rc = check_device_buffer(t, probs, who, "probs_device")) != CB200_OK)
+      return rc;
+    ev = eval, pr = probs;
+  } else if (need > 0) {
+    CB_CUDA(cudaMemcpyAsync(t->d_eval, eval, (size_t)need * sizeof(float), cudaMemcpyHostToDevice, st));
+    CB_CUDA(cudaMemcpyAsync(t->d_probs, probs, (size_t)need * CB200_NUM_MOVES * sizeof(float),
+                            cudaMemcpyHostToDevice, st));
+  }
+  if ((rc = analysis_launch(A, ev, pr, CB200_NUM_MOVES, 1, true)) == CB200_OK) {
+    k_scan_requests<<<1, 1024, 0, st>>>(t->P, -1, t->d_offs, t->d_summary);
+    CB_LAUNCHED();
+    rc = fetch_summary(t);  // an overflow of any position surfaces here
+  }
+  if (rc != CB200_OK) {
+    A->session = cb200_analysis::kNoSession;
+    return rc;
+  }
+  A->requests = t->h_summary[0];
+  if (t->h_summary[1] != 0) return 0;
+  int64_t c4[4];
+  if ((rc = cb200_trainer_counters(t, c4)) != CB200_OK) {
+    A->session = cb200_analysis::kNoSession;
+    return rc;
+  }
+  A->counters[0] = c4[0], A->counters[1] = c4[2];
+  A->session = cb200_analysis::kDone;
+  return 1;
+}
+
+int cb200_analysis_do_iteration(cb200_analysis *A, const float *eval, const float *probs, int rows) {
+  last_error_ref().clear();
+  return analysis_do_iteration(A, eval, probs, rows, false, "cb200_analysis_do_iteration");
+}
+
+int cb200_analysis_do_iteration_device(cb200_analysis *A, const void *eval_device, const void *probs_device,
+                                       int rows) {
+  last_error_ref().clear();
+  return analysis_do_iteration(A, (const float *)eval_device, (const float *)probs_device, rows, true,
+                               "cb200_analysis_do_iteration_device");
+}
+
+int cb200_analysis_results(cb200_analysis *A, int32_t *moves, int32_t *results, float *values, int32_t *visits,
+                           float *evals) {
+  last_error_ref().clear();
+  if (!A || !moves || !results || !values || !visits)
+    return set_error(CB200_ERR_ARG, "cb200_analysis_results: null analysis / moves / results / values / visits");
+  int rc = analysis_session(A, "cb200_analysis_results");
+  if (rc != CB200_OK) return rc;
+  if (A->session != cb200_analysis::kDone)
+    return set_error(CB200_ERR_STATE, "cb200_analysis_results: the session is not done (do_iteration has not returned 1)");
+  return analysis_copy_out(A, moves, results, values, visits, evals);
 }
 
 int cb200_analysis_counters(cb200_analysis *A, int64_t out[2]) {
   last_error_ref().clear();
   if (!A || !out) return set_error(CB200_ERR_ARG, "null analysis / out");
+  if (A->session == cb200_analysis::kOpen) {  // the running totals of the session so far
+    int64_t c4[4];
+    const int rc = cb200_trainer_counters(A->t, c4);
+    if (rc != CB200_OK) return rc;
+    A->counters[0] = c4[0], A->counters[1] = c4[2];
+  }
   out[0] = A->counters[0], out[1] = A->counters[1];
   return CB200_OK;
 }

@@ -298,7 +298,59 @@ int cb200_analysis_set_weights(cb200_analysis *a, const float *weights, size_t n
 int cb200_analysis_run(cb200_analysis *a, int n, const uint64_t *states, int seed,
                        int32_t *moves /* [n] */, int32_t *results /* [n] */, float *values /* [n] */,
                        int32_t *visits /* [n][96] */, float *evals /* [n][96] or NULL */);
-/* out = {simulations, leaf evaluations} of the last run */
+/* External-evaluator protocol: the same searches with the caller's network instead of the resident
+ * one (no weights needed), driven like docker/choose_move.pyx drives DockerMC and like the Trainer's
+ * doIteration / writeRequests:
+ *     begin; while (!do_iteration(eval, probs, rows)) { n = num_requests; write_requests(rows[n][70]);
+ *                                                       evaluate rows -> eval[n], probs[n][96]; }
+ *     results
+ * The first do_iteration takes no answers (num_requests is 0 after begin) and queues the roots.
+ * Given the same answers, every output equals what cb200_analysis_run computes with a network that
+ * gives those answers.
+ *   begin         opens a session on states[n][2]: validation, seeds and errors of cb200_analysis_run
+ *                 (except that no weights are needed). A begin during an open session restarts it;
+ *                 a begin that fails leaves no session open.
+ *   num_requests  rows the next do_iteration reads (no device work).
+ *   write_requests  game_states[num_requests][70], position-major, then in the order the position
+ *                 queued its leaves (Trainer::writeRequests' order).
+ *   do_iteration  one round with row-major answers to the last write_requests: eval[rows],
+ *                 probs[rows][96] (probabilities need not be normalised: the search renormalises over
+ *                 the legal moves). rows = what the buffers hold; fewer than num_requests is
+ *                 CB200_ERR_ARG. Returns 1 when every position is done (and does no work once it is),
+ *                 0 if not, < 0 on error.
+ *   results       the outputs of cb200_analysis_run (evals may be NULL); CB200_ERR_STATE before
+ *                 do_iteration has returned 1. May be called again until the next begin / run.
+ * Calls other than begin without an open session are CB200_ERR_STATE; cb200_analysis_run discards
+ * an open session. Null and negative-size arguments are CB200_ERR_ARG before anything else is looked
+ * at; argument errors leave the session as it was. An error while a round runs -- CB200_ERR_OVERFLOW
+ * when a node arena overflowed, CB200_ERR_CUDA -- ends the session. Either way the object stays
+ * usable for a new begin or run. */
+int cb200_analysis_begin(cb200_analysis *a, int n, const uint64_t *states /* [n][2] */, int seed);
+int cb200_analysis_num_requests(cb200_analysis *a);
+int cb200_analysis_write_requests(cb200_analysis *a, float *game_states /* [num_requests][70] */);
+int cb200_analysis_do_iteration(cb200_analysis *a, const float *eval /* [rows] */,
+                                const float *probs /* [rows][96] */, int rows);
+int cb200_analysis_results(cb200_analysis *a, int32_t *moves /* [n] */, int32_t *results /* [n] */,
+                           float *values /* [n] */, int32_t *visits /* [n][96] */,
+                           float *evals /* [n][96] or NULL */);
+/* Device forms, for an evaluator that lives on the GPU: the same calls on device memory, ordered on
+ * the library's current stream (cb200_set_stream) and never staged through the host.
+ *   write_requests_device  packs the rows (float [num_requests][70]) into rows_device and returns
+ *                 without waiting: the rows are complete in the order of the current stream, so work
+ *                 queued on that stream may read them directly; another stream must wait for it first
+ *                 (an event recorded on the current stream after the call, or a synchronisation).
+ *   do_iteration_device  the kernel reads eval_device[rows] and probs_device[rows][96] (float,
+ *                 row-major) in place. The caller's writes to them must be complete in the order of
+ *                 the current stream when the call is made: issued on that stream, or on a stream the
+ *                 current stream has been made to wait for. The call returns after the round
+ *                 (it reads back the summary), so the buffers may be reused as soon as it returns.
+ * A buffer that is not device (or managed) memory of the device the analysis was created on is
+ * CB200_ERR_ARG. */
+int cb200_analysis_write_requests_device(cb200_analysis *a, void *rows_device);
+int cb200_analysis_do_iteration_device(cb200_analysis *a, const void *eval_device, const void *probs_device,
+                                       int rows);
+/* out = {simulations, leaf evaluations} of the last run or session; while a session is open, its
+ * running totals so far (like the oracle's counters). */
 int cb200_analysis_counters(cb200_analysis *a, int64_t out[2]);
 /* Structural check of cstates given by a caller (no device needed): byte 6 (side to move) 0 or 1,
  * byte 7 zero, at most 4 pieces of a kind in either hand, frozen squares occupied, and for every

@@ -143,6 +143,23 @@ class Analysis {
            int32_t *visits, float *evals = nullptr) {
     check(cb200_analysis_run(h_, n, states, seed, moves, results, values, visits, evals));
   }
+
+  /* External-evaluator protocol (cb200_analysis_begin .. _results): the caller's network answers
+   * the requests between rounds, as docker/choose_move.pyx does for DockerMC. */
+  void begin(int n, const uint64_t *states, int seed) { check(cb200_analysis_begin(h_, n, states, seed)); }
+  int num_requests() { return check(cb200_analysis_num_requests(h_)); }
+  void writeRequests(float *game_states) { check(cb200_analysis_write_requests(h_, game_states)); }
+  bool doIteration(const float *eval, const float *probs, int rows) {
+    return check(cb200_analysis_do_iteration(h_, eval, probs, rows)) == 1;
+  }
+  void results(int32_t *moves, int32_t *results, float *values, int32_t *visits, float *evals = nullptr) {
+    check(cb200_analysis_results(h_, moves, results, values, visits, evals));
+  }
+  /* device buffers, on the library's current stream (see corintho_b200.h) */
+  void writeRequestsDevice(void *rows_device) { check(cb200_analysis_write_requests_device(h_, rows_device)); }
+  bool doIterationDevice(const void *eval_device, const void *probs_device, int rows) {
+    return check(cb200_analysis_do_iteration_device(h_, eval_device, probs_device, rows)) == 1;
+  }
   cb200_analysis *handle() { return h_; }
 
  private:
