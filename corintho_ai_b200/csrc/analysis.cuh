@@ -1,6 +1,6 @@
 // Analysis: the reference's DockerMC (corintho_ai/cpp/src/dockermc.cpp) for a batch of given
-// positions. Position g is searched by one testing-mode TrainMC on the per-game storage of an
-// internal trainer (one "game" per position): its tree of the side to move starts as a single node
+// positions. Position g is searched by one testing-mode TrainMC on the analysis' per-game storage
+// (one "game" per position, engine.cu's GameStore): its tree of the side to move starts as a single node
 // holding the caller's position, TrainMC::doIteration runs until the turn is complete, the root
 // statistics are written out and TrainMC::chooseMove picks the move. Nothing continues into the
 // opponent's turn, which is why this is its own kernel rather than a branch of run_game or

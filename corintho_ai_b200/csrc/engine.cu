@@ -126,16 +126,39 @@ __global__ void __launch_bounds__(256)
 }  // namespace cb200
 
 // ==============================================================================================
-struct cb200_trainer {
+// The per-game device storage of one driver (Trainer, Tourney or Analysis): control blocks, trees
+// and node arenas, request and answer buffers, the summary read-back and the per-game text logs.
+struct GameStore {
   int device = 0;
   TreeParams P{};
   int iterations_done = 0;
-  int stagger_div = 1;
-  std::string log_folder;
   size_t cap = 0;  // num_games * spe request rows
   float *d_eval = nullptr, *d_probs = nullptr, *d_rows = nullptr;
   ulonglong2 *d_packed = nullptr;
-  int32_t *d_offs = nullptr, *d_summary = nullptr, *d_soff = nullptr;
+  int32_t *d_offs = nullptr, *d_summary = nullptr;
+  int32_t *h_summary = nullptr;  // pinned
+  std::vector<int32_t> h_ctl;
+  // text logs: the records of log area i (P.log_buf) are appended to log_paths[i]
+  std::vector<std::string> log_paths;
+  std::vector<std::unique_ptr<std::ofstream>> log_files;  // null = could not open
+  std::vector<int> log_written;                           // records already formatted
+  std::vector<int32_t> h_log_count;
+  std::vector<uint32_t> h_log_rec;
+};
+
+// A device-resident network. Precision codes of cb200_trainer_set_weights: 0 fp32; 1 bf16, 2 fp16,
+// 3 bf16x3 on the tensor-core kernel, which writes its answers move-major.
+struct Net {
+  int precision = -1;  // -1 = no weights on the device
+  NetF32 f32;
+  NetTC tc;
+  bool tensor_core() const { return precision > 0; }
+};
+
+struct cb200_trainer : GameStore {
+  int stagger_div = 1;
+  std::string log_folder;
+  int32_t *d_soff = nullptr;
   float *d_samp = nullptr;  // cached output buffer of write_samples
   size_t samp_rows = 0;
   float *d_raw = nullptr;   // cached [rows][102] buffer of raw_samples_device
@@ -144,12 +167,7 @@ struct cb200_trainer {
   size_t gath_floats = 0;
   int32_t *d_gcounts = nullptr, *h_gcounts = nullptr;  // [world + 1] rows per rank (+ own count)
   int gcounts_world = 0;    // communicator size the count buffers were allocated for
-  int32_t *h_summary = nullptr;  // pinned
-  NetF32 net32[2];
-  NetTC nettc[2];
-  int precision[2] = {-1, -1};
-  std::vector<int32_t> h_ctl;
-  int seed = 0;
+  Net net[2];
   // fused mode: games are split into independent stream groups (no lock-step across groups)
   int n_groups = 1;
   // the rest of the fused loop's schedule, read from the environment once, at creation
@@ -165,11 +183,6 @@ struct cb200_trainer {
   std::vector<int> g_begin, g_end;
   int32_t *d_gctr = nullptr;  // [n_groups][8] device counters (TreeParams::group_ctr)
   int32_t *h_gctr = nullptr;  // pinned mirror
-  // per-game text logs of the first num_logged games (trainer.cpp:243-250)
-  std::vector<std::unique_ptr<std::ofstream>> log_files;  // [P.n_logged]; null = could not open
-  std::vector<int> log_written;                           // records already formatted
-  std::vector<int32_t> h_log_count;
-  std::vector<uint32_t> h_log_rec;
   // persistent fused tail (persistent.cuh): CTA-private request/answer rows and the live list
   int ps_ctas = 0;                 // CTAs the device holds (one per SM)
   int32_t *d_ps_list = nullptr;    // [num_games]
@@ -334,16 +347,18 @@ int game_error(int code) {
                          "CB200_ARENA_NODES) or reached an impossible state");
 }
 
-int fetch_summary(cb200_trainer *t) {
-  CB_CUDA(cudaMemcpyAsync(t->h_summary, t->d_summary, 4 * sizeof(int32_t), cudaMemcpyDeviceToHost,
+int store_fetch_summary(GameStore &s) {
+  CB_CUDA(cudaMemcpyAsync(s.h_summary, s.d_summary, 4 * sizeof(int32_t), cudaMemcpyDeviceToHost,
                           cur_stream()));
   CB_CUDA(cudaStreamSynchronize(cur_stream()));
-  if (t->profiling) {
-    int rc = prof_drain(t);
-    if (rc != CB200_OK) return rc;
-  }
-  if (t->h_summary[2] != 0) return game_error(t->h_summary[2]);
+  if (s.h_summary[2] != 0) return game_error(s.h_summary[2]);
   return CB200_OK;
+}
+
+int fetch_summary(cb200_trainer *t) {
+  const int rc = store_fetch_summary(*t);
+  if (rc != CB200_OK || !t->profiling) return rc;
+  return prof_drain(t);
 }
 
 // probs_move_major: answers were written by the tensor-core network as [96][cap]
@@ -369,22 +384,46 @@ int pack(cb200_trainer *t, int to_play, float *d_rows, ulonglong2 *d_packed) {
   return CB200_OK;
 }
 
-int run_net(cb200_trainer *t, int model, const ulonglong2 *d_states, const int32_t *d_n,
-            int n_static, int n_max) {
-  ProfScope ps(t, 2);
-  if (t->precision[model] == 0)
-    return launch_mlp_f32(t->net32[model], d_states, d_n, n_static, n_max, t->d_eval, t->d_probs);
-  if (t->precision[model] == 1)
-    return launch_mlp_tc(t->nettc[model], d_states, d_n, n_static, n_max, t->d_eval, t->d_probs,
-                         (int)t->cap);
-  return set_error(CB200_ERR_STATE, "no weights set for this model (cb200_trainer_set_weights)");
+// The validation of the three set_weights calls; `who` names the call in the message.
+int check_weights(const float *weights, size_t n_floats, int precision, const char *who) {
+  if (!weights || n_floats != kNetWeightFloats || precision < 0 || precision > 3)
+    return set_error(CB200_ERR_ARG, std::string(who) + ": bad arguments (127997 floats, precision 0|1|2|3)");
+  return CB200_OK;
+}
+
+int net_upload(Net &n, const float *weights, int precision) {
+  // tensor-core operand modes: precision 1 -> bf16, 2 -> fp16, 3 -> bf16x3 (hi + lo operands)
+  const int rc = precision == 0 ? net_f32_upload(n.f32, weights)
+                                : net_tc_upload(n.tc, weights, precision == 1 ? 0 : (precision == 2 ? 1 : 2));
+  if (rc == CB200_OK) n.precision = precision;
+  return rc;
+}
+
+void net_free(Net &n) {
+  cudaFree(n.f32.w);
+  n.f32.w = nullptr;
+  net_tc_free(n.tc);
+}
+
+// Evaluates the cstates states[0 .. n) on the current stream, n = *d_n (n_static when d_n is null),
+// at most n_max. The answer of row k for move m is then at probs[k * 96 + m] from the fp32 kernel and
+// at probs[m * ld + k] from the tensor-core kernel.
+int net_launch(const Net &n, const ulonglong2 *states, const int32_t *d_n, int n_static, int n_max, float *eval,
+               float *probs, int ld) {
+  if (n.precision == 0) return launch_mlp_f32(n.f32, states, d_n, n_static, n_max, eval, probs);
+  if (n.tensor_core()) return launch_mlp_tc(n.tc, states, d_n, n_static, n_max, eval, probs, ld);
+  return set_error(CB200_ERR_STATE, "no weights set for this model");
+}
+
+int store_guard(const GameStore &s) {
+  last_error_ref().clear();  // a message always belongs to the call that failed last
+  CB_CUDA(cudaSetDevice(s.device));
+  return CB200_OK;
 }
 
 int guard(cb200_trainer *t) {
-  last_error_ref().clear();  // a message always belongs to the call that failed last
   if (!t) return set_error(CB200_ERR_ARG, "null trainer");
-  CB_CUDA(cudaSetDevice(t->device));
-  return CB200_OK;
+  return store_guard(*t);
 }
 
 }  // namespace
@@ -522,23 +561,22 @@ static void format_move_choice(std::ostream &os, const uint32_t *rec) {
 }
 
 // append the records written since the last call to the log files
-static int drain_logs(cb200_trainer *t) {
-  TreeParams &P = t->P;
-  if (P.n_logged <= 0) return CB200_OK;
-  t->h_log_count.resize(P.n_logged);
-  CB_CUDA(cudaMemcpy(t->h_log_count.data(), P.log_count, (size_t)P.n_logged * sizeof(int32_t),
-                     cudaMemcpyDeviceToHost));
-  for (int g = 0; g < P.n_logged; ++g) {
-    const int have = t->h_log_count[g], done = t->log_written[g];
+static int store_drain_logs(GameStore &s) {
+  const int n_log = (int)s.log_files.size();
+  if (n_log == 0) return CB200_OK;
+  s.h_log_count.resize(n_log);
+  CB_CUDA(cudaMemcpy(s.h_log_count.data(), s.P.log_count, (size_t)n_log * sizeof(int32_t), cudaMemcpyDeviceToHost));
+  for (int g = 0; g < n_log; ++g) {
+    const int have = s.h_log_count[g], done = s.log_written[g];
     if (have <= done) continue;
-    t->log_written[g] = have;
-    if (!t->log_files[g]) continue;
-    t->h_log_rec.resize((size_t)(have - done) * kLogWords);
-    CB_CUDA(cudaMemcpy(t->h_log_rec.data(), P.log_buf + ((size_t)g * kLogMaxMoves + done) * kLogWords,
-                       t->h_log_rec.size() * sizeof(uint32_t), cudaMemcpyDeviceToHost));
+    s.log_written[g] = have;
+    if (!s.log_files[g]) continue;
+    s.h_log_rec.resize((size_t)(have - done) * kLogWords);
+    CB_CUDA(cudaMemcpy(s.h_log_rec.data(), s.P.log_buf + ((size_t)g * kLogMaxMoves + done) * kLogWords,
+                       s.h_log_rec.size() * sizeof(uint32_t), cudaMemcpyDeviceToHost));
     for (int k = 0; k < have - done; ++k)
-      format_log_record(*t->log_files[g], t->h_log_rec.data() + (size_t)k * kLogWords);
-    t->log_files[g]->flush();
+      format_log_record(*s.log_files[g], s.h_log_rec.data() + (size_t)k * kLogWords);
+    s.log_files[g]->flush();
   }
   return CB200_OK;
 }
@@ -556,28 +594,99 @@ __global__ void k_seed_mt(int n, const uint32_t *__restrict__ seeds, uint32_t *_
   }
 }
 
-// (Re)open log_folder/game_<i>.txt for the logged games of this shard, truncating like the
-// reference's ofstream(..., out) does for every new Trainer (trainer.cpp:243-250); a missing
-// folder silently produces no log.
-static void open_log_files(cb200_trainer *t) {
-  t->log_files.clear();
-  for (int i = 0; i < t->P.n_logged; ++i) {
-    auto f = std::make_unique<std::ofstream>(
-        t->log_folder + "/game_" + std::to_string(t->P.first_game + i) + ".txt", std::ofstream::out);
-    if (!f->is_open()) f.reset();
-    t->log_files.push_back(std::move(f));
+// Allocates the storage of num_games games whose searches take at most max_searches simulations and
+// spe requests per iteration, and uploads the rule tables. c_puct > 0 builds the selection's sqrt
+// table (a tourney's sides bring their own c_puct). The sample buffers exist only with `samples`
+// (training-mode games write them). log_paths names the file of each text-log area. On failure the
+// caller frees the store.
+static int store_create(GameStore &s, int num_games, int max_searches, int spe, float c_puct, float epsilon,
+                        int testing, bool samples, std::vector<std::string> log_paths) {
+  if (cudaGetDevice(&s.device) != cudaSuccess || upload_tables_once() != CB200_OK)
+    return last_error_ref().empty() ? set_error(CB200_ERR_CUDA, "no usable CUDA device") : CB200_ERR_CUDA;
+  TreeParams &P = s.P;
+  P.num_games = num_games, P.first_game = 0, P.total_games = num_games;
+  P.max_searches = max_searches, P.spe = spe;
+  P.c_puct = c_puct, P.epsilon = epsilon, P.testing = testing ? 1 : 0;
+  // arena budget: kept subtree + max_searches new nodes per move with head-room; a game that
+  // still overflows fails loudly (CB200_ERR_OVERFLOW). ~28 slots/node on average.
+  long long nodes = (long long)max_searches * 5 / 2 + 96;
+  long long words = nodes * (8 + 4 * 28);
+  if (const char *env = getenv("CB200_ARENA_NODES")) {
+    words = atoll(env) * (8 + 4 * 28);
+  } else {
+    // Larger arenas make in-place re-rooting the common case (compaction only when room runs
+    // out). The node arenas of one store take at most an explicit budget -- 48 GiB by default,
+    // CB200_ARENA_BUDGET_MB overrides -- capped at 16 moves' worth of nodes per arena and never
+    // below the minimum above; a co-resident store keeps the rest of the HBM.
+    long long budget_bytes = 48ll << 30;
+    if (const char *env = getenv("CB200_ARENA_BUDGET_MB")) budget_bytes = atoll(env) << 20;
+    long long budget = budget_bytes / ((long long)num_games * 3 * 4);
+    const long long cap = (long long)max_searches * 16 * (8 + 4 * 28);
+    if (budget > cap) budget = cap;
+    if (budget > words) words = budget;
   }
+  words = (words + 3) & ~3ll;
+  if (words < 1024) words = 1024;
+  if (words > 0x7fffff00ll) words = 0x7fffff00ll;
+  P.arena_words = (uint32_t)words;
+  const size_t Gn = (size_t)num_games;
+  s.cap = Gn * spe;
+  if (s.cap * CB200_NUM_MOVES >= (size_t)1 << 31)  // the kernels index answers with 31 bits
+    return set_error(CB200_ERR_ARG, "num_games * searches_per_eval too large for one device batch");
+  bool ok = dmalloc(&P.arenas, Gn * 3 * P.arena_words) == CB200_OK &&
+            dmalloc(&P.ctl, Gn * kCtlWords) == CB200_OK &&
+            dmalloc(&P.tree, Gn * 2 * kTreeCtlWords) == CB200_OK &&
+            dmalloc(&P.mt, Gn * 624) == CB200_OK &&
+            dmalloc(&P.pending, s.cap * kPendWords) == CB200_OK &&
+            dmalloc(&P.leaf_state, s.cap) == CB200_OK &&
+            (!samples || (dmalloc(&P.sample_state, Gn * kMaxSamples) == CB200_OK &&
+                          dmalloc(&P.sample_probs, Gn * kMaxSamples * CB200_NUM_MOVES) == CB200_OK)) &&
+            dmalloc(&P.counters, Gn * 4) == CB200_OK &&
+            // (+ kAnswerSlack rows: a fused tourney reads its answers at the reference's own offsets,
+            // tourney.cpp:54-62, which may run a few rows past the requests of the call)
+            dmalloc(&s.d_eval, s.cap + kAnswerSlack) == CB200_OK &&
+            dmalloc(&s.d_probs, (s.cap + kAnswerSlack) * CB200_NUM_MOVES) == CB200_OK &&
+            dmalloc(&s.d_rows, s.cap * CB200_STATE_SIZE) == CB200_OK &&
+            dmalloc(&s.d_packed, s.cap) == CB200_OK && dmalloc(&s.d_offs, Gn) == CB200_OK &&
+            dmalloc(&s.d_summary, 4) == CB200_OK &&
+            cudaMallocHost((void **)&s.h_summary, 4 * sizeof(int32_t)) == cudaSuccess;
+  if (ok && c_puct > 0.0f) {
+    // c_puct * sqrt(visits) exactly as trainmc.cpp:568 evaluates it (double sqrt, double product,
+    // one rounding to float); IEEE sqrt is correctly rounded on host and device alike
+    float *d_vsqrt = nullptr;
+    std::vector<float> vs(kVsqrtCap);
+    for (int i = 0; i < kVsqrtCap; ++i)
+      vs[i] = (float)((double)c_puct * sqrt((double)(float)i));
+    ok = dmalloc(&d_vsqrt, (size_t)kVsqrtCap) == CB200_OK &&
+         cudaMemcpy(d_vsqrt, vs.data(), sizeof(float) * kVsqrtCap, cudaMemcpyHostToDevice) ==
+             cudaSuccess;
+    P.vsqrt = d_vsqrt;
+  }
+  const size_t n_log = log_paths.size();
+  if (ok && n_log > 0) {
+    ok = dmalloc(&P.log_buf, n_log * kLogMaxMoves * kLogWords) == CB200_OK && dmalloc(&P.log_count, n_log) == CB200_OK;
+    s.log_written.assign(n_log, 0);
+  }
+  s.log_paths = std::move(log_paths);
+  if (!ok) return last_error_ref().empty() ? set_error(CB200_ERR_CUDA, "allocation failed") : CB200_ERR_CUDA;
+  P.game_begin = 0, P.game_end = num_games, P.group_row0 = 0, P.group_ctr = nullptr;
+  P.live_list = nullptr, P.live_count = nullptr;
+  P.packed = s.d_packed;
+  P.phase_prof = nullptr;
+  return CB200_OK;
 }
 
-// initialisation: per-game seeds (trainer.cpp:238-256) from the host generator, MT19937 states
-// expanded on the device, control blocks
-static int init_state(cb200_trainer *t) {
-  TreeParams &P = t->P;
-  const size_t Gn = (size_t)P.num_games;
+// Games [0, n) start afresh: per-game seeds (trainer.cpp:238-256) = the outputs first_game,
+// first_game + 1, ... of mt19937(seed), MT19937 states expanded on the device, fresh control blocks
+// and trees, zero counters, request offsets, summary and answers, and the text logs started again.
+static int store_reset(GameStore &s, int n, int seed) {
+  TreeParams &P = s.P;
+  P.num_games = n;
+  const size_t Gn = (size_t)n;
   std::vector<int32_t> ctl(Gn * kCtlWords, 0), tree(Gn * 2 * kTreeCtlWords, 0);
   std::vector<uint32_t> seeds(Gn);
   HostMT gen;
-  gen.seed((uint32_t)t->seed);
+  gen.seed((uint32_t)seed);
   for (int i = 0; i < P.first_game; ++i) gen.next();
   for (size_t g = 0; g < Gn; ++g) {
     seeds[g] = gen.next();
@@ -592,40 +701,78 @@ static int init_state(cb200_trainer *t) {
       tw[TW_ROOT_ALLV] = 1;
     }
   }
-  cudaStream_t s = cur_stream();
-  CB_CUDA(cudaMemcpyAsync(P.ctl, ctl.data(), ctl.size() * 4, cudaMemcpyHostToDevice, s));
-  CB_CUDA(cudaMemcpyAsync(P.tree, tree.data(), tree.size() * 4, cudaMemcpyHostToDevice, s));
+  cudaStream_t st = cur_stream();
+  CB_CUDA(cudaMemcpyAsync(P.ctl, ctl.data(), ctl.size() * 4, cudaMemcpyHostToDevice, st));
+  CB_CUDA(cudaMemcpyAsync(P.tree, tree.data(), tree.size() * 4, cudaMemcpyHostToDevice, st));
   // the seeds travel through the (still unused) request-offset buffer
-  CB_CUDA(cudaMemcpyAsync(t->d_offs, seeds.data(), Gn * sizeof(uint32_t), cudaMemcpyHostToDevice, s));
-  k_seed_mt<<<(int)((Gn + 127) / 128), 128, 0, s>>>((int)Gn, (const uint32_t *)t->d_offs, P.mt);
+  CB_CUDA(cudaMemcpyAsync(s.d_offs, seeds.data(), Gn * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
+  k_seed_mt<<<(int)((Gn + 127) / 128), 128, 0, st>>>((int)Gn, (const uint32_t *)s.d_offs, P.mt);
   CB_LAUNCHED();
   CB_CUDA(cudaGetLastError());
-  CB_CUDA(cudaMemsetAsync(P.counters, 0, Gn * 4 * sizeof(long long), s));
-  CB_CUDA(cudaMemsetAsync(t->d_offs, 0, Gn * sizeof(int32_t), s));
-  CB_CUDA(cudaMemsetAsync(t->d_summary, 0, 4 * sizeof(int32_t), s));
+  CB_CUDA(cudaMemsetAsync(P.counters, 0, Gn * 4 * sizeof(long long), st));
+  CB_CUDA(cudaMemsetAsync(s.d_offs, 0, Gn * sizeof(int32_t), st));
+  CB_CUDA(cudaMemsetAsync(s.d_summary, 0, 4 * sizeof(int32_t), st));
   // The whole answer buffers, slack rows included: a fused two-model tourney reads rows that no
   // evaluation of the run has written yet (the offsets of tourney.cpp:54-62), and they must read as
   // the zeros of the reference loop's fresh buffers. The tensor-core network's move-major layout
   // (leading dimension cap + kAnswerSlack) spreads every row over the whole buffer, so zeroing only
   // cap rows' worth would leave the high move ids of every row to whatever the memory held before.
-  CB_CUDA(cudaMemsetAsync(t->d_eval, 0, (t->cap + kAnswerSlack) * sizeof(float), s));
-  CB_CUDA(cudaMemsetAsync(t->d_probs, 0, (t->cap + kAnswerSlack) * CB200_NUM_MOVES * sizeof(float), s));
-  CB_CUDA(cudaMemsetAsync(t->d_gctr, 0, (size_t)t->n_groups * 8 * sizeof(int32_t), s));
-  CB_CUDA(cudaStreamSynchronize(s));
-  if (P.n_logged > 0) {
-    CB_CUDA(cudaMemset(P.log_count, 0, (size_t)P.n_logged * sizeof(int32_t)));
-    std::fill(t->log_written.begin(), t->log_written.end(), 0);
-    open_log_files(t);  // a run after reset() starts its transcripts afresh
+  CB_CUDA(cudaMemsetAsync(s.d_eval, 0, (s.cap + kAnswerSlack) * sizeof(float), st));
+  CB_CUDA(cudaMemsetAsync(s.d_probs, 0, (s.cap + kAnswerSlack) * CB200_NUM_MOVES * sizeof(float), st));
+  CB_CUDA(cudaStreamSynchronize(st));
+  if (!s.log_paths.empty()) {
+    CB_CUDA(cudaMemset(P.log_count, 0, s.log_paths.size() * sizeof(int32_t)));
+    std::fill(s.log_written.begin(), s.log_written.end(), 0);
+    // truncated like the reference's ofstream(..., out) for every new Trainer or Tourney
+    // (trainer.cpp:243-250, tourney.cpp:88-93); a missing folder silently produces no log
+    s.log_files.clear();
+    for (const std::string &path : s.log_paths) {
+      auto f = std::make_unique<std::ofstream>(path, std::ofstream::out);
+      if (!f->is_open()) f.reset();
+      s.log_files.push_back(std::move(f));
+    }
   }
-  t->iterations_done = 0;
-  t->ps_active = false, t->ps_from_lockstep = false, t->ps_n = 0, t->ps_cur = 0;
-  if (t->stream_on) {
-    CB_CUDA(cudaStreamSynchronize(t->st_stream));
-    CB_CUDA(cudaMemset(t->d_emitted, 0, Gn * sizeof(int32_t)));
-    CB_CUDA(cudaMemset(t->d_st_ctr, 0, 2 * sizeof(int32_t)));
-    t->st_pending = false, t->st_copied = 0, t->st_round = 0;
-    t->h_st_ctr[0] = t->h_st_ctr[1] = 0;
-  }
+  s.iterations_done = 0;
+  return CB200_OK;
+}
+
+static void store_free(GameStore &s) {
+  TreeParams &P = s.P;
+  cudaFree((void *)P.vsqrt), cudaFree(P.arenas), cudaFree(P.ctl), cudaFree(P.tree), cudaFree(P.mt), cudaFree(P.pending);
+  cudaFree(P.leaf_state), cudaFree(P.sample_state), cudaFree(P.sample_probs), cudaFree(P.counters);
+  cudaFree(P.log_buf), cudaFree(P.log_count);
+  cudaFree(s.d_eval), cudaFree(s.d_probs), cudaFree(s.d_rows), cudaFree(s.d_packed);
+  cudaFree(s.d_offs), cudaFree(s.d_summary);
+  if (s.h_summary) cudaFreeHost(s.h_summary);
+  s = GameStore();
+}
+
+static int store_fetch_ctl(GameStore &s) {
+  s.h_ctl.resize((size_t)s.P.num_games * kCtlWords);
+  CB_CUDA(cudaStreamSynchronize(cur_stream()));
+  CB_CUDA(cudaMemcpy(s.h_ctl.data(), s.P.ctl, s.h_ctl.size() * 4, cudaMemcpyDeviceToHost));
+  return CB200_OK;
+}
+
+// out = {simulations, moves, leaf evaluations, iterations}; *searches = the searches so far
+static int store_counters(const GameStore &s, int64_t out[4], long long *searches = nullptr) {
+  std::vector<long long> h((size_t)s.P.num_games * 4);
+  CB_CUDA(cudaStreamSynchronize(cur_stream()));
+  CB_CUDA(cudaMemcpy(h.data(), s.P.counters, h.size() * sizeof(long long), cudaMemcpyDeviceToHost));
+  out[0] = out[1] = out[2] = 0;
+  long long n_searches = 0;
+  for (int g = 0; g < s.P.num_games; ++g)
+    out[0] += h[4 * g], out[1] += h[4 * g + 1], out[2] += h[4 * g + 2], n_searches += h[4 * g + 3];
+  if (searches) *searches = n_searches;
+  out[3] = s.iterations_done;
+  return CB200_OK;
+}
+
+// the caller's row-major answers of n requests into the answer buffers, on the current stream
+static int store_stage_answers(GameStore &s, const float *eval, const float *probs, int n) {
+  CB_CUDA(cudaMemcpyAsync(s.d_eval, eval, (size_t)n * sizeof(float), cudaMemcpyHostToDevice, cur_stream()));
+  CB_CUDA(cudaMemcpyAsync(s.d_probs, probs, (size_t)n * CB200_NUM_MOVES * sizeof(float), cudaMemcpyHostToDevice,
+                          cur_stream()));
   return CB200_OK;
 }
 
@@ -702,96 +849,24 @@ cb200_trainer *cb200_trainer_create_shard(int total_games, int first_game, int n
     set_error(CB200_ERR_ARG, "cb200_trainer_create: invalid argument");
     return nullptr;
   }
-  int dev = 0;
-  if (cudaGetDevice(&dev) != cudaSuccess || upload_tables_once() != CB200_OK) {
-    if (last_error_ref().empty()) set_error(CB200_ERR_CUDA, "no usable CUDA device");
-    return nullptr;
-  }
   cb200_trainer *t = new cb200_trainer();
-  t->device = dev;
   t->log_folder = log_folder ? log_folder : "";
-  TreeParams &P = t->P;
-  P.num_games = num_games, P.first_game = first_game, P.total_games = total_games;
-  P.max_searches = max_searches, P.spe = searches_per_eval;
-  P.c_puct = c_puct, P.epsilon = epsilon, P.testing = testing ? 1 : 0;
-  // arena budget: kept subtree + max_searches new nodes per move with head-room; a game that
-  // still overflows fails loudly (CB200_ERR_OVERFLOW). ~28 slots/node on average.
-  long long nodes = (long long)max_searches * 5 / 2 + 96;
-  long long words = nodes * (8 + 4 * 28);
-  if (const char *env = getenv("CB200_ARENA_NODES")) {
-    words = atoll(env) * (8 + 4 * 28);
-  } else {
-    // Larger arenas make in-place re-rooting the common case (compaction only when room runs
-    // out). The node arenas of one trainer take at most an explicit budget -- 48 GiB by default,
-    // CB200_ARENA_BUDGET_MB overrides -- capped at 16 moves' worth of nodes per arena and never
-    // below the minimum above; a co-resident trainer keeps the rest of the HBM.
-    long long budget_bytes = 48ll << 30;
-    if (const char *env = getenv("CB200_ARENA_BUDGET_MB")) budget_bytes = atoll(env) << 20;
-    long long budget = budget_bytes / ((long long)num_games * 3 * 4);
-    const long long cap = (long long)max_searches * 16 * (8 + 4 * 28);
-    if (budget > cap) budget = cap;
-    if (budget > words) words = budget;
-  }
-  words = (words + 3) & ~3ll;
-  if (words < 1024) words = 1024;
-  if (words > 0x7fffff00ll) words = 0x7fffff00ll;
-  P.arena_words = (uint32_t)words;
-  t->stagger_div = total_games / max_searches;
-  if (t->stagger_div < 1) t->stagger_div = 1;
-  const size_t Gn = (size_t)num_games;
-  t->cap = Gn * searches_per_eval;
-  if (t->cap * CB200_NUM_MOVES >= (size_t)1 << 31) {  // the kernels index answers with 31 bits
-    set_error(CB200_ERR_ARG, "cb200_trainer_create: num_games * searches_per_eval too large for one trainer");
-    delete t;
-    return nullptr;
-  }
-  bool ok = dmalloc(&P.arenas, Gn * 3 * P.arena_words) == CB200_OK &&
-            dmalloc(&P.ctl, Gn * kCtlWords) == CB200_OK &&
-            dmalloc(&P.tree, Gn * 2 * kTreeCtlWords) == CB200_OK &&
-            dmalloc(&P.mt, Gn * 624) == CB200_OK &&
-            dmalloc(&P.pending, t->cap * kPendWords) == CB200_OK &&
-            dmalloc(&P.leaf_state, t->cap) == CB200_OK &&
-            dmalloc(&P.sample_state, Gn * kMaxSamples) == CB200_OK &&
-            dmalloc(&P.sample_probs, Gn * kMaxSamples * CB200_NUM_MOVES) == CB200_OK &&
-            dmalloc(&P.counters, Gn * 4) == CB200_OK &&
-            // (+ kAnswerSlack rows: a fused tourney reads its answers at the reference's own offsets,
-            // tourney.cpp:54-62, which may run a few rows past the requests of the call)
-            dmalloc(&t->d_eval, t->cap + kAnswerSlack) == CB200_OK &&
-            dmalloc(&t->d_probs, (t->cap + kAnswerSlack) * CB200_NUM_MOVES) == CB200_OK &&
-            dmalloc(&t->d_rows, t->cap * CB200_STATE_SIZE) == CB200_OK &&
-            dmalloc(&t->d_packed, t->cap) == CB200_OK && dmalloc(&t->d_offs, Gn) == CB200_OK &&
-            dmalloc(&t->d_soff, Gn) == CB200_OK && dmalloc(&t->d_summary, 4) == CB200_OK &&
-            cudaMallocHost((void **)&t->h_summary, 4 * sizeof(int32_t)) == cudaSuccess;
-  if (ok) {
-    // c_puct * sqrt(visits) exactly as trainmc.cpp:568 evaluates it (double sqrt, double product,
-    // one rounding to float); IEEE sqrt is correctly rounded on host and device alike
-    float *d_vsqrt = nullptr;
-    std::vector<float> vs(kVsqrtCap);
-    for (int i = 0; i < kVsqrtCap; ++i)
-      vs[i] = (float)((double)c_puct * sqrt((double)(float)i));
-    ok = dmalloc(&d_vsqrt, (size_t)kVsqrtCap) == CB200_OK &&
-         cudaMemcpy(d_vsqrt, vs.data(), sizeof(float) * kVsqrtCap, cudaMemcpyHostToDevice) ==
-             cudaSuccess;
-    P.vsqrt = d_vsqrt;
-  }
-  if (ok) {
-    // logged games = global indices [0, num_logged) (trainer.cpp:243-250) that fall in this shard
-    long long nl = (long long)num_logged - first_game;
-    if (nl < 0) nl = 0;
-    if (nl > num_games) nl = num_games;
-    P.n_logged = (int)nl;
-    if (P.n_logged > 0) {
-      ok = dmalloc(&P.log_buf, (size_t)P.n_logged * kLogMaxMoves * kLogWords) == CB200_OK &&
-           dmalloc(&P.log_count, (size_t)P.n_logged) == CB200_OK;
-      if (ok) ok = cudaMemset(P.log_count, 0, (size_t)P.n_logged * sizeof(int32_t)) == cudaSuccess;
-      t->log_written.assign(P.n_logged, 0);
-    }
-  }
-  if (!ok) {
-    if (last_error_ref().empty()) set_error(CB200_ERR_CUDA, "allocation failed");
+  // logged games = global indices [0, num_logged) (trainer.cpp:243-250) that fall in this shard
+  std::vector<std::string> log_paths;
+  for (int g = first_game; g < num_logged && g < first_game + num_games; ++g)
+    log_paths.push_back(t->log_folder + "/game_" + std::to_string(g) + ".txt");
+  // the sample buffers in testing mode too: cb200_trainer_write_raw_samples reads them
+  if (store_create(*t, num_games, max_searches, searches_per_eval, c_puct, epsilon, testing, true, log_paths) !=
+          CB200_OK ||
+      dmalloc(&t->d_soff, (size_t)num_games) != CB200_OK) {
     cb200_trainer_destroy(t);
     return nullptr;
   }
+  t->P.first_game = first_game, t->P.total_games = total_games;
+  t->P.n_logged = (int)log_paths.size();
+  t->stagger_div = total_games / max_searches;
+  if (t->stagger_div < 1) t->stagger_div = 1;
+  const size_t Gn = (size_t)num_games;
   // stream groups for the fused loop
   // A launch ends when its slowest game does, so large batches are split over a few independent
   // streams (a group only waits for its own stragglers); CB200_GROUPS overrides.
@@ -822,7 +897,7 @@ cb200_trainer *cb200_trainer_create_shard(int total_games, int first_game, int n
   t->sched.persistent = getenv("CB200_NO_PERSISTENT") == nullptr;
   {
     int sms = 148;
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, t->device);
     t->ps_ctas = sms;
   }
   t->ps_ld = t->ps_ctas * 16 * kPsRowsPerGame * 2;  // x2: two row regions in two-model runs
@@ -841,12 +916,7 @@ cb200_trainer *cb200_trainer_create_shard(int total_games, int first_game, int n
     cb200_trainer_destroy(t);
     return nullptr;
   }
-  P.game_begin = 0, P.game_end = num_games, P.group_row0 = 0, P.group_ctr = nullptr;
-  P.live_list = nullptr, P.live_count = nullptr;
-  P.packed = t->d_packed;
-  P.phase_prof = nullptr;
-  t->seed = seed;
-  if (init_state(t) != CB200_OK) {
+  if (cb200_trainer_reset(t, seed) != CB200_OK) {
     cb200_trainer_destroy(t);
     return nullptr;
   }
@@ -883,8 +953,18 @@ int cb200_trainer_phase_profile(cb200_trainer *t, int enable, uint64_t out[16]) 
 int cb200_trainer_reset(cb200_trainer *t, int seed) {
   int rc = guard(t);
   if (rc) return rc;
-  t->seed = seed;
-  return init_state(t);
+  // queued before the store's reset, which synchronises the stream
+  CB_CUDA(cudaMemsetAsync(t->d_gctr, 0, (size_t)t->n_groups * 8 * sizeof(int32_t), cur_stream()));
+  if ((rc = store_reset(*t, t->P.num_games, seed)) != CB200_OK) return rc;
+  t->ps_active = false, t->ps_from_lockstep = false, t->ps_n = 0, t->ps_cur = 0;
+  if (t->stream_on) {
+    CB_CUDA(cudaStreamSynchronize(t->st_stream));
+    CB_CUDA(cudaMemset(t->d_emitted, 0, (size_t)t->P.num_games * sizeof(int32_t)));
+    CB_CUDA(cudaMemset(t->d_st_ctr, 0, 2 * sizeof(int32_t)));
+    t->st_pending = false, t->st_copied = 0, t->st_round = 0;
+    t->h_st_ctr[0] = t->h_st_ctr[1] = 0;
+  }
+  return CB200_OK;
 }
 
 int cb200_trainer_set_profiling(cb200_trainer *t, int enable) {
@@ -927,15 +1007,11 @@ void cb200_trainer_destroy(cb200_trainer *t) {
   if (!t) return;
   cudaSetDevice(t->device);
   for (cudaEvent_t e : t->ev_pool) cudaEventDestroy(e);
-  TreeParams &P = t->P;
-  cudaFree(P.log_buf), cudaFree(P.log_count);
   cudaFree(t->d_ps_list), cudaFree(t->d_ps_out), cudaFree(t->d_ps_eval[0]), cudaFree(t->d_ps_eval[1]);
   cudaFree(t->d_ps_probs[0]), cudaFree(t->d_ps_probs[1]);
   cudaFree(t->d_ps_packed), cudaFreeHost(t->h_ps_out);
-  cudaFree((void *)P.vsqrt), cudaFree(P.arenas), cudaFree(P.ctl), cudaFree(P.tree), cudaFree(P.mt), cudaFree(P.pending);
-  cudaFree(P.leaf_state), cudaFree(P.sample_state), cudaFree(P.sample_probs), cudaFree(P.counters);
-  cudaFree(t->d_eval), cudaFree(t->d_probs), cudaFree(t->d_rows), cudaFree(t->d_packed);
-  cudaFree(t->d_offs), cudaFree(t->d_soff), cudaFree(t->d_summary), cudaFree(P.phase_prof);
+  cudaFree(t->d_soff), cudaFree(t->P.phase_prof);
+  store_free(*t);
   cudaFree(t->d_samp);
   cudaFree(t->d_raw);
   cudaFree(t->d_gath), cudaFree(t->d_gcounts);
@@ -946,14 +1022,10 @@ void cb200_trainer_destroy(cb200_trainer *t) {
   if (t->h_st_ctr) cudaFreeHost(t->h_st_ctr);
   if (t->st_ev) cudaEventDestroy(t->st_ev);
   if (t->st_stream) cudaStreamDestroy(t->st_stream);
-  if (t->h_summary) cudaFreeHost(t->h_summary);
   if (t->h_gctr) cudaFreeHost(t->h_gctr);
   cudaFree(t->d_gctr), cudaFree(t->d_live_list), cudaFree(t->d_live_count);
   for (cudaStream_t st : t->g_stream) cudaStreamDestroy(st);
-  for (int m = 0; m < 2; ++m) {
-    cudaFree(t->net32[m].w);
-    net_tc_free(t->nettc[m]);
-  }
+  for (Net &n : t->net) net_free(n);
   delete t;
 }
 
@@ -994,29 +1066,19 @@ int cb200_trainer_do_iteration(cb200_trainer *t, const float *eval, const float 
   const int n = t->h_summary[0];
   if (n > 0) {
     if (!eval || !probs) return set_error(CB200_ERR_ARG, "requests pending but eval/probs null");
-    CB_CUDA(cudaMemcpyAsync(t->d_eval, eval, (size_t)n * sizeof(float), cudaMemcpyHostToDevice,
-                            cur_stream()));
-    CB_CUDA(cudaMemcpyAsync(t->d_probs, probs, (size_t)n * CB200_NUM_MOVES * sizeof(float),
-                            cudaMemcpyHostToDevice, cur_stream()));
+    if ((rc = store_stage_answers(*t, eval, probs, n)) != CB200_OK) return rc;
   }
   if ((rc = iterate(t, t->d_eval, t->d_probs, to_play)) != CB200_OK) return rc;
   if ((rc = scan(t, to_play)) != CB200_OK) return rc;
   if ((rc = fetch_summary(t)) != CB200_OK) return rc;
-  if ((rc = drain_logs(t)) != CB200_OK) return rc;
+  if ((rc = store_drain_logs(*t)) != CB200_OK) return rc;
   return t->h_summary[1] == 0 ? 1 : 0;
-}
-
-static int fetch_ctl(cb200_trainer *t) {
-  t->h_ctl.resize((size_t)t->P.num_games * kCtlWords);
-  CB_CUDA(cudaStreamSynchronize(cur_stream()));
-  CB_CUDA(cudaMemcpy(t->h_ctl.data(), t->P.ctl, t->h_ctl.size() * 4, cudaMemcpyDeviceToHost));
-  return CB200_OK;
 }
 
 int cb200_trainer_num_samples(cb200_trainer *t) {
   int rc = guard(t);
   if (rc) return rc;
-  if ((rc = fetch_ctl(t)) != CB200_OK) return rc;
+  if ((rc = store_fetch_ctl(*t)) != CB200_OK) return rc;
   long long n = 0;
   for (int g = 0; g < t->P.num_games; ++g) n += t->h_ctl[(size_t)g * kCtlWords + CW_N_SAMPLES];
   return (int)n;
@@ -1027,7 +1089,7 @@ int cb200_trainer_write_samples(cb200_trainer *t, float *game_states, float *eva
   int rc = guard(t);
   if (rc) return rc;
   if (!game_states || !eval_samples || !prob_samples) return set_error(CB200_ERR_ARG, "null buffer");
-  if ((rc = fetch_ctl(t)) != CB200_OK) return rc;
+  if ((rc = store_fetch_ctl(*t)) != CB200_OK) return rc;
   const int Gn = t->P.num_games;
   std::vector<int32_t> soff(Gn);
   long long ns = 0;
@@ -1074,7 +1136,7 @@ static float game_score(int result) {  // SelfPlayer::score selfplayer.cpp:57-64
 }
 
 float cb200_trainer_score(cb200_trainer *t) {  // trainer.cpp:59-68
-  if (guard(t) || fetch_ctl(t)) return NAN;
+  if (guard(t) || store_fetch_ctl(*t)) return NAN;
   const int Gn = t->P.num_games;
   float score = 0;
   for (int g = 0; g < Gn; ++g)
@@ -1086,7 +1148,7 @@ float cb200_trainer_score(cb200_trainer *t) {  // trainer.cpp:59-68
 }
 
 float cb200_trainer_avg_mate_length(cb200_trainer *t) {  // trainer.cpp:70-77
-  if (guard(t) || fetch_ctl(t)) return NAN;
+  if (guard(t) || store_fetch_ctl(*t)) return NAN;
   const int Gn = t->P.num_games;
   int total = 0;
   for (int g = 0; g < Gn; ++g) {
@@ -1100,7 +1162,7 @@ int cb200_trainer_write_scores(cb200_trainer *t, const char *file) {  // trainer
   int rc = guard(t);
   if (rc) return rc;
   if (!file) return set_error(CB200_ERR_ARG, "null file");
-  if ((rc = fetch_ctl(t)) != CB200_OK) return rc;
+  if ((rc = store_fetch_ctl(*t)) != CB200_OK) return rc;
   const int Gn = t->P.num_games;
   std::vector<float> scores(Gn);
   for (int g = 0; g < Gn; ++g) {
@@ -1127,24 +1189,14 @@ int cb200_trainer_write_scores(cb200_trainer *t, const char *file) {  // trainer
 }
 
 int cb200_trainer_counters(cb200_trainer *t, int64_t out[4]) {
-  int rc = guard(t);
-  if (rc) return rc;
-  std::vector<long long> h((size_t)t->P.num_games * 4);
-  CB_CUDA(cudaStreamSynchronize(cur_stream()));
-  CB_CUDA(cudaMemcpy(h.data(), t->P.counters, h.size() * sizeof(long long), cudaMemcpyDeviceToHost));
-  out[0] = out[1] = out[2] = 0;
-  long long searches = 0;
-  for (int g = 0; g < t->P.num_games; ++g)
-    out[0] += h[4 * g], out[1] += h[4 * g + 1], out[2] += h[4 * g + 2], searches += h[4 * g + 3];
-  t->searches_now = searches;
-  out[3] = t->iterations_done;
-  return CB200_OK;
+  const int rc = guard(t);
+  return rc != CB200_OK ? rc : store_counters(*t, out, &t->searches_now);
 }
 
 int cb200_trainer_game_results(cb200_trainer *t, int32_t *results) {
   int rc = guard(t);
   if (rc) return rc;
-  if ((rc = fetch_ctl(t)) != CB200_OK) return rc;
+  if ((rc = store_fetch_ctl(*t)) != CB200_OK) return rc;
   for (int g = 0; g < t->P.num_games; ++g) results[g] = t->h_ctl[(size_t)g * kCtlWords + CW_RESULT];
   return CB200_OK;
 }
@@ -1153,7 +1205,7 @@ int cb200_trainer_write_raw_samples(cb200_trainer *t, uint64_t *states, float *p
                                     int32_t *game_of) {
   int rc = guard(t);
   if (rc) return rc;
-  if ((rc = fetch_ctl(t)) != CB200_OK) return rc;
+  if ((rc = store_fetch_ctl(*t)) != CB200_OK) return rc;
   const int Gn = t->P.num_games;
   std::vector<ulonglong2> hs;
   std::vector<float> hp;
@@ -1186,7 +1238,7 @@ int cb200_trainer_raw_samples_device(cb200_trainer *t, void **rows_device, int *
   int rc = guard(t);
   if (rc) return rc;
   if (!rows_device || !n_rows) return set_error(CB200_ERR_ARG, "null output");
-  if ((rc = fetch_ctl(t)) != CB200_OK) return rc;
+  if ((rc = store_fetch_ctl(*t)) != CB200_OK) return rc;
   const int Gn = t->P.num_games;
   std::vector<int32_t> soff(Gn);
   long long ns = 0;
@@ -1374,15 +1426,9 @@ int cb200_trainer_set_weights(cb200_trainer *t, int model, const float *weights,
                               int precision) {
   int rc = guard(t);
   if (rc) return rc;
-  if (model < 0 || model > 1 || !weights || n_floats != kNetWeightFloats ||
-      (precision < 0 || precision > 3))
-    return set_error(CB200_ERR_ARG, "cb200_trainer_set_weights: bad arguments (127997 floats, precision 0|1|2|3)");
-  // tensor-core operand modes: precision 1 -> bf16, 2 -> fp16, 3 -> bf16x3 (hi + lo operands)
-  rc = precision == 0 ? net_f32_upload(t->net32[model], weights)
-                      : net_tc_upload(t->nettc[model], weights, precision == 1 ? 0 : (precision == 2 ? 1 : 2));
-  // precisions 1-3 share the tensor-core kernel and the move-major output
-  if (rc == CB200_OK) t->precision[model] = precision == 0 ? 0 : 1;
-  return rc;
+  if (model < 0 || model > 1) return set_error(CB200_ERR_ARG, "cb200_trainer_set_weights: model must be 0 or 1");
+  if ((rc = check_weights(weights, n_floats, precision, "cb200_trainer_set_weights")) != CB200_OK) return rc;
+  return net_upload(t->net[model], weights, precision);
 }
 
 int cb200_trainer_evaluate(cb200_trainer *t, int model, int n, const float *game_states,
@@ -1405,9 +1451,13 @@ int cb200_trainer_evaluate(cb200_trainer *t, int model, int n, const float *game
   }
   cudaStream_t s = cur_stream();
   CB_CUDA(cudaMemcpyAsync(t->d_packed, hs.data(), (size_t)n * sizeof(ulonglong2), cudaMemcpyHostToDevice, s));
-  if ((rc = run_net(t, model, t->d_packed, nullptr, n, n)) != CB200_OK) return rc;
+  {
+    ProfScope ps(t, 2);
+    rc = net_launch(t->net[model], t->d_packed, nullptr, n, n, t->d_eval, t->d_probs, (int)t->cap);
+  }
+  if (rc != CB200_OK) return rc;
   CB_CUDA(cudaMemcpyAsync(eval, t->d_eval, (size_t)n * sizeof(float), cudaMemcpyDeviceToHost, s));
-  if (t->precision[model] == 1) {  // move-major [96][cap] on the device -> row-major for the caller
+  if (t->net[model].tensor_core()) {  // move-major [96][cap] on the device -> row-major for the caller
     // transposed on the device into the (idle) request-row buffer: cap * 70 floats >= n * 96 is not
     // guaranteed, so rows go through it in slices
     const size_t slice = t->cap * CB200_STATE_SIZE / CB200_NUM_MOVES;
@@ -1436,9 +1486,9 @@ static int ps_games_per_sm(int mode) { return mode == 2 ? 8 : 16; }
 // this many live games or fewer; 0 = never. It needs the tensor-core network (in two-model runs
 // both networks, with the same operand mode) and at most kPsRowsPerGame requests per game.
 static int ps_takeover(const cb200_trainer *t) {
-  const NetTC &n0 = t->nettc[0];
-  if (!t->sched.persistent || t->precision[0] != 1 || t->P.spe > kPsRowsPerGame) return 0;
-  if (t->P.testing && (t->precision[1] != 1 || t->nettc[1].mode != n0.mode)) return 0;
+  const NetTC &n0 = t->net[0].tc;
+  if (!t->sched.persistent || !t->net[0].tensor_core() || t->P.spe > kPsRowsPerGame) return 0;
+  if (t->P.testing && (!t->net[1].tensor_core() || t->net[1].tc.mode != n0.mode)) return 0;
   const long long fit = (long long)t->ps_ctas * ps_games_per_sm(n0.mode);
   return (int)std::max(0ll, std::min(t->sched.ps_capacity, fit));
 }
@@ -1476,9 +1526,9 @@ static int ps_launch(cb200_trainer *t, const TreeParams &P, int rounds, int exit
   // one CTA per SM, games dealt round-robin (every CTA gets ceil or floor of ps_n / grid)
   const int grid = t->ps_n < t->ps_ctas ? t->ps_n : t->ps_ctas;
   // two-model (gating match) runs: model 1 answers the other side's requests
-  const uint8_t *w1 = P.testing ? (const uint8_t *)t->nettc[1].w : nullptr;
+  const uint8_t *w1 = P.testing ? (const uint8_t *)t->net[1].tc.w : nullptr;
   k_selfplay_persistent<kMode, kGames><<<grid, kGames * 32, ps_smem_bytes<kMode, kGames>(), t->g_stream[0]>>>(
-      P, (const uint8_t *)t->nettc[0].w, w1, t->d_ps_list, t->ps_n, ev0, pr0, pcs0, t->d_ps_eval[nxt],
+      P, (const uint8_t *)t->net[0].tc.w, w1, t->d_ps_list, t->ps_n, ev0, pr0, pcs0, t->d_ps_eval[nxt],
       t->d_ps_probs[nxt], t->ps_ld, t->d_ps_packed, rounds, exit_done, t->iterations_done,
       t->d_ps_out);
   CB_LAUNCHED();
@@ -1548,7 +1598,7 @@ static int run_persistent(cb200_trainer *t, int max_rounds, int *rounds_done, bo
     }
     const int rounds = max_rounds - *rounds_done;
     const int exit_done = t->ps_n > kRedealMinGames ? t->ps_n * kRedealPct / 100 : INT_MAX;
-    const int mode = t->nettc[0].mode;  // 0 bf16, 1 fp16, 2 bf16x3
+    const int mode = t->net[0].tc.mode;  // 0 bf16, 1 fp16, 2 bf16x3
     const bool wide = t->ps_n > t->ps_ctas * 8;
     if (t->ps_n > t->ps_ctas * ps_games_per_sm(mode))
       return set_error(CB200_ERR_STATE, "persistent kernel: more live games than fit on the device");
@@ -1591,7 +1641,7 @@ static int run_persistent(cb200_trainer *t, int max_rounds, int *rounds_done, bo
 // its own group while the other groups keep the SMs and the tensor cores busy.
 static int run_selfplay_groups(cb200_trainer *t, int max_iterations) {
   const int model = 0;
-  const bool tc = t->precision[model] == 1;
+  const bool tc = t->net[model].tensor_core();
   const long prs = tc ? 1 : CB200_NUM_MOVES, pcs = tc ? (long)t->cap : 1;
   const int ng = t->n_groups;
   std::vector<char> active(ng, 1);
@@ -1626,7 +1676,7 @@ static int run_selfplay_groups(cb200_trainer *t, int max_iterations) {
         const int row0 = gb * t->P.spe, rows = (ge - gb) * t->P.spe;
         int32_t *ctr = t->d_gctr + g * 8;
         ProfScope ps(t, 2, t->g_stream[g]);
-        int rc = launch_mlp_tc(t->nettc[model], t->d_packed + row0, ctr + (it & 1), 0, rows,
+        int rc = launch_mlp_tc(t->net[model].tc, t->d_packed + row0, ctr + (it & 1), 0, rows,
                                t->d_eval + row0, t->d_probs + row0, (int)t->cap,
                                ctr + ((it + 1) & 1), t->g_stream[g], true);
         if (rc != CB200_OK) return rc;
@@ -1680,10 +1730,10 @@ static int run_selfplay_groups(cb200_trainer *t, int max_iterations) {
         {
           ProfScope ps(t, 2, st);
           if (tc)
-            rc = launch_mlp_tc(t->nettc[model], t->d_packed + row0, ctr + (it & 1), 0, rows, t->d_eval + row0,
+            rc = launch_mlp_tc(t->net[model].tc, t->d_packed + row0, ctr + (it & 1), 0, rows, t->d_eval + row0,
                                t->d_probs + row0, (int)t->cap, ctr + ((it + 1) & 1), st, true, overlap);
           else
-            rc = launch_mlp_f32(t->net32[model], t->d_packed + row0, ctr + (it & 1), 0, rows, t->d_eval + row0,
+            rc = launch_mlp_f32(t->net[model].f32, t->d_packed + row0, ctr + (it & 1), 0, rows, t->d_eval + row0,
                                 t->d_probs + (size_t)row0 * CB200_NUM_MOVES, ctr + ((it + 1) & 1), st, true);
         }
         if (rc != CB200_OK) return rc;
@@ -1745,7 +1795,7 @@ int cb200_trainer_run_selfplay(cb200_trainer *t, int max_iterations, int stagger
   int rc = guard(t);
   if (rc) return rc;
   const bool testing = t->P.testing != 0;
-  if (t->precision[0] < 0 || (testing && t->precision[1] < 0))
+  if (t->net[0].precision < 0 || (testing && t->net[1].precision < 0))
     return set_error(CB200_ERR_STATE, "cb200_trainer_run_selfplay: set weights first");
   const int saved_div = t->stagger_div;
   if (!stagger) t->stagger_div = 0;
@@ -1762,7 +1812,7 @@ int cb200_trainer_run_selfplay(cb200_trainer *t, int max_iterations, int stagger
     }
     t->stagger_div = saved_div;
     if (rc >= 0) {
-      const int lr = drain_logs(t);
+      const int lr = store_drain_logs(*t);
       if (lr != CB200_OK) return lr;
     }
     return rc;
@@ -1780,7 +1830,7 @@ int cb200_trainer_run_selfplay(cb200_trainer *t, int max_iterations, int stagger
     bool all_done = false;
     rc = run_persistent(t, max_iterations > 0 ? max_iterations : (1 << 30), &rounds, &all_done);
     t->stagger_div = saved_div;
-    if (rc == CB200_OK) rc = drain_logs(t);
+    if (rc == CB200_OK) rc = store_drain_logs(*t);
     return rc != CB200_OK ? rc : (all_done ? 1 : 0);
   }
   // otherwise: single lock-step group, requests packed per side
@@ -1794,8 +1844,11 @@ int cb200_trainer_run_selfplay(cb200_trainer *t, int max_iterations, int stagger
       for (int tp = 0; tp < 2 && rc == CB200_OK; ++tp) {  // model 0 = "new" serves to_play 0
         rc = scan(t, tp);
         if (rc == CB200_OK) rc = pack(t, tp, nullptr, t->d_packed);
-        if (rc == CB200_OK) rc = run_net(t, tp == 0 ? 0 : 1, t->d_packed, t->d_summary, 0, n_max);
-        if (rc == CB200_OK) rc = iterate(t, t->d_eval, t->d_probs, tp, t->precision[tp == 0 ? 0 : 1] == 1);
+        if (rc == CB200_OK) {
+          ProfScope ps(t, 2);
+          rc = net_launch(t->net[tp], t->d_packed, t->d_summary, 0, n_max, t->d_eval, t->d_probs, n_max);
+        }
+        if (rc == CB200_OK) rc = iterate(t, t->d_eval, t->d_probs, tp, t->net[tp].tensor_core());
       }
       ++t->iterations_done;
     }
@@ -1809,7 +1862,7 @@ int cb200_trainer_run_selfplay(cb200_trainer *t, int max_iterations, int stagger
     }
   }
   t->stagger_div = saved_div;
-  if (rc == CB200_OK) rc = drain_logs(t);
+  if (rc == CB200_OK) rc = store_drain_logs(*t);
   return rc != CB200_OK ? rc : result;
 }
 
@@ -1838,55 +1891,27 @@ int cb200_trainer_dump_tree(cb200_trainer *t, int game, int player, int64_t out[
 
 
 // ==============================================================================================
-// A device-resident network of the fused tourney (one per model id) and of the analysis. The
-// weights stay on the host until the first run that needs them uploads them (the device state may
-// not exist when they are set). Same weight layout and precision codes as cb200_trainer_set_weights.
+// The network of a fused-tourney model id or of an analysis. The weights stay on the host until the
+// first run that needs them uploads them (the device state may not exist when they are set).
 struct ResidentNet {
   std::vector<float> host;
   int precision = -1;  // -1 = no weights set
-  bool uploaded = false;
-  NetF32 f32;
-  NetTC tc;
+  Net net;             // net.precision < 0 until uploaded
 };
 
 static void resident_net_set(ResidentNet &n, const float *weights, int precision) {
   n.host.assign(weights, weights + kNetWeightFloats);
   n.precision = precision;
-  n.uploaded = false;
+  n.net.precision = -1;
 }
 
 static int resident_net_upload(ResidentNet &n) {
-  if (n.uploaded) return CB200_OK;
-  // tensor-core operand modes: precision 1 -> bf16, 2 -> fp16, 3 -> bf16x3 (hi + lo operands)
-  const int rc = n.precision == 0 ? net_f32_upload(n.f32, n.host.data())
-                                  : net_tc_upload(n.tc, n.host.data(), n.precision == 1 ? 0 : (n.precision == 2 ? 1 : 2));
-  if (rc == CB200_OK) n.uploaded = true;
-  return rc;
-}
-
-static void resident_net_free(ResidentNet &n) {
-  cudaFree(n.f32.w);
-  n.f32.w = nullptr;
-  net_tc_free(n.tc);
-}
-
-// Evaluate the leaf cstates packed[0 .. t->d_summary[0]) into t's answer buffers on the current
-// stream. The answer of row k for move m is then at d_probs[k * prs + m * pcs]: row-major from the
-// fp32 kernel, move-major (leading dimension cap + kAnswerSlack) from the tensor-core kernel.
-static int resident_net_launch(const ResidentNet &n, cb200_trainer *t, const ulonglong2 *packed, long &prs,
-                               long &pcs) {
-  if (n.precision == 0) {
-    prs = CB200_NUM_MOVES, pcs = 1;
-    return launch_mlp_f32(n.f32, packed, t->d_summary, 0, (int)t->cap, t->d_eval, t->d_probs);
-  }
-  prs = 1, pcs = (long)(t->cap + kAnswerSlack);
-  return launch_mlp_tc(n.tc, packed, t->d_summary, 0, (int)t->cap, t->d_eval, t->d_probs,
-                       (int)(t->cap + kAnswerSlack));
+  return n.net.precision >= 0 ? CB200_OK : net_upload(n.net, n.host.data(), n.precision);
 }
 
 // ==============================================================================================
 // Tourney (corintho_ai/cpp/include/tourney.h:12-46) over Match (match.h:33-101); device side in
-// match.cuh. The matches share the per-game storage of a trainer created when the first call
+// match.cuh. One "game" of the tourney's store per match; the store is created when the first call
 // needs the device (all players and matches must have been added by then).
 struct cb200_tourney {
   int num_threads = 1;
@@ -1894,9 +1919,8 @@ struct cb200_tourney {
   std::map<int, MatchSide> players;
   std::vector<std::pair<int, int>> matches;
   std::vector<char> logging;  // per match (Tourney::addMatch, tourney.cpp:80-96)
-  std::vector<std::unique_ptr<std::ofstream>> log_files;  // per logged match; null = not opened
-  std::vector<int> log_written;
-  cb200_trainer *t = nullptr;
+  bool ready = false;         // the store and the match buffers exist
+  GameStore s;
   MatchSide *d_sides = nullptr;
   int32_t *d_pack_offs = nullptr, *d_iter_offs = nullptr;
   // fused mode (cb200_tourney_set_weights / cb200_tourney_run): one device-resident network per
@@ -1905,43 +1929,11 @@ struct cb200_tourney {
   std::map<int, ResidentNet> nets;
 };
 
-static int tourney_ready_build(cb200_tourney *T, cb200_trainer *t, const std::vector<MatchSide> &sides,
-                               int n_log) {
+static int tourney_ready_build(cb200_tourney *T) {
   const int n = (int)T->matches.size();
-  int rc = fetch_ctl(t);
-  if (rc != CB200_OK) return rc;
-  const CState st = start_state();
-  for (int g = 0; g < n; ++g) {
-    int32_t *c = t->h_ctl.data() + (size_t)g * kCtlWords;
-    c[MW_ROOT0] = (int32_t)(uint32_t)st.w0, c[MW_ROOT1] = (int32_t)(uint32_t)(st.w0 >> 32);
-    c[MW_ROOT2] = (int32_t)(uint32_t)st.w1, c[MW_ROOT3] = (int32_t)(uint32_t)(st.w1 >> 32);
-    c[MW_DEPTH] = 0;
-  }
-  CB_CUDA(cudaMemcpy(t->P.ctl, t->h_ctl.data(), t->h_ctl.size() * 4, cudaMemcpyHostToDevice));
-  if ((rc = dmalloc(&T->d_sides, sides.size())) != CB200_OK ||
-      (rc = dmalloc(&T->d_pack_offs, (size_t)n)) != CB200_OK ||
-      (rc = dmalloc(&T->d_iter_offs, (size_t)n)) != CB200_OK)
-    return rc;
-  CB_CUDA(cudaMemcpy(T->d_sides, sides.data(), sides.size() * sizeof(MatchSide), cudaMemcpyHostToDevice));
-  if (n_log > 0) {  // the trainer owns (and frees) the log areas
-    if ((rc = dmalloc(&t->P.log_buf, (size_t)n_log * kLogMaxMoves * kLogWords)) != CB200_OK ||
-        (rc = dmalloc(&t->P.log_count, (size_t)n_log)) != CB200_OK)
-      return rc;
-    CB_CUDA(cudaMemset(t->P.log_count, 0, (size_t)n_log * sizeof(int32_t)));
-  }
-  return CB200_OK;
-}
-
-static int tourney_ready(cb200_tourney *T) {
-  if (!T) return set_error(CB200_ERR_ARG, "null tourney");
-  if (T->t) return CB200_OK;
-  last_error_ref().clear();
-  const int n = (int)T->matches.size();
-  if (n == 0) return set_error(CB200_ERR_STATE, "tourney has no matches");
   int max_ms = 1, max_spe = 1;
   std::vector<MatchSide> sides(2 * (size_t)n);
-  int n_log = 0;
-  T->log_files.clear();
+  std::vector<std::string> log_paths;
   for (int i = 0; i < n; ++i) {
     const int pid[2] = {T->matches[i].first, T->matches[i].second};
     for (int s = 0; s < 2; ++s) {
@@ -1951,66 +1943,62 @@ static int tourney_ready(cb200_tourney *T) {
       if (sides[2 * i + s].spe > max_spe) max_spe = sides[2 * i + s].spe;
     }
     if (T->logging[i]) {  // log_folder/match_<p1>_<p2>_<index>.txt (tourney.cpp:88-93)
-      sides[2 * i].log_slot = n_log++;
-      auto f = std::make_unique<std::ofstream>(T->log_folder + "/match_" + std::to_string(pid[0]) + "_" +
-                                                   std::to_string(pid[1]) + "_" + std::to_string(i) + ".txt",
-                                               std::ofstream::out);
-      if (!f->is_open()) f.reset();
-      T->log_files.push_back(std::move(f));
+      sides[2 * i].log_slot = (int)log_paths.size();
+      log_paths.push_back(T->log_folder + "/match_" + std::to_string(pid[0]) + "_" + std::to_string(pid[1]) + "_" +
+                          std::to_string(i) + ".txt");
     }
   }
-  T->log_written.assign(n_log, 0);
   if (max_spe > max_ms) max_ms = max_spe;
-  // match seeds = successive draws of a default-seeded std::mt19937 (tourney.h:42, tourney.cpp:86)
-  cb200_trainer *t = cb200_trainer_create_shard(n, 0, n, T->log_folder.c_str(), 5489, max_ms, max_spe,
-                                                1.0f, 0.25f, 0, 1);
-  if (!t) return CB200_ERR_CUDA;
-  // the tourney becomes usable (T->t set) only when every buffer exists; a failure on the way
-  // releases the partial allocations so that a later call starts over instead of launching
-  // kernels with null side / offset pointers
-  const int rc = tourney_ready_build(T, t, sides, n_log);
-  if (rc != CB200_OK) {
-    const std::string msg = last_error_ref();
-    cudaFree(T->d_sides), cudaFree(T->d_pack_offs), cudaFree(T->d_iter_offs);
-    T->d_sides = nullptr, T->d_pack_offs = nullptr, T->d_iter_offs = nullptr;
-    cb200_trainer_destroy(t);
-    last_error_ref() = msg;
-    return rc;
+  // c_puct and epsilon are each side's own (MatchSide); the matches choose their moves in testing
+  // mode and write no samples. Match seeds = successive draws of a default-seeded std::mt19937
+  // (tourney.h:42, tourney.cpp:86).
+  GameStore &store = T->s;
+  int rc = store_create(store, n, max_ms, max_spe, 0.0f, 0.0f, 1, false, log_paths);
+  if (rc == CB200_OK) rc = store_reset(store, n, 5489);
+  if (rc == CB200_OK) rc = store_fetch_ctl(store);
+  if (rc != CB200_OK) return rc;
+  const CState start = start_state();
+  for (int g = 0; g < n; ++g) {
+    int32_t *c = store.h_ctl.data() + (size_t)g * kCtlWords;
+    c[MW_ROOT0] = (int32_t)(uint32_t)start.w0, c[MW_ROOT1] = (int32_t)(uint32_t)(start.w0 >> 32);
+    c[MW_ROOT2] = (int32_t)(uint32_t)start.w1, c[MW_ROOT3] = (int32_t)(uint32_t)(start.w1 >> 32);
+    c[MW_DEPTH] = 0;
   }
-  T->t = t;
+  CB_CUDA(cudaMemcpy(store.P.ctl, store.h_ctl.data(), store.h_ctl.size() * 4, cudaMemcpyHostToDevice));
+  if ((rc = dmalloc(&T->d_sides, sides.size())) != CB200_OK ||
+      (rc = dmalloc(&T->d_pack_offs, (size_t)n)) != CB200_OK ||
+      (rc = dmalloc(&T->d_iter_offs, (size_t)n)) != CB200_OK)
+    return rc;
+  CB_CUDA(cudaMemcpy(T->d_sides, sides.data(), sides.size() * sizeof(MatchSide), cudaMemcpyHostToDevice));
   return CB200_OK;
 }
 
-// append the records the matches wrote since the last call to their log files
-static int tourney_drain_logs(cb200_tourney *T) {
-  const int n_log = (int)T->log_written.size();
-  if (n_log == 0) return CB200_OK;
-  cb200_trainer *t = T->t;
-  t->h_log_count.resize(n_log);
-  CB_CUDA(cudaMemcpy(t->h_log_count.data(), t->P.log_count, (size_t)n_log * sizeof(int32_t), cudaMemcpyDeviceToHost));
-  for (int g = 0; g < n_log; ++g) {
-    const int have = t->h_log_count[g], done = T->log_written[g];
-    if (have <= done) continue;
-    T->log_written[g] = have;
-    if (!T->log_files[g]) continue;
-    t->h_log_rec.resize((size_t)(have - done) * kLogWords);
-    CB_CUDA(cudaMemcpy(t->h_log_rec.data(), t->P.log_buf + ((size_t)g * kLogMaxMoves + done) * kLogWords,
-                       t->h_log_rec.size() * sizeof(uint32_t), cudaMemcpyDeviceToHost));
-    for (int k = 0; k < have - done; ++k)
-      format_log_record(*T->log_files[g], t->h_log_rec.data() + (size_t)k * kLogWords);
-    T->log_files[g]->flush();
+static int tourney_ready(cb200_tourney *T) {
+  if (!T) return set_error(CB200_ERR_ARG, "null tourney");
+  if (T->ready) return CB200_OK;
+  last_error_ref().clear();
+  if (T->matches.empty()) return set_error(CB200_ERR_STATE, "tourney has no matches");
+  // the tourney becomes usable only when every buffer exists; a failure on the way releases the
+  // partial allocations so that a later call starts over instead of launching kernels with null
+  // side / offset pointers
+  const int rc = tourney_ready_build(T);
+  if (rc != CB200_OK) {
+    cudaFree(T->d_sides), cudaFree(T->d_pack_offs), cudaFree(T->d_iter_offs);
+    T->d_sides = nullptr, T->d_pack_offs = nullptr, T->d_iter_offs = nullptr;
+    store_free(T->s);
+    return rc;
   }
+  T->ready = true;
   return CB200_OK;
 }
 
 // offsets + summary for one model id; h_summary = {requests, live matches, error, rows read}
 static int tourney_scan(cb200_tourney *T, int id) {
-  cb200_trainer *t = T->t;
-  k_match_scan<<<1, 1024, 0, cur_stream()>>>(t->P, T->d_sides, id, T->d_pack_offs, T->d_iter_offs,
-                                         t->d_summary);
+  GameStore &s = T->s;
+  k_match_scan<<<1, 1024, 0, cur_stream()>>>(s.P, T->d_sides, id, T->d_pack_offs, T->d_iter_offs, s.d_summary);
   CB_LAUNCHED();
   CB_CUDA(cudaGetLastError());
-  return fetch_summary(t);
+  return store_fetch_summary(s);
 }
 
 cb200_tourney *cb200_tourney_create(int num_threads, const char *log_folder) {
@@ -2026,16 +2014,17 @@ cb200_tourney *cb200_tourney_create(int num_threads, const char *log_folder) {
 
 void cb200_tourney_destroy(cb200_tourney *T) {
   if (!T) return;
+  if (T->ready) cudaSetDevice(T->s.device);
   cudaFree(T->d_sides), cudaFree(T->d_pack_offs), cudaFree(T->d_iter_offs);
-  for (auto &kv : T->nets) resident_net_free(kv.second);
-  if (T->t) cb200_trainer_destroy(T->t);
+  for (auto &kv : T->nets) net_free(kv.second.net);
+  if (T->ready) store_free(T->s);
   delete T;
 }
 
 int cb200_tourney_add_player(cb200_tourney *T, int player_id, int model_id, int max_searches,
                              int searches_per_eval, float c_puct, float epsilon, int random) {
   if (!T) return set_error(CB200_ERR_ARG, "null tourney");
-  if (T->t) return set_error(CB200_ERR_STATE, "players must be added before the first iteration");
+  if (T->ready) return set_error(CB200_ERR_STATE, "players must be added before the first iteration");
   if (!random && (max_searches <= 0 || searches_per_eval <= 0 || searches_per_eval > 64 ||
                   !(c_puct > 0.0f) || !(epsilon >= 0.0f) || !(epsilon <= 1.0f)))
     return set_error(CB200_ERR_ARG, "cb200_tourney_add_player: invalid search parameters");
@@ -2051,7 +2040,7 @@ int cb200_tourney_add_player(cb200_tourney *T, int player_id, int model_id, int 
 
 int cb200_tourney_add_match(cb200_tourney *T, int player1, int player2, int logging) {
   if (!T) return set_error(CB200_ERR_ARG, "null tourney");
-  if (T->t) return set_error(CB200_ERR_STATE, "matches must be added before the first iteration");
+  if (T->ready) return set_error(CB200_ERR_STATE, "matches must be added before the first iteration");
   if (!T->players.count(player1) || !T->players.count(player2))
     return set_error(CB200_ERR_ARG, "cb200_tourney_add_match: unknown player id");
   T->matches.emplace_back(player1, player2);
@@ -2063,14 +2052,14 @@ int cb200_tourney_all_done(cb200_tourney *T) {
   int rc = tourney_ready(T);
   if (rc) return rc;
   if ((rc = tourney_scan(T, 0x7fffffff)) != CB200_OK) return rc;
-  return T->t->h_summary[1] == 0 ? 1 : 0;
+  return T->s.h_summary[1] == 0 ? 1 : 0;
 }
 
 int cb200_tourney_num_requests(cb200_tourney *T, int id) {
   int rc = tourney_ready(T);
   if (rc) return rc;
   if ((rc = tourney_scan(T, id)) != CB200_OK) return rc;
-  return T->t->h_summary[0];
+  return T->s.h_summary[0];
 }
 
 int cb200_tourney_write_requests(cb200_tourney *T, float *game_states, int id) {
@@ -2078,14 +2067,14 @@ int cb200_tourney_write_requests(cb200_tourney *T, float *game_states, int id) {
   if (rc) return rc;
   if (!game_states) return set_error(CB200_ERR_ARG, "null game_states");
   if ((rc = tourney_scan(T, id)) != CB200_OK) return rc;
-  cb200_trainer *t = T->t;
-  const int n = t->h_summary[0];
+  GameStore &s = T->s;
+  const int n = s.h_summary[0];
   if (n <= 0) return CB200_OK;
-  k_match_pack<<<(t->P.num_games + 7) / 8, 256, 0, cur_stream()>>>(t->P, T->d_sides, id,
-                                                                 T->d_pack_offs, t->d_rows, nullptr);
+  k_match_pack<<<(s.P.num_games + 7) / 8, 256, 0, cur_stream()>>>(s.P, T->d_sides, id, T->d_pack_offs, s.d_rows,
+                                                                 nullptr);
   CB_LAUNCHED();
   CB_CUDA(cudaGetLastError());
-  CB_CUDA(cudaMemcpyAsync(game_states, t->d_rows, (size_t)n * CB200_STATE_SIZE * sizeof(float),
+  CB_CUDA(cudaMemcpyAsync(game_states, s.d_rows, (size_t)n * CB200_STATE_SIZE * sizeof(float),
                           cudaMemcpyDeviceToHost, cur_stream()));
   CB_CUDA(cudaStreamSynchronize(cur_stream()));
   return CB200_OK;
@@ -2096,29 +2085,23 @@ int cb200_tourney_do_iteration(cb200_tourney *T, const float *eval, const float 
   int rc = tourney_ready(T);
   if (rc) return rc;
   if ((rc = tourney_scan(T, id)) != CB200_OK) return rc;
-  cb200_trainer *t = T->t;
-  const int need = t->h_summary[3];  // rows the matches will read (reference offset rule)
+  GameStore &s = T->s;
+  const int need = s.h_summary[3];  // rows the matches will read (reference offset rule)
   if (need > 0) {
     if (!eval || !probs) return set_error(CB200_ERR_ARG, "requests pending but eval/probs null");
-    if (need > rows || (size_t)need > t->cap)
+    if (need > rows || (size_t)need > s.cap)
       return set_error(CB200_ERR_ARG, "cb200_tourney_do_iteration: the answer offsets of "
                                       "tourney.cpp:54-62 reach past the caller's buffers");
-    CB_CUDA(cudaMemcpyAsync(t->d_eval, eval, (size_t)need * sizeof(float), cudaMemcpyHostToDevice,
-                            cur_stream()));
-    CB_CUDA(cudaMemcpyAsync(t->d_probs, probs, (size_t)need * CB200_NUM_MOVES * sizeof(float),
-                            cudaMemcpyHostToDevice, cur_stream()));
+    if ((rc = store_stage_answers(s, eval, probs, need)) != CB200_OK) return rc;
   }
-  const int grid = (t->P.num_games + kTreeWarps - 1) / kTreeWarps;
-  k_match_iterate<<<grid, kTreeWarps * 32, 0, cur_stream()>>>(t->P, T->d_sides, t->d_eval, t->d_probs,
+  const int grid = (s.P.num_games + kTreeWarps - 1) / kTreeWarps;
+  k_match_iterate<<<grid, kTreeWarps * 32, 0, cur_stream()>>>(s.P, T->d_sides, s.d_eval, s.d_probs,
                                                             T->d_iter_offs, id, CB200_NUM_MOVES, 1);
   CB_LAUNCHED();
   CB_CUDA(cudaGetLastError());
   if ((rc = tourney_scan(T, id)) != CB200_OK) return rc;
-  if (t->h_summary[2] != 0)
-    return set_error(t->h_summary[2], "a match overflowed its node arena / path buffer (raise "
-                                      "CB200_ARENA_NODES) or reached an impossible state");
-  ++t->iterations_done;
-  return tourney_drain_logs(T);
+  ++s.iterations_done;
+  return store_drain_logs(s);
 }
 
 // ---- fused tourney: the per-model evaluation of rating/tourney.pyx:139-155 on the device ------
@@ -2126,18 +2109,17 @@ int cb200_tourney_set_weights(cb200_tourney *T, int model_id, const float *weigh
                               int precision) {
   last_error_ref().clear();
   if (!T) return set_error(CB200_ERR_ARG, "null tourney");
-  if (model_id < 0 || !weights || n_floats != kNetWeightFloats || precision < 0 || precision > 3)
-    return set_error(CB200_ERR_ARG, "cb200_tourney_set_weights: bad arguments (model id >= 0, 127997 floats, "
-                                    "precision 0|1|2|3)");
-  resident_net_set(T->nets[model_id], weights, precision);
-  return CB200_OK;
+  if (model_id < 0) return set_error(CB200_ERR_ARG, "cb200_tourney_set_weights: model id must be >= 0");
+  const int rc = check_weights(weights, n_floats, precision, "cb200_tourney_set_weights");
+  if (rc == CB200_OK) resident_net_set(T->nets[model_id], weights, precision);
+  return rc;
 }
 
 int cb200_tourney_run(cb200_tourney *T, int max_rounds) {
   int rc = tourney_ready(T);
   if (rc) return rc;
-  cb200_trainer *t = T->t;
-  if ((rc = guard(t)) != CB200_OK) return rc;
+  GameStore &s = T->s;
+  if ((rc = store_guard(s)) != CB200_OK) return rc;
   for (int id : T->model_order) {
     if (id < 0) continue;  // random players: no network (tourney.pyx feeds them no evaluation)
     auto it = T->nets.find(id);
@@ -2146,40 +2128,44 @@ int cb200_tourney_run(cb200_tourney *T, int max_rounds) {
     if ((rc = resident_net_upload(it->second)) != CB200_OK) return rc;
   }
   cudaStream_t st = cur_stream();
-  const int grid = (t->P.num_games + kTreeWarps - 1) / kTreeWarps;
+  const int grid = (s.P.num_games + kTreeWarps - 1) / kTreeWarps;
+  const int ld = (int)(s.cap + kAnswerSlack);  // leading dimension of move-major answers
   int rounds = 0;
   for (;;) {
     // all_done() check (tourney.pyx:118) every few rounds: one small read-back
-    k_match_scan<<<1, 1024, 0, st>>>(t->P, T->d_sides, 0x7fffffff, T->d_pack_offs, T->d_iter_offs, t->d_summary);
+    k_match_scan<<<1, 1024, 0, st>>>(s.P, T->d_sides, 0x7fffffff, T->d_pack_offs, T->d_iter_offs, s.d_summary);
     CB_LAUNCHED();
     CB_CUDA(cudaGetLastError());
-    if ((rc = fetch_summary(t)) != CB200_OK) return rc;
-    if (t->h_summary[1] == 0) return tourney_drain_logs(T) != CB200_OK ? CB200_ERR_CUDA : 1;
+    if ((rc = store_fetch_summary(s)) != CB200_OK) return rc;
+    if (s.h_summary[1] == 0) return store_drain_logs(s) != CB200_OK ? CB200_ERR_CUDA : 1;
     if (max_rounds > 0 && rounds >= max_rounds) break;
     int batch = 8;
     if (max_rounds > 0 && max_rounds - rounds < batch) batch = max_rounds - rounds;
     for (int r = 0; r < batch; ++r) {
       for (int id : T->model_order) {
         // offsets of both kinds + request count of this model (summary[0], read by the network)
-        k_match_scan<<<1, 1024, 0, st>>>(t->P, T->d_sides, id, T->d_pack_offs, T->d_iter_offs, t->d_summary);
+        k_match_scan<<<1, 1024, 0, st>>>(s.P, T->d_sides, id, T->d_pack_offs, T->d_iter_offs, s.d_summary);
         CB_LAUNCHED();
         long prs = CB200_NUM_MOVES, pcs = 1;
         if (id >= 0) {
-          k_match_pack<<<(t->P.num_games + 7) / 8, 256, 0, st>>>(t->P, T->d_sides, id, T->d_pack_offs, nullptr,
-                                                                 t->d_packed);
+          k_match_pack<<<(s.P.num_games + 7) / 8, 256, 0, st>>>(s.P, T->d_sides, id, T->d_pack_offs, nullptr,
+                                                                 s.d_packed);
           CB_LAUNCHED();
-          if ((rc = resident_net_launch(T->nets[id], t, t->d_packed, prs, pcs)) != CB200_OK) return rc;
+          const Net &net = T->nets[id].net;
+          if ((rc = net_launch(net, s.d_packed, s.d_summary, 0, (int)s.cap, s.d_eval, s.d_probs, ld)) != CB200_OK)
+            return rc;
+          if (net.tensor_core()) prs = 1, pcs = ld;
         }
-        k_match_iterate<<<grid, kTreeWarps * 32, 0, st>>>(t->P, T->d_sides, t->d_eval, t->d_probs, T->d_iter_offs,
+        k_match_iterate<<<grid, kTreeWarps * 32, 0, st>>>(s.P, T->d_sides, s.d_eval, s.d_probs, T->d_iter_offs,
                                                           id, prs, pcs);
         CB_LAUNCHED();
         CB_CUDA(cudaGetLastError());
       }
-      ++t->iterations_done;
+      ++s.iterations_done;
     }
     rounds += batch;
   }
-  rc = tourney_drain_logs(T);
+  rc = store_drain_logs(s);
   return rc != CB200_OK ? rc : 0;
 }
 
@@ -2188,12 +2174,12 @@ int cb200_tourney_write_scores(cb200_tourney *T, const char *file) {
   int rc = tourney_ready(T);
   if (rc) return rc;
   if (!file) return set_error(CB200_ERR_ARG, "null file name");
-  cb200_trainer *t = T->t;
-  if ((rc = fetch_ctl(t)) != CB200_OK) return rc;
+  GameStore &s = T->s;
+  if ((rc = store_fetch_ctl(s)) != CB200_OK) return rc;
   std::ofstream f(file, std::ofstream::out);
   if (!f) return set_error(CB200_ERR_ARG, std::string("cannot open ") + file);
-  for (int g = 0; g < t->P.num_games; ++g) {
-    const int32_t *c = t->h_ctl.data() + (size_t)g * kCtlWords;
+  for (int g = 0; g < s.P.num_games; ++g) {
+    const int32_t *c = s.h_ctl.data() + (size_t)g * kCtlWords;
     if (!c[CW_DONE]) continue;
     f << T->matches[g].first << ' ' << T->matches[g].second << ' ' << game_score(c[CW_RESULT]) << '\n';
   }
@@ -2203,13 +2189,14 @@ int cb200_tourney_write_scores(cb200_tourney *T, const char *file) {
 int cb200_tourney_counters(cb200_tourney *T, int64_t out[4]) {
   int rc = tourney_ready(T);
   if (rc) return rc;
-  return cb200_trainer_counters(T->t, out);
+  if ((rc = store_guard(T->s)) != CB200_OK) return rc;
+  return store_counters(T->s, out);
 }
 
 // ==============================================================================================
 // Analysis (the reference's DockerMC, dockermc.cpp, for a batch of given positions); device side
-// in analysis.cuh. The positions use the per-game storage of an internal testing-mode trainer, one
-// "game" per position, created with the analysis object; every run re-seeds and resets it.
+// in analysis.cuh. One "game" of the analysis' store per position, sized for max_positions when the
+// analysis is created; every run re-seeds and resets it.
 
 // The structural invariants of a cstate that the engine accepts from a caller (checked over the
 // reachable positions of 1 000 000 random play-outs by tests/test_oracle_analysis.py): side to move
@@ -2241,14 +2228,14 @@ int64_t cb200_check_states(int64_t n, const uint64_t *states, uint8_t *valid) {
 
 struct cb200_analysis {
   int max_positions = 0, max_searches = 0;
-  cb200_trainer *t = nullptr;  // trainer max_searches = max(max_searches, spe): it sizes the arenas only
+  GameStore s;  // its P.max_searches = max(max_searches, spe) sizes the arenas only
   ulonglong2 *d_roots = nullptr;   // [max_positions] the positions of the current run
   int32_t *d_moves = nullptr, *d_results = nullptr, *d_visits = nullptr;
   float *d_values = nullptr, *d_evals = nullptr;
   ResidentNet net;
   int64_t counters[2] = {0, 0};    // {simulations, leaf evaluations} of the last run or session
   // external-evaluator session (cb200_analysis_begin .. _results): kNoSession, kOpen or kDone;
-  // `requests` = rows the next do_iteration reads, at the offsets the last scan left in t->d_offs
+  // `requests` = rows the next do_iteration reads, at the offsets the last scan left in s.d_offs
   enum { kNoSession, kOpen, kDone };
   int session = kNoSession;
   int requests = 0;
@@ -2265,14 +2252,12 @@ static int analysis_check_states(const cb200_analysis *A, int n, const uint64_t 
   return CB200_OK;
 }
 
-// positions [0, n) become games [0, n) of the trainer: seeds = outputs 0 .. n-1 of mt19937(seed),
+// positions [0, n) become games [0, n) of the store: seeds = outputs 0 .. n-1 of mt19937(seed),
 // fresh control blocks and trees (the kernel builds each root on its first round); the reset leaves
 // zero request offsets and a zero summary behind
 static int analysis_start(cb200_analysis *A, int n, const uint64_t *states, int seed) {
-  cb200_trainer *t = A->t;
   A->counters[0] = A->counters[1] = 0;
-  t->P.num_games = n;
-  int rc = cb200_trainer_reset(t, seed);
+  const int rc = store_reset(A->s, n, seed);
   if (rc != CB200_OK) return rc;
   CB_CUDA(cudaMemcpyAsync(A->d_roots, states, (size_t)n * sizeof(ulonglong2), cudaMemcpyHostToDevice, cur_stream()));
   return CB200_OK;
@@ -2282,14 +2267,14 @@ static int analysis_start(cb200_analysis *A, int n, const uint64_t *states, int 
 // eval[row], probs[row * prs + move * pcs].
 static int analysis_launch(cb200_analysis *A, const float *eval, const float *probs, long prs, long pcs,
                            bool want_evals) {
-  cb200_trainer *t = A->t;
+  GameStore &s = A->s;
   const AnalysisOut out{A->d_moves, A->d_results, A->d_values, A->d_visits, want_evals ? A->d_evals : nullptr};
-  const int grid = (t->P.num_games + kTreeWarps - 1) / kTreeWarps;
-  k_analysis_iterate<<<grid, kTreeWarps * 32, 0, cur_stream()>>>(t->P, A->max_searches, A->d_roots, eval, probs,
-                                                                 prs, pcs, t->d_offs, out);
+  const int grid = (s.P.num_games + kTreeWarps - 1) / kTreeWarps;
+  k_analysis_iterate<<<grid, kTreeWarps * 32, 0, cur_stream()>>>(s.P, A->max_searches, A->d_roots, eval, probs,
+                                                                 prs, pcs, s.d_offs, out);
   CB_LAUNCHED();
   CB_CUDA(cudaGetLastError());
-  ++t->iterations_done;
+  ++s.iterations_done;
   return CB200_OK;
 }
 
@@ -2297,8 +2282,7 @@ static int analysis_launch(cb200_analysis *A, const float *eval, const float *pr
 // read-back synchronises the stream).
 static int analysis_copy_out(cb200_analysis *A, int32_t *moves, int32_t *results, float *values, int32_t *visits,
                              float *evals) {
-  cb200_trainer *t = A->t;
-  const size_t n = (size_t)t->P.num_games;
+  const size_t n = (size_t)A->s.P.num_games;
   cudaStream_t st = cur_stream();
   CB_CUDA(cudaMemcpyAsync(moves, A->d_moves, n * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
   CB_CUDA(cudaMemcpyAsync(results, A->d_results, n * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
@@ -2307,7 +2291,7 @@ static int analysis_copy_out(cb200_analysis *A, int32_t *moves, int32_t *results
   if (evals)
     CB_CUDA(cudaMemcpyAsync(evals, A->d_evals, n * CB200_NUM_MOVES * sizeof(float), cudaMemcpyDeviceToHost, st));
   int64_t c4[4];
-  int rc = cb200_trainer_counters(t, c4);
+  int rc = store_counters(A->s, c4);
   if (rc != CB200_OK) return rc;
   A->counters[0] = c4[0], A->counters[1] = c4[2];
   return CB200_OK;
@@ -2322,14 +2306,13 @@ cb200_analysis *cb200_analysis_create(int max_positions, int max_searches, int s
     set_error(CB200_ERR_ARG, "cb200_analysis_create: invalid argument");
     return nullptr;
   }
-  cb200_trainer *t = cb200_trainer_create_shard(max_positions, 0, max_positions, "", 0,
-                                                std::max(max_searches, searches_per_eval), searches_per_eval,
-                                                c_puct, epsilon, 0, 1);
-  if (!t) return nullptr;
   cb200_analysis *A = new cb200_analysis();
-  A->max_positions = max_positions, A->max_searches = max_searches, A->t = t;
+  A->max_positions = max_positions, A->max_searches = max_searches;
   const size_t n = (size_t)max_positions;
-  if (dmalloc(&A->d_roots, n) != CB200_OK || dmalloc(&A->d_moves, n) != CB200_OK ||
+  // c_puct and epsilon go into P: k_analysis_iterate searches with them and with the sqrt table
+  if (store_create(A->s, max_positions, std::max(max_searches, searches_per_eval), searches_per_eval, c_puct, epsilon,
+                   1, false, {}) != CB200_OK ||
+      dmalloc(&A->d_roots, n) != CB200_OK || dmalloc(&A->d_moves, n) != CB200_OK ||
       dmalloc(&A->d_results, n) != CB200_OK || dmalloc(&A->d_values, n) != CB200_OK ||
       dmalloc(&A->d_visits, n * CB200_NUM_MOVES) != CB200_OK ||
       dmalloc(&A->d_evals, n * CB200_NUM_MOVES) != CB200_OK) {
@@ -2343,21 +2326,20 @@ cb200_analysis *cb200_analysis_create(int max_positions, int max_searches, int s
 
 void cb200_analysis_destroy(cb200_analysis *A) {
   if (!A) return;
-  if (A->t) cudaSetDevice(A->t->device);
+  cudaSetDevice(A->s.device);
   cudaFree(A->d_roots), cudaFree(A->d_moves), cudaFree(A->d_results), cudaFree(A->d_values);
   cudaFree(A->d_visits), cudaFree(A->d_evals);
-  resident_net_free(A->net);
-  if (A->t) cb200_trainer_destroy(A->t);
+  net_free(A->net.net);
+  store_free(A->s);
   delete A;
 }
 
 int cb200_analysis_set_weights(cb200_analysis *A, const float *weights, size_t n_floats, int precision) {
   last_error_ref().clear();
   if (!A) return set_error(CB200_ERR_ARG, "null analysis");
-  if (!weights || n_floats != kNetWeightFloats || precision < 0 || precision > 3)
-    return set_error(CB200_ERR_ARG, "cb200_analysis_set_weights: bad arguments (127997 floats, precision 0|1|2|3)");
-  resident_net_set(A->net, weights, precision);
-  return CB200_OK;
+  const int rc = check_weights(weights, n_floats, precision, "cb200_analysis_set_weights");
+  if (rc == CB200_OK) resident_net_set(A->net, weights, precision);
+  return rc;
 }
 
 int cb200_analysis_run(cb200_analysis *A, int n, const uint64_t *states, int seed, int32_t *moves,
@@ -2370,27 +2352,29 @@ int cb200_analysis_run(cb200_analysis *A, int n, const uint64_t *states, int see
   int rc = analysis_check_states(A, n, states, "cb200_analysis_run");
   if (rc != CB200_OK) return rc;
   if (A->net.precision < 0) return set_error(CB200_ERR_STATE, "cb200_analysis_run: no weights set");
-  cb200_trainer *t = A->t;
-  if ((rc = guard(t)) != CB200_OK) return rc;
+  GameStore &s = A->s;
+  if ((rc = store_guard(s)) != CB200_OK) return rc;
   if ((rc = resident_net_upload(A->net)) != CB200_OK) return rc;
   if ((rc = analysis_start(A, n, states, seed)) != CB200_OK) return rc;
   cudaStream_t st = cur_stream();
+  const Net &net = A->net.net;
+  const int ld = (int)(s.cap + kAnswerSlack);  // leading dimension of move-major answers
+  const long prs = net.tensor_core() ? 1 : CB200_NUM_MOVES, pcs = net.tensor_core() ? ld : 1;
   // every round completes at least one search or the turn of each live position
   const int max_rounds = A->max_searches + 8;
   for (int round = 0;; ++round) {
     // request offsets of every live position (contiguous packing) and the live count
-    k_scan_requests<<<1, 1024, 0, st>>>(t->P, -1, t->d_offs, t->d_summary);
+    k_scan_requests<<<1, 1024, 0, st>>>(s.P, -1, s.d_offs, s.d_summary);
     CB_LAUNCHED();
     if (round % 8 == 0) {  // one small read-back every few rounds
-      if ((rc = fetch_summary(t)) != CB200_OK) return rc;
-      if (t->h_summary[1] == 0) break;
+      if ((rc = store_fetch_summary(s)) != CB200_OK) return rc;
+      if (s.h_summary[1] == 0) break;
       if (round > max_rounds) return set_error(CB200_ERR_STATE, "cb200_analysis_run: the searches did not finish");
     }
-    k_pack_requests<<<(n + 7) / 8, 256, 0, st>>>(t->P, -1, t->d_offs, nullptr, t->d_packed);
+    k_pack_requests<<<(n + 7) / 8, 256, 0, st>>>(s.P, -1, s.d_offs, nullptr, s.d_packed);
     CB_LAUNCHED();
-    long prs = 0, pcs = 0;
-    if ((rc = resident_net_launch(A->net, t, t->d_packed, prs, pcs)) != CB200_OK) return rc;
-    if ((rc = analysis_launch(A, t->d_eval, t->d_probs, prs, pcs, evals != nullptr)) != CB200_OK) return rc;
+    if ((rc = net_launch(net, s.d_packed, s.d_summary, 0, (int)s.cap, s.d_eval, s.d_probs, ld)) != CB200_OK) return rc;
+    if ((rc = analysis_launch(A, s.d_eval, s.d_probs, prs, pcs, evals != nullptr)) != CB200_OK) return rc;
   }
   return analysis_copy_out(A, moves, results, values, visits, evals);
 }
@@ -2403,7 +2387,7 @@ int cb200_analysis_run(cb200_analysis *A, int n, const uint64_t *states, int see
 static int analysis_session(cb200_analysis *A, const char *who) {
   if (A->session == cb200_analysis::kNoSession)
     return set_error(CB200_ERR_STATE, std::string(who) + ": no open session (cb200_analysis_begin)");
-  const int rc = guard(A->t);
+  const int rc = store_guard(A->s);
   if (rc == CB200_OK) return CB200_OK;
   A->session = cb200_analysis::kNoSession;
   return rc;
@@ -2415,7 +2399,7 @@ int cb200_analysis_begin(cb200_analysis *A, int n, const uint64_t *states, int s
   A->session = cb200_analysis::kNoSession;  // a new begin discards an open session, even when it fails
   int rc = analysis_check_states(A, n, states, "cb200_analysis_begin");
   if (rc != CB200_OK) return rc;
-  if ((rc = guard(A->t)) != CB200_OK) return rc;
+  if ((rc = store_guard(A->s)) != CB200_OK) return rc;
   if ((rc = analysis_start(A, n, states, seed)) != CB200_OK) return rc;
   A->requests = 0;  // the first do_iteration queues the roots
   A->session = cb200_analysis::kOpen;
@@ -2431,14 +2415,14 @@ int cb200_analysis_num_requests(cb200_analysis *A) {
 
 // A caller's buffer of the device forms must be device (or managed) memory of the analysis' device:
 // anything else would fault inside the kernel.
-static int check_device_buffer(const cb200_trainer *t, const void *p, const char *who, const char *what) {
+static int check_device_buffer(const GameStore &s, const void *p, const char *who, const char *what) {
   cudaPointerAttributes at{};
   const bool ok = cudaPointerGetAttributes(&at, p) == cudaSuccess &&
-                  (at.type == cudaMemoryTypeDevice || at.type == cudaMemoryTypeManaged) && at.device == t->device;
+                  (at.type == cudaMemoryTypeDevice || at.type == cudaMemoryTypeManaged) && at.device == s.device;
   cudaGetLastError();  // a failed query leaves nothing behind for the next launch check
   if (ok) return CB200_OK;
   return set_error(CB200_ERR_ARG, std::string(who) + ": " + what + " is not device memory of device " +
-                                      std::to_string(t->device));
+                                      std::to_string(s.device));
 }
 
 // Packs the pending requests (position-major, pending order within a position) into rows on the
@@ -2446,10 +2430,10 @@ static int check_device_buffer(const cb200_trainer *t, const void *p, const char
 static int analysis_write_requests(cb200_analysis *A, float *rows, float *host_out, const char *who) {
   int rc = analysis_session(A, who);
   if (rc != CB200_OK || A->requests == 0) return rc;
-  cb200_trainer *t = A->t;
-  if (!host_out && (rc = check_device_buffer(t, rows, who, "rows_device")) != CB200_OK) return rc;
+  GameStore &s = A->s;
+  if (!host_out && (rc = check_device_buffer(s, rows, who, "rows_device")) != CB200_OK) return rc;
   cudaStream_t st = cur_stream();
-  k_pack_requests<<<(t->P.num_games + 7) / 8, 256, 0, st>>>(t->P, -1, t->d_offs, rows, nullptr);
+  k_pack_requests<<<(s.P.num_games + 7) / 8, 256, 0, st>>>(s.P, -1, s.d_offs, rows, nullptr);
   CB_LAUNCHED();
   CB_CUDA(cudaGetLastError());
   if (host_out) {
@@ -2463,7 +2447,7 @@ static int analysis_write_requests(cb200_analysis *A, float *rows, float *host_o
 int cb200_analysis_write_requests(cb200_analysis *A, float *game_states) {
   last_error_ref().clear();
   if (!A || !game_states) return set_error(CB200_ERR_ARG, "cb200_analysis_write_requests: null analysis / game_states");
-  return analysis_write_requests(A, A->t->d_rows, game_states, "cb200_analysis_write_requests");
+  return analysis_write_requests(A, A->s.d_rows, game_states, "cb200_analysis_write_requests");
 }
 
 int cb200_analysis_write_requests_device(cb200_analysis *A, void *rows_device) {
@@ -2487,32 +2471,29 @@ static int analysis_do_iteration(cb200_analysis *A, const float *eval, const flo
   if (rows < need)
     return set_error(CB200_ERR_ARG, std::string(who) + ": " + std::to_string(rows) + " answer rows given, " +
                                         std::to_string(need) + " requests pending");
-  cb200_trainer *t = A->t;
-  cudaStream_t st = cur_stream();
-  const float *ev = t->d_eval, *pr = t->d_probs;
+  GameStore &s = A->s;
+  const float *ev = s.d_eval, *pr = s.d_probs;
   if (need > 0 && on_device) {
-    if ((rc = check_device_buffer(t, eval, who, "eval_device")) != CB200_OK ||
-        (rc = check_device_buffer(t, probs, who, "probs_device")) != CB200_OK)
+    if ((rc = check_device_buffer(s, eval, who, "eval_device")) != CB200_OK ||
+        (rc = check_device_buffer(s, probs, who, "probs_device")) != CB200_OK)
       return rc;
     ev = eval, pr = probs;
-  } else if (need > 0) {
-    CB_CUDA(cudaMemcpyAsync(t->d_eval, eval, (size_t)need * sizeof(float), cudaMemcpyHostToDevice, st));
-    CB_CUDA(cudaMemcpyAsync(t->d_probs, probs, (size_t)need * CB200_NUM_MOVES * sizeof(float),
-                            cudaMemcpyHostToDevice, st));
+  } else if (need > 0 && (rc = store_stage_answers(s, eval, probs, need)) != CB200_OK) {
+    return rc;
   }
   if ((rc = analysis_launch(A, ev, pr, CB200_NUM_MOVES, 1, true)) == CB200_OK) {
-    k_scan_requests<<<1, 1024, 0, st>>>(t->P, -1, t->d_offs, t->d_summary);
+    k_scan_requests<<<1, 1024, 0, cur_stream()>>>(s.P, -1, s.d_offs, s.d_summary);
     CB_LAUNCHED();
-    rc = fetch_summary(t);  // an overflow of any position surfaces here
+    rc = store_fetch_summary(s);  // an overflow of any position surfaces here
   }
   if (rc != CB200_OK) {
     A->session = cb200_analysis::kNoSession;
     return rc;
   }
-  A->requests = t->h_summary[0];
-  if (t->h_summary[1] != 0) return 0;
+  A->requests = s.h_summary[0];
+  if (s.h_summary[1] != 0) return 0;
   int64_t c4[4];
-  if ((rc = cb200_trainer_counters(t, c4)) != CB200_OK) {
+  if ((rc = store_counters(s, c4)) != CB200_OK) {
     A->session = cb200_analysis::kNoSession;
     return rc;
   }
@@ -2550,7 +2531,8 @@ int cb200_analysis_counters(cb200_analysis *A, int64_t out[2]) {
   if (!A || !out) return set_error(CB200_ERR_ARG, "null analysis / out");
   if (A->session == cb200_analysis::kOpen) {  // the running totals of the session so far
     int64_t c4[4];
-    const int rc = cb200_trainer_counters(A->t, c4);
+    int rc = store_guard(A->s);
+    if (rc == CB200_OK) rc = store_counters(A->s, c4);
     if (rc != CB200_OK) return rc;
     A->counters[0] = c4[0], A->counters[1] = c4[2];
   }
