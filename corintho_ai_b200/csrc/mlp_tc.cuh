@@ -34,6 +34,9 @@
 #include <cuda_bf16.h>
 #include <cuda_fp16.h>
 
+#include <cstring>
+#include <vector>
+
 #include "common.cuh"
 
 namespace cb200 {
@@ -202,21 +205,24 @@ __device__ __forceinline__ void tmem_wait_st() {
 __device__ __forceinline__ void tmem_wait_ld() {
   asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
 }
-// two fp32 -> packed 16-bit pair (bf16 or fp16) with ReLU, `lo` in bits 0-15
+// two fp32 -> packed 16-bit pair (bf16 or fp16) with ReLU, `lo` in bits 0-15. fp16 saturates at
+// +-65504: a plain round would give inf past it, and the next layer's inf * 0 would put NaN into
+// every output.
 template <bool kFp16>
 __device__ __forceinline__ uint32_t relu_pack16(uint32_t lo, uint32_t hi) {
   uint32_t d;
   if (kFp16)
-    asm("cvt.rn.relu.f16x2.f32 %0, %1, %2;" : "=r"(d) : "f"(__uint_as_float(hi)), "f"(__uint_as_float(lo)));
+    asm("cvt.rn.satfinite.relu.f16x2.f32 %0, %1, %2;" : "=r"(d) : "f"(__uint_as_float(hi)), "f"(__uint_as_float(lo)));
   else
     asm("cvt.rn.relu.bf16x2.f32 %0, %1, %2;" : "=r"(d) : "f"(__uint_as_float(hi)), "f"(__uint_as_float(lo)));
   return d;
 }
 template <bool kFp16>
 __device__ __forceinline__ uint32_t pack16(float a, float b) {
-  if (kFp16) {
-    const __half2 h = __floats2half2_rn(a, b);
-    return *reinterpret_cast<const uint32_t *>(&h);
+  if (kFp16) {  // saturating like relu_pack16
+    uint32_t d;
+    asm("cvt.rn.satfinite.f16x2.f32 %0, %1, %2;" : "=r"(d) : "f"(b), "f"(a));
+    return d;
   }
   const __nv_bfloat162 h = __floats2bfloat162_rn(a, b);
   return *reinterpret_cast<const uint32_t *>(&h);

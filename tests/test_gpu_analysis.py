@@ -46,7 +46,7 @@ def positions(oracle):
     return st
 
 
-@pytest.mark.parametrize("precision", ["fp32", "bf16"])
+@pytest.mark.parametrize("precision", ["fp32", "bf16", "fp16", "bf16x3"])
 @pytest.mark.parametrize("ms,spe,c_puct,eps", PARAMS)
 def test_analysis_equals_oracle_driven_by_the_same_network(oracle, positions, precision, ms, spe, c_puct,
                                                            eps):

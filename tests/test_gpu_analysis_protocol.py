@@ -98,7 +98,7 @@ def test_protocol_equals_oracle_round_by_round(oracle, positions, evaluator, ms,
     assert c["leaf_evals"] == rows_served
 
 
-@pytest.mark.parametrize("precision", ["fp32", "bf16"])
+@pytest.mark.parametrize("precision", ["fp32", "bf16", "fp16", "bf16x3"])
 @pytest.mark.parametrize("ms,spe,c_puct,eps", PARAMS)
 def test_protocol_with_the_network_equals_the_fused_run(positions, precision, ms, spe, c_puct, eps):
     weights = cb.fold_batchnorm(cb.random_weights(31))

@@ -484,3 +484,82 @@ def test_bf16x3_persistent_tail_equals_lock_step(monkeypatch, testing):
     got, kt1 = run()
     assert kt1["fused_tail"]["launches"] >= 1
     assert got == base
+
+
+def test_fused_selfplay_fp16_equals_oracle_driven_by_the_same_network(oracle):
+    """fp16 operands through the fused loop: 40 games that hand over to the persistent tail
+    (k_selfplay_persistent in fp16), against the oracle fed with the same kernel's outputs."""
+    flat = cb.fold_batchnorm(cb.random_weights(34))
+    cfg = dict(num_games=40, seed=6, max_searches=48, searches_per_eval=16, c_puct=1.0, epsilon=0.25)
+    fused = cb.Trainer(cfg["num_games"], "", cfg["seed"], cfg["max_searches"], cfg["searches_per_eval"],
+                       cfg["c_puct"], cfg["epsilon"])
+    fused.set_weights(flat, 0, "fp16")
+    fused.set_profiling(True)
+    assert fused.run_selfplay(0, stagger=True)
+    assert fused.kernel_times()["fused_tail"]["launches"] >= 1
+    helper = cb.Trainer(cfg["num_games"], "", 1, 64, cfg["searches_per_eval"])
+    helper.set_weights(flat, 0, "fp16")
+    o = oracle.trainer(**cfg)
+    r = run_trainer(o, lambda req: helper.evaluate(req))
+    gs, ev, pr = fused.write_samples()
+    assert fused.num_samples() == r["num_samples"]
+    assert gs.tobytes() == r["samples"][0].tobytes()
+    assert ev.tobytes() == r["samples"][1].tobytes()
+    assert pr.tobytes() == r["samples"][2].tobytes()
+    oc, ec = oracle.counters(o), fused.counters()
+    assert (oc["simulations"], oc["moves"], oc["leaf_evals"]) == (ec["simulations"], ec["moves"], ec["leaf_evals"])
+
+
+def test_fused_testing_mode_two_models_fp16(oracle):
+    """Two-model match with both networks in fp16 operands (persistent tail, one row region per
+    model) == the oracle driven by the same two networks."""
+    fa, fb = cb.fold_batchnorm(cb.random_weights(15)), cb.fold_batchnorm(cb.random_weights(16))
+    G, MS, SPE = 40, 48, 8
+    t = cb.Trainer(G, "", 4, MS, SPE, 1.0, 0.0, 0, 1, True)
+    t.set_weights(fa, 0, "fp16")
+    t.set_weights(fb, 1, "fp16")
+    t.set_profiling(True)
+    assert t.run_selfplay(0)
+    assert t.kernel_times()["fused_tail"]["launches"] >= 1
+    h = [cb.Trainer(G, "", 1, 16, SPE) for _ in range(2)]
+    h[0].set_weights(fa, 0, "fp16")
+    h[1].set_weights(fb, 0, "fp16")
+    o = oracle.trainer(num_games=G, seed=4, max_searches=MS, searches_per_eval=SPE, c_puct=1.0,
+                       epsilon=0.0, testing=True)
+    ev = np.zeros(G * SPE, np.float32)
+    pr = np.zeros((G * SPE, 96), np.float32)
+    done, tp = False, 0
+    while not done:
+        n = o.num_requests(tp)
+        if n:
+            e, p = h[tp].evaluate(o.write_requests(tp))
+            ev[:n], pr[:n] = e, p
+        done = o.do_iteration(ev, pr, tp)
+        tp = 1 - tp
+    oc, ec = oracle.counters(o), t.counters()
+    assert t.score().tobytes() == o.score().tobytes()
+    assert (oc["simulations"], oc["moves"], oc["leaf_evals"]) == (ec["simulations"], ec["moves"], ec["leaf_evals"])
+    assert (t.game_results() != 0).all()
+
+
+@pytest.mark.parametrize("precision", ["fp16", "bf16x3"])
+def test_single_tile_network_in_stream_groups_equals_one_group(monkeypatch, precision):
+    """With more than one stream group the lock-step loop runs the single-tile network CTA
+    (k_mlp_tc1<1> for fp16, k_mlp_tc1<2> for bf16x3) beside the game step; 2 and 3 groups must
+    play exactly the games of one group."""
+    flat = cb.fold_batchnorm(cb.random_weights(23))
+
+    def run(groups):
+        monkeypatch.setenv("CB200_GROUPS", str(groups))
+        monkeypatch.setenv("CB200_PS_CAPACITY", "40")  # lock-step until 40 games are left
+        t = cb.Trainer(240, "", 55, 48, 16, 1.0, 0.25)
+        t.set_weights(flat, 0, precision)
+        assert t.run_selfplay(0, stagger=False)
+        gs, ev, pr = t.write_samples()
+        c = t.counters()
+        return (gs.tobytes(), ev.tobytes(), pr.tobytes(), t.score().tobytes(),
+                (c["simulations"], c["moves"], c["leaf_evals"]))
+
+    base = run(1)
+    assert run(2) == base
+    assert run(3) == base

@@ -75,7 +75,7 @@ def test_tourney_protocol_and_errors(tmp_path):
     assert rows[0].split()[:2] == ["0", "1"] and rows[1].split()[:2] == ["1", "0"]
 
 
-@pytest.mark.parametrize("precision", ["fp32", "bf16"])
+@pytest.mark.parametrize("precision", ["fp32", "bf16", "fp16", "bf16x3"])
 @pytest.mark.parametrize("name", ["two_models", "with_random", "deeper"])
 def test_fused_tourney_equals_oracle_driven_by_the_same_networks(oracle, name, precision):
     """Fused tourney (cb200_tourney_set_weights / cb200_tourney_run): every model id has a
