@@ -577,12 +577,16 @@ __device__ __forceinline__ void receive_eval(Ctx &c, const TreeParams &P, WarpSm
       sm.fval[i] = __fadd_rn(__fmul_rn(sm.fval[i], sm.l_a[k]), __fmul_rn(sm.dval[i], sm.l_b[k]));
     }
     g_sync(c);
-    // ---- leaf phase 5: max (from 0.0f), denom = 511 / max
+    // ---- leaf phase 5: max (from 0.0f), denom = 511 / max. std::max(w, max) keeps a NaN w and
+    // drops a NaN max, where fmaxf would drop the NaN w (an infinite probability makes one).
     {
       float mx = 0.0f;
 #pragma unroll 4
       for (int j = 0; j < nmax; ++j)
-        if (j < my_cnt) mx = fmaxf(mx, sm.fval[my_i0 + j]);
+        if (j < my_cnt) {
+          const float w = sm.fval[my_i0 + j];
+          mx = w < mx ? mx : w;
+        }
       if (mine) sm.l_a[lane] = __fdiv_rn(511.0f, mx);
     }
     g_sync(c);
@@ -671,8 +675,10 @@ __device__ __forceinline__ void receive_eval(Ctx &c, const TreeParams &P, WarpSm
   c.n_pending = 0;
 }
 
-// PUCT value of one slot (chooseNext, trainmc.cpp:540-600); -inf = not selectable
-__device__ __forceinline__ float puct_u(const uint4 s, float denominator, float v_sqrt) {
+// PUCT value of one slot (chooseNext, trainmc.cpp:540-600); -inf = not selectable. divided =
+// the fast path could not decide the rounding and the value came from the two IEEE divisions.
+__device__ __forceinline__ float puct_u(const uint4 s, float denominator, float v_sqrt, bool &divided) {
+  divided = false;
   const float prob = __fmul_rn((float)s3_prior(s.w), denominator);
   const float pvf = __fmul_rn(prob, v_sqrt);
   float u = pvf;  // no child yet, or a drawn child
@@ -689,7 +695,8 @@ __device__ __forceinline__ float puct_u(const uint4 s, float denominator, float 
       const int cvi = (int)s.y;
       const double ne = -(double)__uint_as_float(s.x);
       const double pv = (double)pvf;
-      const double dn = (double)cvi, dn1 = (double)(cvi + 1);
+      // the reference divides by float(N) and float(N) + 1.0, which differ from N and N + 1 above 2^24
+      const double dn = (double)(float)cvi, dn1 = __dadd_rn(dn, 1.0);
       const double ra = fast_rcp(dn), rb = fast_rcp(dn1);
       const double a = __dmul_rn(ne, ra);
       const double b = __dmul_rn(pv, rb);
@@ -699,14 +706,18 @@ __device__ __forceinline__ float puct_u(const uint4 s, float denominator, float 
       const float uhi = __double2float_rn(__dadd_rn(sf, tol));
       u = ulo;
       if (!(ulo == uhi)) {
-        const double cv = (double)(float)cvi;
-        const double a = __ddiv_rn(ne, cv);
-        const double b = __ddiv_rn(pv, __dadd_rn(cv, 1.0));
+        divided = true;
+        const double a = __ddiv_rn(ne, dn);
+        const double b = __ddiv_rn(pv, dn1);
         u = __double2float_rn(__dadd_rn(a, b));
       }
     }
   }
   return __fadd_rn(u, 0.0f);  // -0.0 -> +0.0 so the integer key orders like operator>
+}
+__device__ __forceinline__ float puct_u(const uint4 s, float denominator, float v_sqrt) {
+  bool divided;
+  return puct_u(s, denominator, v_sqrt, divided);
 }
 
 // Cheap screening of the same value: an interval [lo, hi] that provably contains puct_u().
@@ -754,6 +765,83 @@ __device__ __forceinline__ float skey_inv(int k) {
   return __int_as_float(k ^ ((k >> 31) & 0x7fffffff));
 }
 
+// ---- TrainMC::chooseNext (trainmc.cpp:540-600) at one node, for the whole warp ---------------
+// s[j] = slot lane + 32 * j of the record at r (lanes past the last slot hold a word that
+// classifies as "not selectable"); slots from kS * 32 on are read from r. Returns the chosen slot
+// (the first maximum); no_slot = no slot is selectable; exact = the level went to the exact pass.
+template <int kS>
+__device__ __forceinline__ int select_slot(const Ctx &c, const TreeParams &P, const uint32_t *r,
+                                           const uint4 (&s)[kS], int n, float denominator,
+                                           int cur_visits, bool &no_slot, bool &exact) {
+  // sqrt(float) binds to double sqrt(double) (SURVEY Q9); small arguments come from a table
+  // filled by the host with the same expression
+  float v_sqrt;
+  if (P.vsqrt != nullptr && (unsigned)cur_visits < (unsigned)kVsqrtCap)
+    v_sqrt = __ldg(P.vsqrt + cur_visits);
+  else
+    v_sqrt = __double2float_rn(__dmul_rn((double)P.c_puct, sqrt((double)(float)cur_visits)));
+  int emin = -1;
+  bool none = false;
+  exact = false;
+  if (n <= kS * 32) {
+    // screening pass: interval per slot, decide when a single slot (or only exact ones) can
+    // hold the maximum
+    float lo[kS], hi[kS];
+    bool in[kS];
+    float lmx = -INFINITY;
+#pragma unroll
+    for (int j = 0; j < kS; ++j) {
+      lo[j] = hi[j] = -INFINITY, in[j] = false;
+      if (j == 0 || n > 32 * j) in[j] = puct_bounds(s[j], denominator, v_sqrt, lo[j], hi[j]);  // warp-uniform
+      lmx = fmaxf(lmx, lo[j]);
+    }
+    const float lmax = skey_inv(g_max(c, skey(lmx)));
+    if (lmax == -INFINITY) {
+      none = true;
+    } else {
+      // candidates = slots whose interval reaches lmax; per lane: how many, the first one, and
+      // whether any of them is inexact -- then three warp collectives whatever kS is
+      int cnt_l = 0, first_l = 0x7fffffff;
+      bool cin = false;
+#pragma unroll
+      for (int j = kS - 1; j >= 0; --j) {
+        const bool cj = hi[j] >= lmax;
+        cin = cin || (cj && in[j]);
+        cnt_l += cj ? 1 : 0;
+        first_l = cj ? c.lane + 32 * j : first_l;
+      }
+      const int cnt = g_add(c, cnt_l);
+      const bool any_in = g_ballot(c, cin) != 0u;
+      if (!any_in || cnt == 1) emin = g_min(c, first_l);  // ties: the lowest slot wins (operator>)
+    }
+  }
+  if (emin < 0 && !none) {
+    // exact pass (rare): the reference's expression for every slot
+    exact = true;
+    float best_u = -INFINITY;
+    int best_e = 0x7fffffff;
+    for (int e = c.lane, j = 0; e < n; e += 32, ++j) {
+      uint4 sx;
+      if (j < kS) {
+        sx = s[0];
+#pragma unroll
+        for (int q = 1; q < kS; ++q)
+          if (j == q) sx = s[q];
+      } else {
+        sx = ld4(r + 8 + 4 * e);
+      }
+      const float u = puct_u(sx, denominator, v_sqrt);
+      if (u > best_u) best_u = u, best_e = e;
+    }
+    const uint32_t key = fkey(best_u);
+    const uint32_t kmax = g_max(c, key);
+    none = (kmax == kKeyNegInf);
+    if (!none) emin = g_min(c, key == kmax ? best_e : 0x7fffffff);
+  }
+  no_slot = none;  // a copy of the local flag, not emin < 0: search() compiles as it did inline
+  return emin;
+}
+
 // ---- TrainMC::search (trainmc.cpp:602-696) --------------------------------------------------
 // The select loop only walks down existing children; a new edge ends it and the expansion
 // (do_move + legal moves + record write, the long scalar part) runs after the loop.
@@ -794,70 +882,9 @@ __device__ __forceinline__ void search(Ctx &c, const TreeParams &P, WarpSm &sm) 
     const uint4 h1 = ld4(r + 4);
     const int depth = (int)((h1.x >> 8) & 0xffu);
     const float denominator = __uint_as_float(h1.y);
-    // sqrt(float) binds to double sqrt(double) (SURVEY Q9); small arguments come from a table
-    // filled by the host with the same expression
-    float v_sqrt;
-    if (P.vsqrt != nullptr && (unsigned)cur_visits < (unsigned)kVsqrtCap)
-      v_sqrt = __ldg(P.vsqrt + cur_visits);
-    else
-      v_sqrt = __double2float_rn(__dmul_rn((double)P.c_puct, sqrt((double)(float)cur_visits)));
-    int emin = -1;
-    bool none = false;
-    if (n <= kS * 32) {
-      // screening pass: interval per slot, decide when a single slot (or only exact ones) can
-      // hold the maximum
-      float lo[kS], hi[kS];
-      bool in[kS];
-      float lmx = -INFINITY;
-#pragma unroll
-      for (int j = 0; j < kS; ++j) {
-        lo[j] = hi[j] = -INFINITY, in[j] = false;
-        if (j == 0 || n > 32 * j) in[j] = puct_bounds(s[j], denominator, v_sqrt, lo[j], hi[j]);  // warp-uniform
-        lmx = fmaxf(lmx, lo[j]);
-      }
-      const float lmax = skey_inv(g_max(c, skey(lmx)));
-      if (lmax == -INFINITY) {
-        none = true;
-      } else {
-        // candidates = slots whose interval reaches lmax; per lane: how many, the first one, and
-        // whether any of them is inexact -- then three warp collectives whatever kS is
-        int cnt_l = 0, first_l = 0x7fffffff;
-        bool cin = false;
-#pragma unroll
-        for (int j = kS - 1; j >= 0; --j) {
-          const bool cj = hi[j] >= lmax;
-          cin = cin || (cj && in[j]);
-          cnt_l += cj ? 1 : 0;
-          first_l = cj ? c.lane + 32 * j : first_l;
-        }
-        const int cnt = g_add(c, cnt_l);
-        const bool any_in = g_ballot(c, cin) != 0u;
-        if (!any_in || cnt == 1) emin = g_min(c, first_l);  // ties: the lowest slot wins (operator>)
-      }
-    }
-    if (emin < 0 && !none) {
-      // exact pass (rare): the reference's expression for every slot
-      CB_PROF(c.n_exact += 1;)
-      float best_u = -INFINITY;
-      int best_e = 0x7fffffff;
-      for (int e = c.lane, j = 0; e < n; e += 32, ++j) {
-        uint4 sx;
-        if (j < kS) {
-          sx = s[0];
-#pragma unroll
-          for (int q = 1; q < kS; ++q)
-            if (j == q) sx = s[q];
-        } else {
-          sx = ld4(r + 8 + 4 * e);
-        }
-        const float u = puct_u(sx, denominator, v_sqrt);
-        if (u > best_u) best_u = u, best_e = e;
-      }
-      const uint32_t key = fkey(best_u);
-      const uint32_t kmax = g_max(c, key);
-      none = (kmax == kKeyNegInf);
-      if (!none) emin = g_min(c, key == kmax ? best_e : 0x7fffffff);
-    }
+    bool none, exact;
+    const int emin = select_slot(c, P, r, s, n, denominator, cur_visits, none, exact);
+    CB_PROF(c.n_exact += exact ? 1 : 0;)
     // virtual loss on the node we stand on (trainmc.cpp:611,625)
     if (level == 0) {
       c.root_visits += 1;

@@ -296,6 +296,17 @@ def have_ref():
 
 
 # ---- deterministic synthetic evaluator shared by every parity test --------------------------
+def _row_hash(game_states):
+    gs = np.ascontiguousarray(game_states, np.float32).reshape(-1, 70)
+    q = np.rint(gs * 4.0).astype(np.uint64)  # entries are multiples of 1/4
+    h = np.full(gs.shape[0], 0x9E3779B97F4A7C15, np.uint64)
+    with np.errstate(over="ignore"):
+        for j in range(70):
+            h = (h ^ q[:, j]) * np.uint64(0x100000001B3)
+            h ^= h >> np.uint64(29)
+    return h
+
+
 def synth_eval(game_states):
     """Pure function of the 70-float request rows -> (eval[n] in [-1,1), probs[n,96] in (0,1]).
 
@@ -303,14 +314,8 @@ def synth_eval(game_states):
     (tests/cpp/trainer_test.cpp:37-49) the probabilities are NOT normalised; the search
     renormalises over legal moves (trainmc.cpp:212-234).
     """
-    gs = np.ascontiguousarray(game_states, np.float32).reshape(-1, 70)
-    n = gs.shape[0]
-    q = np.rint(gs * 4.0).astype(np.uint64)  # entries are multiples of 1/4
-    h = np.full(n, 0x9E3779B97F4A7C15, np.uint64)
+    h = _row_hash(game_states)
     with np.errstate(over="ignore"):
-        for j in range(70):
-            h = (h ^ q[:, j]) * np.uint64(0x100000001B3)
-            h ^= h >> np.uint64(29)
         ev = ((h >> np.uint64(11)) & np.uint64(0xFFFF)).astype(np.float32) / np.float32(32768.0) \
             - np.float32(1.0)
         k = np.arange(96, dtype=np.uint64)[None, :]
@@ -320,6 +325,36 @@ def synth_eval(game_states):
         m ^= m >> np.uint64(32)
         pr = ((m & np.uint64(0xFFFF)).astype(np.float32) + np.float32(1.0)) / np.float32(65536.0)
     return ev.astype(np.float32), np.ascontiguousarray(pr, np.float32)
+
+
+# ---- adversarial evaluators: inputs under which the search's ties and degenerate priors decide --
+def tie_storm_eval(game_states):
+    """Evaluations in {-1, -0.5, 0, 0.5, 1} from the row hash and all probabilities equal: equal
+    priors everywhere and many exactly tied PUCT values, so that every tie-break is exercised."""
+    h = _row_hash(game_states)
+    ev = np.array([-1.0, -0.5, 0.0, 0.5, 1.0], np.float32)[(h % np.uint64(5)).astype(np.int64)]
+    return ev, np.ones((len(h), 96), np.float32)
+
+
+def onehot_eval(game_states):
+    """Probability 1 on one hash-chosen move and 0 elsewhere; the move is illegal in most
+    positions, which leaves every legal probability at zero (the priors then come from NaN)."""
+    ev, _ = synth_eval(game_states)
+    h = _row_hash(game_states)
+    pr = np.zeros((len(h), 96), np.float32)
+    pr[np.arange(len(h)), ((h >> np.uint64(17)) % np.uint64(96)).astype(np.int64)] = 1.0
+    return ev, pr
+
+
+def subnormal_eval(game_states):
+    """Probabilities that are 0 to 63 times the smallest subnormal float: their sum's reciprocal
+    overflows float, so the scaled priors are inf, or NaN where a probability is zero."""
+    ev, pr = synth_eval(game_states)
+    k = np.rint(pr * 65536.0).astype(np.uint32) & np.uint32(63)
+    return ev, np.ascontiguousarray(k.astype(np.float32) * np.float32(2.0 ** -149), np.float32)
+
+
+ADVERSARIAL_EVALUATORS = {"tie_storm": tie_storm_eval, "onehot": onehot_eval, "subnormal": subnormal_eval}
 
 
 def play_out(trainer, evaluator=synth_eval, to_play=-1, record=None, max_iters=10_000_000,

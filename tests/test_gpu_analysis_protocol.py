@@ -6,6 +6,7 @@ import pytest
 
 import corintho_ai_b200 as cb
 from analysis_oracle import AnalysisOracle
+from oracle.pyoracle import tie_storm_eval
 from test_gpu_analysis import N, PARAMS, network_evaluator
 from torch_net import torch_network
 
@@ -66,11 +67,13 @@ def assert_same_outputs(got, ref):
             assert (got[k] == ref[k]).all(), k
 
 
-@pytest.mark.parametrize("evaluator", ["fp32", "bf16", "synthetic"])
+@pytest.mark.parametrize("evaluator", ["fp32", "bf16", "synthetic", "tie_storm"])
 @pytest.mark.parametrize("ms,spe,c_puct,eps", PARAMS)
 def test_protocol_equals_oracle_round_by_round(oracle, positions, evaluator, ms, spe, c_puct, eps):
     if evaluator == "synthetic":
         f = synthetic_evaluator(ms)
+    elif evaluator == "tie_storm":
+        f = tie_storm_eval
     else:
         f = network_evaluator(cb.fold_batchnorm(cb.random_weights(31)), evaluator)
     seed = 2000 + ms

@@ -8,7 +8,7 @@ import pytest
 
 import corintho_ai_b200 as cb
 from diag import first_divergence
-from oracle.pyoracle import synth_eval
+from oracle.pyoracle import ADVERSARIAL_EVALUATORS, synth_eval
 from test_oracle_trainer import check_against_golden
 from util import TRAINER_GRID, grid_key, run_trainer
 
@@ -62,6 +62,21 @@ def test_engine_matches_oracle(oracle, cfg):
     run_trainer(o, synth_eval, cfg[6])
     oc, ec = oracle.counters(o), e.counters()
     assert (oc["simulations"], oc["moves"], oc["leaf_evals"]) == (ec["simulations"], ec["moves"], ec["leaf_evals"])
+
+
+@pytest.mark.parametrize("evaluator", sorted(ADVERSARIAL_EVALUATORS))
+@pytest.mark.parametrize("cfg", [(24, 9, 100, 8, 1.0, 0.25, False), (8, 3, 300, 16, 1.0, 0.0, True)],
+                         ids=grid_key)
+def test_engine_matches_oracle_with_degenerate_evaluators(oracle, cfg, evaluator):
+    """Tie storms, all-zero legal probabilities and subnormal probabilities, in training and
+    testing mode: the PUCT tie-breaks, move choice and the NaN / inf prior paths."""
+    f = ADVERSARIAL_EVALUATORS[evaluator]
+    a = run_trainer(make_oracle(oracle, cfg), f, cfg[6])
+    b = run_trainer(make_engine(cfg), f, cfg[6])
+    assert a["rounds"] == b["rounds"] and (a["counts"] == b["counts"]).all()
+    assert a["req_hash"] == b["req_hash"]
+    assert a["score"].tobytes() == b["score"].tobytes() and a["mate"].tobytes() == b["mate"].tobytes()
+    assert cfg[6] or a["samples_hash"] == b["samples_hash"]
 
 
 def test_sharded_trainers_equal_single_trainer():

@@ -6,7 +6,7 @@ import os
 import numpy as np
 import pytest
 
-from oracle.pyoracle import synth_eval
+from oracle.pyoracle import ADVERSARIAL_EVALUATORS, synth_eval
 from util import TRAINER_GRID, grid_key, run_trainer
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -53,6 +53,21 @@ def test_oracle_matches_compiled_reference(oracle, ref, cfg):
     assert a["score"].tobytes() == b["score"].tobytes() and a["mate"].tobytes() == b["mate"].tobytes()
     if not cfg[6]:
         assert a["samples_hash"] == b["samples_hash"]
+
+
+@pytest.mark.parametrize("evaluator", sorted(ADVERSARIAL_EVALUATORS))
+@pytest.mark.parametrize("cfg", [(5, 4242, 48, 16, 1.0, 0.25, False), (6, 3, 32, 4, 1.0, 0.0, True)],
+                         ids=grid_key)
+def test_oracle_matches_compiled_reference_with_degenerate_evaluators(oracle, ref, cfg, evaluator):
+    """The same comparison under tie storms, all-zero and subnormal probabilities: the
+    reference's NaN max and x86 lround decide the priors there."""
+    f = ADVERSARIAL_EVALUATORS[evaluator]
+    a = run_trainer(make(ref, cfg), f, cfg[6])
+    b = run_trainer(make(oracle, cfg), f, cfg[6])
+    assert a["rounds"] == b["rounds"] and (a["counts"] == b["counts"]).all()
+    assert a["req_hash"] == b["req_hash"]
+    assert a["score"].tobytes() == b["score"].tobytes() and a["mate"].tobytes() == b["mate"].tobytes()
+    assert cfg[6] or a["samples_hash"] == b["samples_hash"]
 
 
 def test_max_searches_1_quirk(oracle):

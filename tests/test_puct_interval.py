@@ -1,20 +1,34 @@
 """Host check of the interval screening used by the game step's PUCT selection
 (corintho_ai_b200/csrc/tree.cuh, puct_bounds): for visited children the float expression
 -E*rcp(N) + pv*rcp(N+1) with a 1-ulp reciprocal must stay within 2^-20*(|a|+|b|) of the reference's
-float(double(-E/N) + double(pv/(N+1))) (trainmc.cpp:540-600). The reciprocal of the hardware
+float(-E/float(N) + pv/(float(N) + 1.0)) in double (trainmc.cpp:540-600). The reciprocal of the hardware
 (rcp.approx.f32, <= 1 ulp) is emulated by the correctly rounded one and both of its neighbours, so
 every value it may return is covered."""
 import numpy as np
 
 
-def test_interval_contains_reference_value():
+def samples():
+    """visits up to 2^20 and from 2^24 to 2^31 - 1 (where float(N) != N), evaluation sums of any sign
+    up to the visit count, small and large priors"""
     rng = np.random.default_rng(7)
     n = 400_000
-    # visits up to 2^20, evaluation sums of any sign up to the visit count, small and large priors
-    N = np.concatenate([rng.integers(1, 64, n // 2), rng.integers(1, 1 << 20, n // 2)]).astype(np.int64)
+    N = np.concatenate([rng.integers(1, 64, n // 2), rng.integers(1, 1 << 20, n // 2),
+                        rng.integers(1 << 24, 1 << 31, n // 2)]).astype(np.int64)
+    n = len(N)
     E = (rng.uniform(-1, 1, n) * N * rng.choice([1.0, 1e-3, 1e-7], n)).astype(np.float32)
     pv = (rng.uniform(0, 1, n) ** 3 * rng.choice([1.0, 40.0, 1e-4], n)).astype(np.float32)
-    ref = ((-E.astype(np.float64)) / N.astype(np.float64) + pv.astype(np.float64) / (N + 1).astype(np.float64)).astype(np.float32)
+    return N, E, pv
+
+
+def reference(N, E, pv):
+    """float(-E / float(N) + pv / (float(N) + 1.0)), quotients and sum in double"""
+    fn = N.astype(np.float32).astype(np.float64)
+    return ((-E.astype(np.float64)) / fn + pv.astype(np.float64) / (fn + 1.0)).astype(np.float32)
+
+
+def test_interval_contains_reference_value():
+    N, E, pv = samples()
+    ref = reference(N, E, pv)
     fn = N.astype(np.float32)
     fn1 = (fn + np.float32(1.0)).astype(np.float32)
     worst = 0.0
