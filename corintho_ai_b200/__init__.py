@@ -120,6 +120,7 @@ def lib():
         "cb200_analysis_results": (i32, [vp, vp, vp, vp, vp, vp]),
         "cb200_analysis_write_requests_device": (i32, [vp, vp]),
         "cb200_analysis_do_iteration_device": (i32, [vp, vp, vp, i32]),
+        "cb200_analysis_run_device": (i32, [vp, i32, vp, i32, vp, vp, vp, vp, vp, vp]),
         "cb200_check_states": (i64, [i64, vp, vp]),
     }
     for name, (res, args) in sig.items():
@@ -574,21 +575,26 @@ def _out_buf(a, dtype, min_size, what):
     return a
 
 
-def _dev_f32(t, min_size, what):
-    """Device buffer of the analysis' device forms: a contiguous float32 CUDA tensor with at least
-    `min_size` elements. Duck-typed on torch.Tensor's dtype / device / is_contiguous / numel /
-    data_ptr, so this package does not import torch. Returns the device address."""
+def _dev_buf(t, min_size, what, dtypes=("torch.float32",)):
+    """Device buffer of the analysis' device forms: a contiguous CUDA tensor of one of `dtypes` with
+    at least `min_size` elements. Duck-typed on torch.Tensor's dtype / device / is_contiguous /
+    numel / data_ptr, so this package does not import torch. Returns the device address."""
     try:
         dtype, device = str(t.dtype), t.device
         contiguous, numel = bool(t.is_contiguous()), int(t.numel())
     except (AttributeError, TypeError):
         raise Corintho200Error(f"{what}: need a CUDA tensor, got {type(t).__name__}") from None
-    if dtype != "torch.float32" or getattr(device, "type", None) != "cuda" or not contiguous:
-        raise Corintho200Error(f"{what}: need a contiguous float32 CUDA tensor, got {dtype} on {device}"
+    if dtype not in dtypes or getattr(device, "type", None) != "cuda" or not contiguous:
+        want = " or ".join(d.replace("torch.", "") for d in dtypes)
+        raise Corintho200Error(f"{what}: need a contiguous {want} CUDA tensor, got {dtype} on {device}"
                                f"{'' if contiguous else ' (not contiguous)'}")
     if numel < min_size:
         raise Corintho200Error(f"{what}: {numel} elements given, {min_size} needed")
     return int(t.data_ptr())
+
+
+def _dev_f32(t, min_size, what):
+    return _dev_buf(t, min_size, what)
 
 
 def check_states(states):
@@ -718,6 +724,49 @@ class Analysis:
         pr = _dev_f32(probs, n * NUM_MOVES, "do_iteration_device: probs")
         rows = min(int(eval.numel()), int(probs.numel()) // NUM_MOVES)
         return bool(_check(lib().cb200_analysis_do_iteration_device(self._h, ev, pr, rows)))
+
+    def run_device(self, states, seed=0, out=None, evals=True):
+        """run() on positions already on the GPU, in one persistent kernel on the library's current
+        stream (cb200_set_stream), returning without waiting: the outputs are complete in the order
+        of that stream, and `states` must not change before then. states: a contiguous int64 or
+        uint64 CUDA tensor [n, 2] of cstate words; needs bf16, fp16 or bf16x3 weights. out=None
+        allocates the outputs with torch on the states' device; else `out` is a dict of the caller's
+        CUDA tensors "moves" [n] int32, "results" [n] int32, "values" [n] float32, "visits" [n, 96]
+        int32 and optionally "evals" [n, 96] float32 and "status" [2] int32, written in place.
+        Returns the dict run() returns plus "status" = {positions with an error result, most
+        negative error result or 0}: a rejected state gets result -1, an overflowed search -3, both
+        with move -1. See cb200_analysis_run_device in include/corintho_b200.h."""
+        shape = tuple(getattr(states, "shape", ()))
+        if len(shape) != 2 or shape[1] != 2 or shape[0] < 1:
+            raise Corintho200Error("run_device: states must be an [n, 2] CUDA tensor of cstate words")
+        n = int(shape[0])
+        st = _dev_buf(states, 2 * n, "run_device: states", ("torch.int64", "torch.uint64"))
+        if out is None or "status" not in out:
+            import torch
+            dev = states.device
+            res = {"status": torch.zeros(2, dtype=torch.int32, device=dev)}
+            if out is None:
+                res.update(moves=torch.empty(n, dtype=torch.int32, device=dev),
+                           results=torch.empty(n, dtype=torch.int32, device=dev),
+                           values=torch.empty(n, dtype=torch.float32, device=dev),
+                           visits=torch.empty((n, NUM_MOVES), dtype=torch.int32, device=dev))
+                if evals:
+                    res["evals"] = torch.empty((n, NUM_MOVES), dtype=torch.float32, device=dev)
+            else:
+                res.update(out)
+        else:
+            res = dict(out)
+        if not evals:
+            res.pop("evals", None)
+        i32 = ("torch.int32",)
+        ptrs = [_dev_buf(res["moves"], n, "run_device: moves", i32),
+                _dev_buf(res["results"], n, "run_device: results", i32),
+                _dev_buf(res["values"], n, "run_device: values"),
+                _dev_buf(res["visits"], n * NUM_MOVES, "run_device: visits", i32),
+                _dev_buf(res["evals"], n * NUM_MOVES, "run_device: evals") if "evals" in res else None,
+                _dev_buf(res["status"], 2, "run_device: status", i32)]
+        _check(lib().cb200_analysis_run_device(self._h, n, st, int(seed), *ptrs))
+        return res
 
     def search(self, states, seed, evaluator, evals=True):
         """run() with the caller's network: evaluator(rows [k,70] float32) -> (eval [k], probs [k,96])

@@ -2198,23 +2198,8 @@ int cb200_tourney_counters(cb200_tourney *T, int64_t out[4]) {
 // in analysis.cuh. One "game" of the analysis' store per position, sized for max_positions when the
 // analysis is created; every run re-seeds and resets it.
 
-// The structural invariants of a cstate that the engine accepts from a caller (checked over the
-// reachable positions of 1 000 000 random play-outs by tests/test_oracle_analysis.py): side to move
-// 0 or 1, byte 7 zero, at most 4 pieces of a kind in a hand, frozen squares occupied, and every
-// piece of a kind either on the board or in a hand (8 of each kind).
-static bool valid_state(uint64_t w0, uint64_t w1) {
-  if (((w1 >> 48) & 0xff) > 1 || (w1 >> 56) != 0) return false;
-  const uint32_t base = (uint32_t)(w0 & 0xffff), column = (uint32_t)((w0 >> 16) & 0xffff);
-  const uint32_t capital = (uint32_t)((w0 >> 32) & 0xffff), frozen = (uint32_t)(w0 >> 48);
-  if (frozen & ~(base | column | capital)) return false;
-  const uint32_t plane[3] = {base, column, capital};
-  for (int t = 0; t < 3; ++t) {
-    const int h0 = (int)((w1 >> (8 * t)) & 0xff), h1 = (int)((w1 >> (8 * (3 + t))) & 0xff);
-    if (h0 > 4 || h1 > 4 || __builtin_popcount(plane[t]) != 8 - h0 - h1) return false;
-  }
-  return true;
-}
-
+// valid_state (analysis.cuh): the structural check of a caller's cstate, on the host and in
+// k_analysis_persistent.
 int64_t cb200_check_states(int64_t n, const uint64_t *states, uint8_t *valid) {
   if (n < 0 || (n > 0 && !states)) return set_error(CB200_ERR_ARG, "cb200_check_states: bad arguments");
   int64_t bad = 0;
@@ -2239,7 +2224,26 @@ struct cb200_analysis {
   enum { kNoSession, kOpen, kDone };
   int session = kNoSession;
   int requests = 0;
+  // device-resident runs (cb200_analysis_run_device, k_analysis_persistent): the CTA-private request
+  // and answer rows (SMs x 16 positions x spe rows, allocated by the first call), the work counters
+  // {next position, failed positions, min error}, and the event recorded after the last call, which
+  // the host-synchronous calls wait for
+  int dev_ctas = 0, dev_ld = 0;
+  float *d_dev_eval = nullptr, *d_dev_probs = nullptr;
+  ulonglong2 *d_dev_packed = nullptr;
+  int32_t *d_dev_ctr = nullptr;
+  cudaEvent_t dev_ev = nullptr;
+  bool dev_pending = false;   // dev_ev marks a call the host has not waited for
+  bool dev_counters = false;  // the counters are those of the last device-resident run
 };
+
+// Host-synchronous calls wait for the last cb200_analysis_run_device, on whatever stream it ran.
+static void analysis_wait_device(cb200_analysis *A) {
+  if (!A->dev_pending) return;
+  cudaSetDevice(A->s.device);
+  cudaEventSynchronize(A->dev_ev);
+  A->dev_pending = false;
+}
 
 // The checks of cb200_analysis_run and _begin: n in [1, max_positions], non-null states, every
 // state accepted by cb200_check_states.
@@ -2257,6 +2261,7 @@ static int analysis_check_states(const cb200_analysis *A, int n, const uint64_t 
 // zero request offsets and a zero summary behind
 static int analysis_start(cb200_analysis *A, int n, const uint64_t *states, int seed) {
   A->counters[0] = A->counters[1] = 0;
+  A->dev_counters = false;
   const int rc = store_reset(A->s, n, seed);
   if (rc != CB200_OK) return rc;
   CB_CUDA(cudaMemcpyAsync(A->d_roots, states, (size_t)n * sizeof(ulonglong2), cudaMemcpyHostToDevice, cur_stream()));
@@ -2326,7 +2331,10 @@ cb200_analysis *cb200_analysis_create(int max_positions, int max_searches, int s
 
 void cb200_analysis_destroy(cb200_analysis *A) {
   if (!A) return;
+  analysis_wait_device(A);
   cudaSetDevice(A->s.device);
+  cudaFree(A->d_dev_eval), cudaFree(A->d_dev_probs), cudaFree(A->d_dev_packed), cudaFree(A->d_dev_ctr);
+  if (A->dev_ev) cudaEventDestroy(A->dev_ev);
   cudaFree(A->d_roots), cudaFree(A->d_moves), cudaFree(A->d_results), cudaFree(A->d_values);
   cudaFree(A->d_visits), cudaFree(A->d_evals);
   net_free(A->net.net);
@@ -2338,7 +2346,9 @@ int cb200_analysis_set_weights(cb200_analysis *A, const float *weights, size_t n
   last_error_ref().clear();
   if (!A) return set_error(CB200_ERR_ARG, "null analysis");
   const int rc = check_weights(weights, n_floats, precision, "cb200_analysis_set_weights");
-  if (rc == CB200_OK) resident_net_set(A->net, weights, precision);
+  if (rc != CB200_OK) return rc;
+  analysis_wait_device(A);  // the next upload overwrites the weights a running call reads
+  resident_net_set(A->net, weights, precision);
   return rc;
 }
 
@@ -2346,6 +2356,7 @@ int cb200_analysis_run(cb200_analysis *A, int n, const uint64_t *states, int see
                        int32_t *results, float *values, int32_t *visits, float *evals) {
   last_error_ref().clear();
   if (!A) return set_error(CB200_ERR_ARG, "null analysis");
+  analysis_wait_device(A);
   A->session = cb200_analysis::kNoSession;  // a run discards an open session
   if (!moves || !results || !values || !visits)
     return set_error(CB200_ERR_ARG, "cb200_analysis_run: null states / moves / results / values / visits");
@@ -2396,6 +2407,7 @@ static int analysis_session(cb200_analysis *A, const char *who) {
 int cb200_analysis_begin(cb200_analysis *A, int n, const uint64_t *states, int seed) {
   last_error_ref().clear();
   if (!A) return set_error(CB200_ERR_ARG, "null analysis");
+  analysis_wait_device(A);
   A->session = cb200_analysis::kNoSession;  // a new begin discards an open session, even when it fails
   int rc = analysis_check_states(A, n, states, "cb200_analysis_begin");
   if (rc != CB200_OK) return rc;
@@ -2519,6 +2531,7 @@ int cb200_analysis_results(cb200_analysis *A, int32_t *moves, int32_t *results, 
   last_error_ref().clear();
   if (!A || !moves || !results || !values || !visits)
     return set_error(CB200_ERR_ARG, "cb200_analysis_results: null analysis / moves / results / values / visits");
+  analysis_wait_device(A);
   int rc = analysis_session(A, "cb200_analysis_results");
   if (rc != CB200_OK) return rc;
   if (A->session != cb200_analysis::kDone)
@@ -2529,7 +2542,8 @@ int cb200_analysis_results(cb200_analysis *A, int32_t *moves, int32_t *results, 
 int cb200_analysis_counters(cb200_analysis *A, int64_t out[2]) {
   last_error_ref().clear();
   if (!A || !out) return set_error(CB200_ERR_ARG, "null analysis / out");
-  if (A->session == cb200_analysis::kOpen) {  // the running totals of the session so far
+  analysis_wait_device(A);
+  if (A->session == cb200_analysis::kOpen || A->dev_counters) {  // a session's running totals, or a device run's
     int64_t c4[4];
     int rc = store_guard(A->s);
     if (rc == CB200_OK) rc = store_counters(A->s, c4);
@@ -2537,6 +2551,112 @@ int cb200_analysis_counters(cb200_analysis *A, int64_t out[2]) {
     A->counters[0] = c4[0], A->counters[1] = c4[2];
   }
   out[0] = A->counters[0], out[1] = A->counters[1];
+  return CB200_OK;
+}
+
+// ---- device-resident positions and outputs (cb200_analysis_run_device) -----------------------------
+
+// First call after create / set_weights: the weights, the CTA rows, the event (not capturable).
+static int analysis_device_prepare(cb200_analysis *A) {
+  int rc = CB200_OK;
+  if (A->net.net.precision < 0 && (rc = resident_net_upload(A->net)) != CB200_OK) return rc;
+  if (A->d_dev_ctr) return CB200_OK;
+  GameStore &s = A->s;
+  int sms = 148;
+  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, s.device);
+  const size_t rows = (size_t)sms * 16 * s.P.spe;
+  if (dmalloc(&A->d_dev_eval, rows) != CB200_OK || dmalloc(&A->d_dev_probs, rows * CB200_NUM_MOVES) != CB200_OK ||
+      dmalloc(&A->d_dev_packed, rows) != CB200_OK || dmalloc(&A->d_dev_ctr, 3) != CB200_OK ||
+      (!A->dev_ev && cudaEventCreateWithFlags(&A->dev_ev, cudaEventDisableTiming) != cudaSuccess)) {
+    cudaFree(A->d_dev_eval), cudaFree(A->d_dev_probs), cudaFree(A->d_dev_packed), cudaFree(A->d_dev_ctr);
+    A->d_dev_eval = A->d_dev_probs = nullptr, A->d_dev_packed = nullptr, A->d_dev_ctr = nullptr;
+    return last_error_ref().empty() ? set_error(CB200_ERR_CUDA, "allocation failed") : CB200_ERR_CUDA;
+  }
+  A->dev_ctas = sms, A->dev_ld = (int)rows;
+  return CB200_OK;
+}
+
+extern "C++" {
+// Device-side reset of positions [0, n) (store_reset's values, seeds from k_mt_outputs), then the
+// persistent analysis, one CTA per SM (at most one per position).
+template <int kMode, int kGames>
+static int analysis_device_launch(cb200_analysis *A, int n, const ulonglong2 *states, int seed, const AnalysisOut &out) {
+  GameStore &s = A->s;
+  static bool attr_set[16] = {false};
+  if (s.device < 16 && !attr_set[s.device]) {
+    CB_CUDA(cudaFuncSetAttribute(k_analysis_persistent<kMode, kGames>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                 (int)ps_smem_bytes<kMode, kGames>()));
+    attr_set[s.device] = true;
+  }
+  cudaStream_t st = cur_stream();
+  s.P.num_games = n;
+  s.iterations_done = 0;
+  const int grid = std::min(A->dev_ctas, n);
+  // the seeds travel through the request-offset buffer, as in store_reset
+  k_mt_outputs<<<1, kMtThreads, 0, st>>>((uint32_t)seed, n, (uint32_t *)s.d_offs);
+  CB_LAUNCHED();
+  k_seed_mt<<<(n + 127) / 128, 128, 0, st>>>(n, (const uint32_t *)s.d_offs, s.P.mt);
+  CB_LAUNCHED();
+  k_analysis_reset<<<(n + 127) / 128, 128, 0, st>>>(s.P, A->d_dev_ctr, grid * kGames);
+  CB_LAUNCHED();
+  CB_CUDA(cudaMemsetAsync(s.P.counters, 0, (size_t)n * 4 * sizeof(long long), st));
+  k_analysis_persistent<kMode, kGames><<<grid, kGames * 32, ps_smem_bytes<kMode, kGames>(), st>>>(
+      s.P, A->max_searches, (const uint8_t *)A->net.net.tc.w, states, A->d_dev_eval, A->d_dev_probs, A->dev_ld,
+      A->d_dev_packed, A->d_dev_ctr, out);
+  CB_LAUNCHED();
+  CB_CUDA(cudaGetLastError());
+  return CB200_OK;
+}
+}  // extern "C++"
+
+int cb200_analysis_run_device(cb200_analysis *A, int n, const void *states_device, int seed, void *moves_device,
+                              void *results_device, void *values_device, void *visits_device, void *evals_device,
+                              void *status_device) {
+  last_error_ref().clear();
+  const char *who = "cb200_analysis_run_device";
+  if (!A) return set_error(CB200_ERR_ARG, "null analysis");
+  A->session = cb200_analysis::kNoSession;  // a run discards an open session
+  if (n <= 0 || n > A->max_positions) return set_error(CB200_ERR_ARG, std::string(who) + ": n must be in [1, max_positions]");
+  if (!states_device || !moves_device || !results_device || !values_device || !visits_device)
+    return set_error(CB200_ERR_ARG, std::string(who) + ": null states / moves / results / values / visits");
+  if ((uintptr_t)states_device % 16 != 0)
+    return set_error(CB200_ERR_ARG, std::string(who) + ": states_device is not 16-byte aligned");
+  if (A->net.precision < 0) return set_error(CB200_ERR_STATE, std::string(who) + ": no weights set");
+  if (A->net.precision == 0)
+    return set_error(CB200_ERR_STATE, std::string(who) + ": needs tensor-core weights (bf16, fp16 or bf16x3); "
+                                                         "fp32 weights run with cb200_analysis_run");
+  GameStore &s = A->s;
+  int rc = store_guard(s);
+  if (rc != CB200_OK) return rc;
+  const void *bufs[7] = {states_device, moves_device, results_device, values_device, visits_device, evals_device,
+                         status_device};
+  const char *names[7] = {"states_device", "moves_device", "results_device", "values_device", "visits_device",
+                          "evals_device", "status_device"};
+  for (int i = 0; i < 7; ++i)
+    if (bufs[i] && (rc = check_device_buffer(s, bufs[i], who, names[i])) != CB200_OK) return rc;
+  if (A->net.net.precision < 0) analysis_wait_device(A);  // the upload overwrites the weights it reads
+  if ((rc = analysis_device_prepare(A)) != CB200_OK) return rc;
+  A->counters[0] = A->counters[1] = 0;
+  A->dev_counters = true;
+  const AnalysisOut out{(int32_t *)moves_device, (int32_t *)results_device, (float *)values_device,
+                        (int32_t *)visits_device, (float *)evals_device};
+  const ulonglong2 *states = (const ulonglong2 *)states_device;
+  const int mode = A->net.net.tc.mode;  // 0 bf16, 1 fp16, 2 bf16x3
+  rc = mode == 2 ? analysis_device_launch<2, 8>(A, n, states, seed, out)
+                 : mode == 1 ? analysis_device_launch<1, 16>(A, n, states, seed, out)
+                             : analysis_device_launch<0, 16>(A, n, states, seed, out);
+  if (rc != CB200_OK) return rc;
+  cudaStream_t st = cur_stream();
+  if (status_device)
+    CB_CUDA(cudaMemcpyAsync(status_device, A->d_dev_ctr + 1, 2 * sizeof(int32_t), cudaMemcpyDeviceToDevice, st));
+  // a call captured into a graph records nothing: its replays are ordered like any work of the
+  // caller's stream
+  cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
+  CB_CUDA(cudaStreamIsCapturing(st, &cs));
+  if (cs == cudaStreamCaptureStatusNone) {
+    CB_CUDA(cudaEventRecord(A->dev_ev, st));
+    A->dev_pending = true;
+  }
   return CB200_OK;
 }
 

@@ -349,8 +349,37 @@ int cb200_analysis_results(cb200_analysis *a, int32_t *moves /* [n] */, int32_t 
 int cb200_analysis_write_requests_device(cb200_analysis *a, void *rows_device);
 int cb200_analysis_do_iteration_device(cb200_analysis *a, const void *eval_device, const void *probs_device,
                                        int rows);
-/* out = {simulations, leaf evaluations} of the last run or session; while a session is open, its
- * running totals so far (like the oracle's counters). */
+/* cb200_analysis_run for positions and outputs in device memory, with the resident tensor-core
+ * network, in one persistent kernel: stream-ordered, no host round trip.
+ *   Outputs: for every valid position, bit for bit those of cb200_analysis_run on the same states,
+ *     seed, parameters and weights (moves, results, values, visits, evals; same seed rule).
+ *   Stream order: everything is enqueued on the library's current stream (cb200_set_stream) and the
+ *     call returns without waiting for the device. It makes no synchronisation, host copy,
+ *     allocation or read-back, so it may be captured in a CUDA graph -- except the first call after
+ *     create / set_weights, which uploads the weights and allocates its buffers (make one warm-up
+ *     call before capturing). The outputs are complete in the order of that stream. states_device is
+ *     read while the kernel runs: do not change it before then. Two calls on different streams must
+ *     be ordered by the caller. The host-synchronous calls on the object (run, begin, results,
+ *     counters, set_weights, destroy) first wait for the last uncaptured call; replays of a captured
+ *     one are ordered by the caller like any other work on their stream.
+ *   Per-position errors (the call cannot return them): a state cb200_check_states rejects gets
+ *     results[i] = CB200_ERR_ARG, moves[i] = -1 and zero value, visits and evals; a search that
+ *     overflows its node arena gets results[i] = CB200_ERR_OVERFLOW, moves[i] = -1 and the same zeros.
+ *     The other positions are searched as usual. status_device (may be NULL) receives
+ *     {positions with an error result, most negative error result or 0}.
+ *   Call errors, checked before anything is enqueued (the object stays usable): CB200_ERR_ARG for n
+ *     outside [1, max_positions], a null required pointer, a buffer that is not device (or managed)
+ *     memory of the analysis' device, or states_device not 16-byte aligned; CB200_ERR_STATE without
+ *     weights or with fp32 weights (precision 0: use cb200_analysis_run); CB200_ERR_CUDA without a
+ *     usable device. Like cb200_analysis_run, the call discards an open protocol session.
+ *   cb200_analysis_counters afterwards returns this call's totals (equal to cb200_analysis_run's). */
+int cb200_analysis_run_device(cb200_analysis *a, int n, const void *states_device /* u64 [n][2] */, int seed,
+                              void *moves_device /* i32 [n] */, void *results_device /* i32 [n] */,
+                              void *values_device /* f32 [n] */, void *visits_device /* i32 [n][96] */,
+                              void *evals_device /* f32 [n][96] or NULL */,
+                              void *status_device /* i32 [2] or NULL */);
+/* out = {simulations, leaf evaluations} of the last run, device run or session; while a session is
+ * open, its running totals so far (like the oracle's counters). */
 int cb200_analysis_counters(cb200_analysis *a, int64_t out[2]);
 /* Structural check of cstates given by a caller (no device needed): byte 6 (side to move) 0 or 1,
  * byte 7 zero, at most 4 pieces of a kind in either hand, frozen squares occupied, and for every

@@ -143,6 +143,14 @@ class Analysis {
            int32_t *visits, float *evals = nullptr) {
     check(cb200_analysis_run(h_, n, states, seed, moves, results, values, visits, evals));
   }
+  /* run() on device buffers in one persistent kernel, enqueued on the library's current stream
+   * without waiting (cb200_analysis_run_device: per-position error results, graph capture). */
+  void runDevice(int n, const void *states_device, int seed, void *moves_device, void *results_device,
+                 void *values_device, void *visits_device, void *evals_device = nullptr,
+                 void *status_device = nullptr) {
+    check(cb200_analysis_run_device(h_, n, states_device, seed, moves_device, results_device, values_device,
+                                    visits_device, evals_device, status_device));
+  }
 
   /* External-evaluator protocol (cb200_analysis_begin .. _results): the caller's network answers
    * the requests between rounds, as docker/choose_move.pyx does for DockerMC. */
