@@ -89,20 +89,8 @@ __device__ __forceinline__ bool analysis_step(const TreeParams &P, int max_searc
   const ulonglong2 rv = roots[g];
   const CState root{rv.x, rv.y};
   Ctx c;
-  c.to_play = (int)((root.w1 >> 48) & 0xffu), c.parity = 0, c.result = ctl[CW_RESULT];
-  c.mate_turn = 0, c.n_samples = 0;
-  c.n_pending = ctl[CW_N_PENDING], c.error = ctl[CW_ERROR], c.spare = ctl[CW_SPARE];
-  c.mt_idx = ctl[CW_MT_IDX];
-  c.d_sims = 0, c.d_evals = 0, c.d_moves = 0, c.d_searches = 0;
-  CB_PROF(c.t_ingest = c.t_search = c.t_move = c.n_none = c.n_copy = 0;
-          c.t_sel = c.t_exp = c.n_lvl = c.n_exp = c.n_exact = 0;)
-  c.work = 0, c.yielded = 0;
-  c.arenas = P.arenas + (size_t)g * 3 * P.arena_words;
-  c.mt = P.mt + (size_t)g * 624;
-  c.pending = P.pending + (size_t)g * P.spe * kPendWords;
-  c.tree_ctl = P.tree + (size_t)g * 2 * kTreeCtlWords;
-  c.leaf_state = P.leaf_state + (size_t)g * P.spe;
-  c.sample_state = nullptr, c.sample_probs = nullptr;
+  ctx_open(c, P, g, ctl, false);
+  c.to_play = (int)((root.w1 >> 48) & 0xffu), c.result = kResultNone;  // a position, not a game
   TreeParams Pm = P;
   Pm.testing = 1, Pm.yield_budget = 0, Pm.max_searches = max_searches;
   load_tree(c, Pm, c.to_play);
@@ -130,8 +118,7 @@ __device__ __forceinline__ bool analysis_step(const TreeParams &P, int max_searc
   if (c.error) done = true;
   store_tree(c);
   if (c.lane == 0) {
-    ctl[CW_TO_PLAY] = c.to_play, ctl[CW_N_PENDING] = c.n_pending, ctl[CW_ERROR] = c.error;
-    ctl[CW_SPARE] = c.spare, ctl[CW_MT_IDX] = c.mt_idx;
+    ctx_close(c, ctl, false);
     if (done) ctl[CW_DONE] = 1;
     long long *cnt = P.counters + (size_t)g * 4;
     cnt[0] += c.d_sims, cnt[1] += c.d_moves, cnt[2] += c.d_evals, cnt[3] += c.d_searches;
@@ -168,90 +155,25 @@ __device__ __forceinline__ void write_failed(int lane, int g, const AnalysisOut 
   if (lane == 0) out.moves[g] = -1, out.results[g] = code, out.values[g] = 0.0f;
 }
 
-// The first n outputs of std::mt19937(seed) (the per-position seeds of store_reset) by one CTA of
-// kMtThreads threads. The state is seeded by one thread (the recurrence is sequential); every block
-// twist runs in the phases of its in-place dependencies -- words [0, 227) read old words only,
-// [227, 454) and [454, 623) read words the previous phase wrote, word 623 reads the new words 0 and
-// 396 -- each phase reading into registers before a barrier and writing after it.
-constexpr int kMtThreads = 256;  // >= 227, the longest phase
-__global__ void __launch_bounds__(kMtThreads) k_mt_outputs(uint32_t seed, int n, uint32_t *__restrict__ out) {
-  __shared__ uint32_t mt[624];
-  const int t = threadIdx.x;
-  if (t == 0) {
-    uint32_t prev = seed;
-    mt[0] = prev;
-    for (int i = 1; i < 624; ++i) {
-      prev = 1812433253u * (prev ^ (prev >> 30)) + (uint32_t)i;
-      mt[i] = prev;
-    }
-  }
-  __syncthreads();
-  constexpr int kPhase[5] = {0, 227, 454, 623, 624};
-  for (int b0 = 0; b0 < n; b0 += 624) {
-#pragma unroll
-    for (int ph = 0; ph < 4; ++ph) {
-      const int i = kPhase[ph] + t;  // a phase has at most 227 words: one per thread
-      const bool mine = i < kPhase[ph + 1];
-      uint32_t v = 0;
-      if (mine) {
-        const uint32_t y = (mt[i] & 0x80000000u) | (mt[(i + 1) % 624] & 0x7fffffffu);
-        v = mt[(i + 397) % 624] ^ (y >> 1) ^ ((y & 1) ? 0x9908b0dfu : 0u);
-      }
-      __syncthreads();
-      if (mine) mt[i] = v;
-      __syncthreads();
-    }
-    for (int i = t; i < 624 && b0 + i < n; i += kMtThreads) {
-      uint32_t y = mt[i];
-      y ^= y >> 11;
-      y ^= (y << 7) & 0x9d2c5680u;
-      y ^= (y << 15) & 0xefc60000u;
-      y ^= y >> 18;
-      out[b0 + i] = y;
-    }
-  }
-}
-
-// The control and tree blocks store_reset writes, for positions [0, P.num_games) (first_game 0),
-// and the work counter of k_analysis_persistent: ctr = {next position, failed positions, min error}.
-__global__ void k_analysis_reset(TreeParams P, int32_t *__restrict__ ctr, int next0) {
-  const int g = blockIdx.x * blockDim.x + threadIdx.x;
-  if (g == 0) ctr[0] = next0, ctr[1] = 0, ctr[2] = 0;
-  if (g >= P.num_games) return;
-  int32_t *c = P.ctl + (size_t)g * kCtlWords;
-  for (int w = 0; w < kCtlWords; ++w) c[w] = 0;
-  c[CW_PARITY] = g & 1;
-  c[CW_SPARE] = 2;
-  c[CW_MT_IDX] = 624;
-  for (int p = 0; p < 2; ++p) {
-    int32_t *tw = P.tree + ((size_t)g * 2 + p) * kTreeCtlWords;
-    for (int w = 0; w < kTreeCtlWords; ++w) tw[w] = 0;
-    tw[TW_ARENA] = p;
-    tw[TW_ROOT_VISITS] = 1;
-    tw[TW_ROOT_ALLV] = 1;
-  }
-}
-
 // Analysis in one persistent launch: one CTA per SM holds kGames positions, one warp each (16 with
 // bf16 / fp16 operands, 512 threads, the network on the first 256; 8 with bf16x3, 256 threads, one
 // network tile on the first 128). A round is analysis_step of every warp's position, its requests
 // appended to the CTA's rows [row0, row0 + kGames * spe) with one shared atomicAdd per position,
 // then tc_forward over those rows, whose answers (move-major, leading dimension ld) the next round
 // reads. The first wave is dealt round-robin (slot = warp * grid + block) so that a small batch
-// spreads over every SM; a warp whose position finishes takes the next one from ctr[0] in the same
-// round, and the CTA leaves once no warp holds a live position. A position's first round checks its
-// state (valid_state); rejected ones and searches that fail get write_failed, counted in ctr[1], the
-// most negative code in ctr[2]. A position's order of operations is k_analysis_iterate's, and a
-// network row does not depend on the other rows of its batch: the outputs are cb200_analysis_run's.
+// spreads over every SM; a warp whose position finishes takes the next one in the same round
+// (ctr[0] counts the draws after the first wave), and the CTA leaves once no warp holds a live
+// position. A position's first round checks its state (valid_state); rejected ones and searches that
+// fail get write_failed, counted in ctr[1], the most negative code in ctr[2]; ctr starts at zero. A
+// position's order of operations is k_analysis_iterate's, and a network row does not depend on the
+// other rows of its batch: the outputs are cb200_analysis_run's.
 template <int kMode, int kGames>
 __global__ void __launch_bounds__(kGames * 32, 1)
     k_analysis_persistent(TreeParams P, int max_searches, const uint8_t *__restrict__ W,
                           const ulonglong2 *__restrict__ states, float *eval, float *probs, int ld,
                           ulonglong2 *packed, int32_t *ctr, AnalysisOut out) {
-  static_assert(kGames == 8 || kGames == 16, "one or two network tiles per CTA");
-  static_assert(ps_smem_bytes<kMode, kGames>() <= 227 * 1024, "bf16x3 fits with 8 games per CTA only");
-  constexpr int kNetThreads = kGames == 8 ? 128 : kTcThreads;  // one tile or two
-  constexpr int kTileRows = kNetThreads;                        // rows per tc_forward call
+  constexpr int kNetThreads = ps_net_threads<kGames>();
+  constexpr int kTileRows = kNetThreads;  // rows per tc_forward call
   const bool net_thread = threadIdx.x < kNetThreads;
   extern __shared__ __align__(128) uint8_t smem[];
   __shared__ int32_t s_ctr[2];  // requests of this round, live positions
@@ -299,7 +221,7 @@ __global__ void __launch_bounds__(kGames * 32, 1)
         if (lane == 0) atomicAdd(ctr + 1, 1), atomicMin(ctr + 2, error);
       }
       int next = 0;
-      if (lane == 0) next = atomicAdd(ctr, 1);
+      if (lane == 0) next = atomicAdd(ctr, 1) + gridDim.x * kGames;  // past the first wave
       next = __shfl_sync(0xffffffffu, next, 0);
       g = next < n ? next : -1;
       fresh = true;

@@ -234,33 +234,6 @@ namespace {
 
 constexpr size_t kAnswerSlack = 128;  // spare rows behind the answer buffers
 
-uint32_t mt_seed_word(uint32_t prev, int i) { return 1812433253u * (prev ^ (prev >> 30)) + i; }
-
-struct HostMT {
-  uint32_t mt[624];
-  int idx = 624;
-  void seed(uint32_t s) {
-    mt[0] = s;
-    for (int i = 1; i < 624; ++i) mt[i] = mt_seed_word(mt[i - 1], i);
-    idx = 624;
-  }
-  uint32_t next() {
-    if (idx >= 624) {
-      for (int i = 0; i < 624; ++i) {
-        uint32_t y = (mt[i] & 0x80000000u) | (mt[(i + 1) % 624] & 0x7fffffffu);
-        mt[i] = mt[(i + 397) % 624] ^ (y >> 1) ^ ((y & 1) ? 0x9908b0dfu : 0u);
-      }
-      idx = 0;
-    }
-    uint32_t y = mt[idx++];
-    y ^= y >> 11;
-    y ^= (y << 7) & 0x9d2c5680u;
-    y ^= (y << 15) & 0xefc60000u;
-    y ^= y >> 18;
-    return y;
-  }
-};
-
 int upload_tables_once() {
   int rc = ensure_tables();
   if (rc != CB200_OK) return rc;
@@ -278,6 +251,23 @@ int upload_tables_once() {
 template <class T>
 int dmalloc(T **p, size_t count) {
   CB_CUDA(cudaMalloc((void **)p, count * sizeof(T)));
+  return CB200_OK;
+}
+
+// SMs of a device: the persistent kernels run one CTA on each
+int sm_count(int device) {
+  int sms = 148;
+  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
+  return sms;
+}
+
+// Lets kKernel launch with `bytes` of dynamic shared memory on a device (set once per device)
+template <auto kKernel>
+int allow_smem_once(int device, size_t bytes) {
+  static bool set[16] = {false};
+  if (device < 16 && set[device]) return CB200_OK;
+  CB_CUDA(cudaFuncSetAttribute(kKernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
+  if (device < 16) set[device] = true;
   return CB200_OK;
 }
 
@@ -581,16 +571,70 @@ static int store_drain_logs(GameStore &s) {
   return CB200_OK;
 }
 
-// std::mt19937(seed) state expansion (one thread per game; the recurrence is sequential)
-__global__ void k_seed_mt(int n, const uint32_t *__restrict__ seeds, uint32_t *__restrict__ mt) {
-  const int g = blockIdx.x * blockDim.x + threadIdx.x;
-  if (g >= n) return;
-  uint32_t *m = mt + (size_t)g * 624;
-  uint32_t prev = seeds[g];
+// std::mt19937's state expansion of seed into m[0 .. 624) (the recurrence is sequential)
+__device__ __forceinline__ void mt_seed(uint32_t *m, uint32_t seed) {
+  uint32_t prev = seed;
   m[0] = prev;
   for (int i = 1; i < 624; ++i) {
     prev = 1812433253u * (prev ^ (prev >> 30)) + (uint32_t)i;
     m[i] = prev;
+  }
+}
+
+// MT19937 states of games [0, n) from their seeds, one thread per game
+__global__ void k_seed_mt(int n, const uint32_t *__restrict__ seeds, uint32_t *__restrict__ mt) {
+  const int g = blockIdx.x * blockDim.x + threadIdx.x;
+  if (g >= n) return;
+  mt_seed(mt + (size_t)g * 624, seeds[g]);
+}
+
+// Outputs skip, skip + 1, ..., skip + n - 1 of std::mt19937(seed) (the per-game seeds of a store) by
+// one CTA of kMtThreads threads. The state is seeded by one thread; every block twist runs in the
+// phases of its in-place dependencies -- words [0, 227) read old words only, [227, 454) and
+// [454, 623) read words the previous phase wrote, word 623 reads the new words 0 and 396 -- each
+// phase reading into registers before a barrier and writing after it.
+constexpr int kMtThreads = 256;  // >= 227, the longest phase
+__global__ void __launch_bounds__(kMtThreads)
+    k_mt_outputs(uint32_t seed, int skip, int n, uint32_t *__restrict__ out) {
+  __shared__ uint32_t mt[624];
+  const int t = threadIdx.x;
+  if (t == 0) mt_seed(mt, seed);
+  __syncthreads();
+  constexpr int kPhase[5] = {0, 227, 454, 623, 624};
+  for (int b0 = 0; b0 < skip + n; b0 += 624) {
+#pragma unroll
+    for (int ph = 0; ph < 4; ++ph) {
+      const int i = kPhase[ph] + t;  // a phase has at most 227 words: one per thread
+      const bool mine = i < kPhase[ph + 1];
+      const uint32_t v = mine ? mt_next_word(mt, i) : 0u;
+      __syncthreads();
+      if (mine) mt[i] = v;
+      __syncthreads();
+    }
+    for (int i = t; i < 624; i += kMtThreads) {
+      const int k = b0 + i - skip;
+      if (k >= 0 && k < n) out[k] = mt_temper(mt[i]);
+    }
+  }
+}
+
+// The one layout of a fresh game: control block and both trees of games [0, P.num_games), all zero
+// but the parity of the global game index, 2 spare moves, an MT19937 ring that twists at its first
+// draw, tree p in arena p, and roots of 1 visit that count as all visited.
+__global__ void k_store_reset(TreeParams P) {
+  const int g = blockIdx.x * blockDim.x + threadIdx.x;
+  if (g >= P.num_games) return;
+  int32_t *c = P.ctl + (size_t)g * kCtlWords;
+  for (int w = 0; w < kCtlWords; ++w) c[w] = 0;
+  c[CW_PARITY] = (P.first_game + g) & 1;
+  c[CW_SPARE] = 2;
+  c[CW_MT_IDX] = 624;
+  for (int p = 0; p < 2; ++p) {
+    int32_t *tw = P.tree + ((size_t)g * 2 + p) * kTreeCtlWords;
+    for (int w = 0; w < kTreeCtlWords; ++w) tw[w] = 0;
+    tw[TW_ARENA] = p;
+    tw[TW_ROOT_VISITS] = 1;
+    tw[TW_ROOT_ALLV] = 1;
   }
 }
 
@@ -676,40 +720,36 @@ static int store_create(GameStore &s, int num_games, int max_searches, int spe, 
   return CB200_OK;
 }
 
-// Games [0, n) start afresh: per-game seeds (trainer.cpp:238-256) = the outputs first_game,
-// first_game + 1, ... of mt19937(seed), MT19937 states expanded on the device, fresh control blocks
-// and trees, zero counters, request offsets, summary and answers, and the text logs started again.
-static int store_reset(GameStore &s, int n, int seed) {
+// Games [0, n) start afresh, on the current stream and nothing else (no host copy, synchronisation
+// or allocation, so that a graph can capture it): per-game seeds (trainer.cpp:238-256) = the outputs
+// first_game, first_game + 1, ... of mt19937(seed), the MT19937 states expanded from them, fresh
+// control blocks and trees, zero counters. The seeds travel through the (still unused) request-offset
+// buffer.
+static int store_reset_enqueue(GameStore &s, int n, int seed) {
   TreeParams &P = s.P;
   P.num_games = n;
-  const size_t Gn = (size_t)n;
-  std::vector<int32_t> ctl(Gn * kCtlWords, 0), tree(Gn * 2 * kTreeCtlWords, 0);
-  std::vector<uint32_t> seeds(Gn);
-  HostMT gen;
-  gen.seed((uint32_t)seed);
-  for (int i = 0; i < P.first_game; ++i) gen.next();
-  for (size_t g = 0; g < Gn; ++g) {
-    seeds[g] = gen.next();
-    int32_t *c = ctl.data() + g * kCtlWords;
-    c[CW_PARITY] = (int)((P.first_game + g) & 1);
-    c[CW_SPARE] = 2;
-    c[CW_MT_IDX] = 624;
-    for (int p = 0; p < 2; ++p) {
-      int32_t *tw = tree.data() + (g * 2 + p) * kTreeCtlWords;
-      tw[TW_ARENA] = p;
-      tw[TW_ROOT_VISITS] = 1;
-      tw[TW_ROOT_ALLV] = 1;
-    }
-  }
+  s.iterations_done = 0;
   cudaStream_t st = cur_stream();
-  CB_CUDA(cudaMemcpyAsync(P.ctl, ctl.data(), ctl.size() * 4, cudaMemcpyHostToDevice, st));
-  CB_CUDA(cudaMemcpyAsync(P.tree, tree.data(), tree.size() * 4, cudaMemcpyHostToDevice, st));
-  // the seeds travel through the (still unused) request-offset buffer
-  CB_CUDA(cudaMemcpyAsync(s.d_offs, seeds.data(), Gn * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
-  k_seed_mt<<<(int)((Gn + 127) / 128), 128, 0, st>>>((int)Gn, (const uint32_t *)s.d_offs, P.mt);
+  const int grid = (n + 127) / 128;
+  k_mt_outputs<<<1, kMtThreads, 0, st>>>((uint32_t)seed, P.first_game, n, (uint32_t *)s.d_offs);
+  CB_LAUNCHED();
+  k_seed_mt<<<grid, 128, 0, st>>>(n, (const uint32_t *)s.d_offs, P.mt);
+  CB_LAUNCHED();
+  k_store_reset<<<grid, 128, 0, st>>>(P);
   CB_LAUNCHED();
   CB_CUDA(cudaGetLastError());
-  CB_CUDA(cudaMemsetAsync(P.counters, 0, Gn * 4 * sizeof(long long), st));
+  CB_CUDA(cudaMemsetAsync(P.counters, 0, (size_t)n * 4 * sizeof(long long), st));
+  return CB200_OK;
+}
+
+// store_reset_enqueue, then zero request offsets, summary and answers, and the text logs started
+// again; returns once the device is done.
+static int store_reset(GameStore &s, int n, int seed) {
+  const int rc = store_reset_enqueue(s, n, seed);
+  if (rc != CB200_OK) return rc;
+  TreeParams &P = s.P;
+  const size_t Gn = (size_t)n;
+  cudaStream_t st = cur_stream();
   CB_CUDA(cudaMemsetAsync(s.d_offs, 0, Gn * sizeof(int32_t), st));
   CB_CUDA(cudaMemsetAsync(s.d_summary, 0, 4 * sizeof(int32_t), st));
   // The whole answer buffers, slack rows included: a fused two-model tourney reads rows that no
@@ -732,7 +772,6 @@ static int store_reset(GameStore &s, int n, int seed) {
       s.log_files.push_back(std::move(f));
     }
   }
-  s.iterations_done = 0;
   return CB200_OK;
 }
 
@@ -895,11 +934,7 @@ cb200_trainer *cb200_trainer_create_shard(int total_games, int first_game, int n
   if (const char *env = getenv("CB200_YIELD_MIN_LIVE")) t->sched.yield_min_live = atoi(env);
   if (const char *env = getenv("CB200_PS_CAPACITY")) t->sched.ps_capacity = atoll(env);
   t->sched.persistent = getenv("CB200_NO_PERSISTENT") == nullptr;
-  {
-    int sms = 148;
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, t->device);
-    t->ps_ctas = sms;
-  }
+  t->ps_ctas = sm_count(t->device);
   t->ps_ld = t->ps_ctas * 16 * kPsRowsPerGame * 2;  // x2: two row regions in two-model runs
   const size_t ps_rows = (size_t)t->ps_ld;
   if (dmalloc(&t->d_gctr, (size_t)t->n_groups * 8) != CB200_OK ||
@@ -1500,7 +1535,7 @@ static int ps_takeover(const cb200_trainer *t) {
 // buffer the previous launch (or the lock-step loop) wrote, and writes its own into the other.
 static int ps_list_games(cb200_trainer *t) {
   cudaStream_t st = t->g_stream[0];
-  k_live_list<<<1, 32, 0, st>>>(t->P, t->d_ps_list, t->d_ps_out + 4);
+  k_group_live_list<<<1, 32, 0, st>>>(t->P, t->d_ps_list, t->d_ps_out + 4);  // every game of the trainer
   CB_LAUNCHED();
   CB_CUDA(cudaGetLastError());
   CB_CUDA(cudaMemcpyAsync(t->h_ps_out + 4, t->d_ps_out + 4, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
@@ -1512,13 +1547,8 @@ static int ps_list_games(cb200_trainer *t) {
 extern "C++" {
 template <int kMode, int kGames>
 static int ps_launch(cb200_trainer *t, const TreeParams &P, int rounds, int exit_done) {
-  static bool attr_set[16] = {false};
-  if (t->device < 16 && !attr_set[t->device]) {
-    CB_CUDA(cudaFuncSetAttribute(k_selfplay_persistent<kMode, kGames>,
-                                 cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                 (int)ps_smem_bytes<kMode, kGames>()));
-    attr_set[t->device] = true;
-  }
+  int rc = allow_smem_once<k_selfplay_persistent<kMode, kGames>>(t->device, ps_smem_bytes<kMode, kGames>());
+  if (rc != CB200_OK) return rc;
   const float *ev0 = t->ps_from_lockstep ? t->d_eval : t->d_ps_eval[t->ps_cur];
   const float *pr0 = t->ps_from_lockstep ? t->d_probs : t->d_ps_probs[t->ps_cur];
   const long pcs0 = t->ps_from_lockstep ? (long)t->cap : (long)t->ps_ld;
@@ -2562,8 +2592,7 @@ static int analysis_device_prepare(cb200_analysis *A) {
   if (A->net.net.precision < 0 && (rc = resident_net_upload(A->net)) != CB200_OK) return rc;
   if (A->d_dev_ctr) return CB200_OK;
   GameStore &s = A->s;
-  int sms = 148;
-  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, s.device);
+  const int sms = sm_count(s.device);
   const size_t rows = (size_t)sms * 16 * s.P.spe;
   if (dmalloc(&A->d_dev_eval, rows) != CB200_OK || dmalloc(&A->d_dev_probs, rows * CB200_NUM_MOVES) != CB200_OK ||
       dmalloc(&A->d_dev_packed, rows) != CB200_OK || dmalloc(&A->d_dev_ctr, 3) != CB200_OK ||
@@ -2577,29 +2606,16 @@ static int analysis_device_prepare(cb200_analysis *A) {
 }
 
 extern "C++" {
-// Device-side reset of positions [0, n) (store_reset's values, seeds from k_mt_outputs), then the
-// persistent analysis, one CTA per SM (at most one per position).
+// Device-side reset of positions [0, n), then the persistent analysis, one CTA per SM (at most one
+// per position).
 template <int kMode, int kGames>
 static int analysis_device_launch(cb200_analysis *A, int n, const ulonglong2 *states, int seed, const AnalysisOut &out) {
   GameStore &s = A->s;
-  static bool attr_set[16] = {false};
-  if (s.device < 16 && !attr_set[s.device]) {
-    CB_CUDA(cudaFuncSetAttribute(k_analysis_persistent<kMode, kGames>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                 (int)ps_smem_bytes<kMode, kGames>()));
-    attr_set[s.device] = true;
-  }
+  int rc = allow_smem_once<k_analysis_persistent<kMode, kGames>>(s.device, ps_smem_bytes<kMode, kGames>());
+  if (rc != CB200_OK || (rc = store_reset_enqueue(s, n, seed)) != CB200_OK) return rc;
   cudaStream_t st = cur_stream();
-  s.P.num_games = n;
-  s.iterations_done = 0;
+  CB_CUDA(cudaMemsetAsync(A->d_dev_ctr, 0, 3 * sizeof(int32_t), st));
   const int grid = std::min(A->dev_ctas, n);
-  // the seeds travel through the request-offset buffer, as in store_reset
-  k_mt_outputs<<<1, kMtThreads, 0, st>>>((uint32_t)seed, n, (uint32_t *)s.d_offs);
-  CB_LAUNCHED();
-  k_seed_mt<<<(n + 127) / 128, 128, 0, st>>>(n, (const uint32_t *)s.d_offs, s.P.mt);
-  CB_LAUNCHED();
-  k_analysis_reset<<<(n + 127) / 128, 128, 0, st>>>(s.P, A->d_dev_ctr, grid * kGames);
-  CB_LAUNCHED();
-  CB_CUDA(cudaMemsetAsync(s.P.counters, 0, (size_t)n * 4 * sizeof(long long), st));
   k_analysis_persistent<kMode, kGames><<<grid, kGames * 32, ps_smem_bytes<kMode, kGames>(), st>>>(
       s.P, A->max_searches, (const uint8_t *)A->net.net.tc.w, states, A->d_dev_eval, A->d_dev_probs, A->dev_ld,
       A->d_dev_packed, A->d_dev_ctr, out);

@@ -67,20 +67,7 @@ __global__ void __launch_bounds__(kTreeWarps * 32, 4)
   if (!match_selected(ctl, sides, model_id)) return;
   WarpSm &sm = sm_all[warp];
   Ctx c;
-  c.to_play = ctl[CW_TO_PLAY], c.parity = 0, c.result = ctl[CW_RESULT];
-  c.mate_turn = 0, c.n_samples = 0;
-  c.n_pending = ctl[CW_N_PENDING], c.error = ctl[CW_ERROR], c.spare = ctl[CW_SPARE];
-  c.mt_idx = ctl[CW_MT_IDX];
-  c.d_sims = 0, c.d_evals = 0, c.d_moves = 0, c.d_searches = 0;
-  CB_PROF(c.t_ingest = c.t_search = c.t_move = c.n_none = c.n_copy = 0;
-          c.t_sel = c.t_exp = c.n_lvl = c.n_exp = c.n_exact = 0;)
-  c.work = 0, c.yielded = 0;
-  c.arenas = P.arenas + (size_t)g * 3 * P.arena_words;
-  c.mt = P.mt + (size_t)g * 624;
-  c.pending = P.pending + (size_t)g * P.spe * kPendWords;  // P.spe = largest budget (stride)
-  c.tree_ctl = P.tree + (size_t)g * 2 * kTreeCtlWords;
-  c.leaf_state = P.leaf_state + (size_t)g * P.spe;
-  c.sample_state = nullptr, c.sample_probs = nullptr;
+  ctx_open(c, P, g, ctl, false);
   CState root;
   root.w0 = (uint64_t)(uint32_t)ctl[MW_ROOT0] | ((uint64_t)(uint32_t)ctl[MW_ROOT1] << 32);
   root.w1 = (uint64_t)(uint32_t)ctl[MW_ROOT2] | ((uint64_t)(uint32_t)ctl[MW_ROOT3] << 32);
@@ -179,9 +166,7 @@ __global__ void __launch_bounds__(kTreeWarps * 32, 4)
   if (c.error) done = true;
   if (!is_random) store_tree(c);
   if (c.lane == 0) {
-    ctl[CW_TO_PLAY] = c.to_play, ctl[CW_RESULT] = c.result;
-    ctl[CW_N_PENDING] = c.n_pending, ctl[CW_ERROR] = c.error;
-    ctl[CW_SPARE] = c.spare, ctl[CW_MT_IDX] = c.mt_idx;
+    ctx_close(c, ctl, false);
     ctl[MW_ROOT0] = (int32_t)(uint32_t)root.w0, ctl[MW_ROOT1] = (int32_t)(uint32_t)(root.w0 >> 32);
     ctl[MW_ROOT2] = (int32_t)(uint32_t)root.w1, ctl[MW_ROOT3] = (int32_t)(uint32_t)(root.w1 >> 32);
     ctl[MW_DEPTH] = depth;
@@ -258,22 +243,12 @@ __global__ void __launch_bounds__(256)
                  const int32_t *__restrict__ pack_offs, float *__restrict__ rows,
                  ulonglong2 *__restrict__ packed) {
   const int g = blockIdx.x * 8 + (threadIdx.x >> 5);
-  const int lane = threadIdx.x & 31;
   if (g >= P.num_games) return;
   const int32_t *ctl = P.ctl + (size_t)g * kCtlWords;
   const MatchSide *sides = sides_all + 2 * (size_t)g;
   if (!match_selected(ctl, sides, model_id)) return;
-  const int np = match_requests(ctl, sides);
-  const ulonglong2 *ls = P.leaf_state + (size_t)g * P.spe;
-  if (packed)  // fused tourney: leaf cstates in request order for the device-resident network
-    for (int k = lane; k < np; k += 32) packed[(size_t)pack_offs[g] + k] = ls[k];
-  if (!rows) return;
-  float *out = rows + (size_t)pack_offs[g] * CB200_STATE_SIZE;
-  for (int f = lane; f < np * CB200_STATE_SIZE; f += 32) {
-    const int k = f / CB200_STATE_SIZE, j = f - k * CB200_STATE_SIZE;
-    const ulonglong2 v = ls[k];
-    out[f] = encode_elem(CState{v.x, v.y}, j);
-  }
+  // packed: a fused tourney's leaf cstates in request order for the device-resident network
+  pack_game_requests(P, g, match_requests(ctl, sides), (size_t)pack_offs[g], threadIdx.x & 31, rows, packed);
 }
 
 }  // namespace cb200

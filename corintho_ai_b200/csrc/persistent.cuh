@@ -26,22 +26,15 @@ __host__ __device__ constexpr size_t ps_tree_smem_off() {
 }
 template <int kMode, int kGames>
 __host__ __device__ constexpr size_t ps_smem_bytes() {
-  return ps_tree_smem_off<kMode, kGames>() + kGames * sizeof(WarpSm);
+  constexpr size_t bytes = ps_tree_smem_off<kMode, kGames>() + kGames * sizeof(WarpSm);
+  static_assert(bytes <= 227 * 1024, "bf16x3 fits with 8 games per CTA only");
+  return bytes;
 }
-
-// live games in ascending index order: one warp, 32 flags per trip, ballot-ordered append
-__global__ void k_live_list(TreeParams P, int32_t *__restrict__ list, int32_t *__restrict__ count) {
-  if (blockIdx.x != 0 || threadIdx.x >= 32) return;
-  const int lane = threadIdx.x;
-  int n = 0;
-  for (int g0 = 0; g0 < P.num_games; g0 += 32) {
-    const int g = g0 + lane;
-    const bool live = g < P.num_games && !P.ctl[(size_t)g * kCtlWords + CW_DONE];
-    const unsigned m = __ballot_sync(0xffffffffu, live);
-    if (live) list[n + __popc(m & ((1u << lane) - 1u))] = g;
-    n += __popc(m);
-  }
-  if (lane == 0) *count = n;
+// threads of a persistent CTA that run the network: one tile for 8 games, two for 16
+template <int kGames>
+__host__ __device__ constexpr int ps_net_threads() {
+  static_assert(kGames == 8 || kGames == 16, "one or two network tiles per CTA");
+  return kGames == 8 ? 128 : kTcThreads;
 }
 
 // kGames = 8 (one network tile) or 16 (two tiles) games per CTA, one warp each (256 / 512
@@ -58,10 +51,7 @@ __global__ void __launch_bounds__(kGames * 32, 1)
                           int n_list, const float *eval0, const float *probs0, long pcs0,
                           float *eval, float *probs, int ld, ulonglong2 *packed, int max_rounds,
                           int exit_done, int iteration0, int32_t *out) {
-  static_assert(kGames == 8 || kGames == 16, "one or two network tiles per CTA");
-  static_assert(ps_smem_bytes<kMode, kGames>() <= 227 * 1024, "bf16x3 fits with 8 games per CTA only");
-  constexpr int kNetThreads = kGames == 8 ? 128 : kTcThreads;  // one tile or two
-  static_assert(kGames * 32 >= kNetThreads, "too few threads for the network");
+  constexpr int kNetThreads = ps_net_threads<kGames>();
   const bool net_thread = threadIdx.x < kNetThreads;
   constexpr int kRows = kGames * kPsRowsPerGame;
   extern __shared__ __align__(128) uint8_t smem[];

@@ -1390,6 +1390,36 @@ __device__ __forceinline__ bool game_selected(const int32_t *ctl, int to_play) {
   return ctl[CW_TO_PLAY] == ((to_play + ctl[CW_PARITY]) & 1);
 }
 
+// ---- the per-game frame of every driver (run_game, k_match_iterate, analysis_step) ------------
+// Game g's Ctx from its control block ctl: the control words, no work done yet, the game's storage.
+// Self-play games keep their parity, mate turn and samples; matches and analyses search in testing
+// mode from parity 0 and keep no samples.
+__device__ __forceinline__ void ctx_open(Ctx &c, const TreeParams &P, int g, const int32_t *ctl,
+                                         bool self_play) {
+  c.to_play = ctl[CW_TO_PLAY], c.parity = self_play ? ctl[CW_PARITY] : 0, c.result = ctl[CW_RESULT];
+  c.mate_turn = self_play ? ctl[CW_MATE_TURN] : 0, c.n_samples = self_play ? ctl[CW_N_SAMPLES] : 0;
+  c.n_pending = ctl[CW_N_PENDING], c.error = ctl[CW_ERROR], c.spare = ctl[CW_SPARE];
+  c.mt_idx = ctl[CW_MT_IDX];
+  c.d_sims = 0, c.d_evals = 0, c.d_moves = 0, c.d_searches = 0;
+  CB_PROF(c.t_ingest = c.t_search = c.t_move = c.n_none = c.n_copy = 0;
+          c.t_sel = c.t_exp = c.n_lvl = c.n_exp = c.n_exact = 0;)
+  c.work = 0, c.yielded = 0;
+  c.arenas = P.arenas + (size_t)g * 3 * P.arena_words;
+  c.mt = P.mt + (size_t)g * 624;
+  c.pending = P.pending + (size_t)g * P.spe * kPendWords;  // P.spe = the largest budget (stride)
+  c.tree_ctl = P.tree + (size_t)g * 2 * kTreeCtlWords;
+  c.leaf_state = P.leaf_state + (size_t)g * P.spe;
+  c.sample_state = self_play ? P.sample_state + (size_t)g * kMaxSamples : nullptr;
+  c.sample_probs = self_play ? P.sample_probs + (size_t)g * kMaxSamples * CB200_NUM_MOVES : nullptr;
+}
+// The control words back (lane 0); CW_DONE and the counters are the caller's.
+__device__ __forceinline__ void ctx_close(const Ctx &c, int32_t *ctl, bool self_play) {
+  ctl[CW_TO_PLAY] = c.to_play, ctl[CW_RESULT] = c.result;
+  if (self_play) ctl[CW_MATE_TURN] = c.mate_turn, ctl[CW_N_SAMPLES] = c.n_samples;
+  ctl[CW_N_PENDING] = c.n_pending, ctl[CW_ERROR] = c.error;
+  ctl[CW_SPARE] = c.spare, ctl[CW_MT_IDX] = c.mt_idx;
+}
+
 // One SelfPlayer::doIteration for game g, executed by one warp. offs[g] = index of
 // game g's first answer row in eval/probs (exclusive prefix sum of the request counts the answers
 // were produced for). kFused: answers are read at the row the game was handed last time
@@ -1413,22 +1443,8 @@ __device__ __forceinline__ void run_game(const TreeParams &P, int g, WarpSm &sm,
     if (kFused && c.lane == 0) atomicAdd(live_ctr, 1);
     return;  // not started yet, but alive
   }
-  c.to_play = ctl[CW_TO_PLAY], c.parity = ctl[CW_PARITY], c.result = ctl[CW_RESULT];
-  c.mate_turn = ctl[CW_MATE_TURN], c.n_samples = ctl[CW_N_SAMPLES];
-  c.n_pending = ctl[CW_N_PENDING], c.error = ctl[CW_ERROR], c.spare = ctl[CW_SPARE];
-  c.mt_idx = ctl[CW_MT_IDX];
-  c.d_sims = 0, c.d_evals = 0, c.d_moves = 0, c.d_searches = 0;
-  CB_PROF(c.t_ingest = c.t_search = c.t_move = c.n_none = c.n_copy = 0;
-          c.t_sel = c.t_exp = c.n_lvl = c.n_exp = c.n_exact = 0;)
-  c.work = 0, c.yielded = 0;
+  ctx_open(c, P, g, ctl, true);
   bool resume = kFused && ctl[CW_YIELD] != 0;
-  c.arenas = P.arenas + (size_t)g * 3 * P.arena_words;
-  c.mt = P.mt + (size_t)g * 624;
-  c.pending = P.pending + (size_t)g * P.spe * kPendWords;
-  c.tree_ctl = P.tree + (size_t)g * 2 * kTreeCtlWords;
-  c.leaf_state = P.leaf_state + (size_t)g * P.spe;
-  c.sample_state = P.sample_state + (size_t)g * kMaxSamples;
-  c.sample_probs = P.sample_probs + (size_t)g * kMaxSamples * CB200_NUM_MOVES;
   const int off = kFused ? ctl[CW_REQ_BASE] : offs[g];
   if (kFused && c.n_pending > 0 && !resume) {
     // This launch will ingest evaluations: request everything whose address is already known
@@ -1478,9 +1494,7 @@ __device__ __forceinline__ void run_game(const TreeParams &P, int g, WarpSm &sm,
     if (c.lane == 0) ctl[CW_YIELD] = c.yielded;
   }
   if (c.lane == 0) {
-    ctl[CW_TO_PLAY] = c.to_play, ctl[CW_RESULT] = c.result, ctl[CW_MATE_TURN] = c.mate_turn;
-    ctl[CW_N_SAMPLES] = c.n_samples, ctl[CW_N_PENDING] = c.n_pending, ctl[CW_ERROR] = c.error;
-    ctl[CW_SPARE] = c.spare, ctl[CW_MT_IDX] = c.mt_idx;
+    ctx_close(c, ctl, true);
     if (done) {
       // a finished game's samples may be picked up by the streaming emit kernel on another
       // stream: everything the game wrote must be visible before the flag is
@@ -1595,19 +1609,12 @@ __global__ void __launch_bounds__(1024)
   if (t == 0) summary[1] = s_live, summary[2] = s_err;
 }
 
-// Trainer::writeRequests (trainer.cpp:79-101): expand the queued leaf states of the selected
-// games to 70-float rows, game-index-major; also emits the packed cstates for the fused net.
-__global__ void __launch_bounds__(256)
-    k_pack_requests(TreeParams P, int to_play, const int32_t *__restrict__ offs,
-                    float *__restrict__ rows, ulonglong2 *__restrict__ packed) {
-  const int g = blockIdx.x * 8 + (threadIdx.x >> 5);
-  const int lane = threadIdx.x & 31;
-  if (g >= P.num_games) return;
-  const int32_t *ctl = P.ctl + (size_t)g * kCtlWords;
-  if (!game_selected(ctl, to_play)) return;
-  const int np = ctl[CW_N_PENDING];
+// The first np queued leaf states of game g as request rows off, off + 1, ... (one warp): the
+// packed cstates for a device-resident network (packed != null) and the 70-float rows
+// (rows != null).
+__device__ __forceinline__ void pack_game_requests(const TreeParams &P, int g, int np, size_t off, int lane,
+                                                   float *__restrict__ rows, ulonglong2 *__restrict__ packed) {
   const ulonglong2 *ls = P.leaf_state + (size_t)g * P.spe;
-  const size_t off = (size_t)offs[g];
   if (packed)
     for (int k = lane; k < np; k += 32) packed[off + k] = ls[k];
   if (rows) {
@@ -1618,6 +1625,18 @@ __global__ void __launch_bounds__(256)
       out[f] = encode_elem(CState{v.x, v.y}, j);
     }
   }
+}
+
+// Trainer::writeRequests (trainer.cpp:79-101): expand the queued leaf states of the selected
+// games to 70-float rows, game-index-major; also emits the packed cstates for the fused net.
+__global__ void __launch_bounds__(256)
+    k_pack_requests(TreeParams P, int to_play, const int32_t *__restrict__ offs,
+                    float *__restrict__ rows, ulonglong2 *__restrict__ packed) {
+  const int g = blockIdx.x * 8 + (threadIdx.x >> 5);
+  if (g >= P.num_games) return;
+  const int32_t *ctl = P.ctl + (size_t)g * kCtlWords;
+  if (!game_selected(ctl, to_play)) return;
+  pack_game_requests(P, g, ctl[CW_N_PENDING], (size_t)offs[g], threadIdx.x & 31, rows, packed);
 }
 
 }  // namespace cb200

@@ -8,7 +8,7 @@ import pytest
 
 import corintho_ai_b200 as cb
 from diag import first_divergence
-from oracle.pyoracle import ADVERSARIAL_EVALUATORS, synth_eval
+from oracle.pyoracle import ADVERSARIAL_EVALUATORS, play_out, synth_eval
 from test_oracle_trainer import check_against_golden
 from util import TRAINER_GRID, grid_key, run_trainer
 
@@ -81,23 +81,27 @@ def test_engine_matches_oracle_with_degenerate_evaluators(oracle, cfg, evaluator
 
 def test_sharded_trainers_equal_single_trainer():
     """Multi-GPU partitioning rule (SURVEY.md 8e): shards of one seed stream reproduce the
-    single-trainer run game by game."""
-    cfg = (12, 31, 32, 8, 1.0, 0.25, False)
-    whole = make_engine(cfg)
-    run_trainer(whole, synth_eval)
-    st_w, pr_w, lb_w, go_w = whole.raw_samples()
-    parts = []
-    for first, cnt in ((0, 5), (5, 7)):
-        t = cb.Trainer(cnt, "", 31, 32, 8, 1.0, 0.25, 0, 1, False, total_games=12, first_game=first)
-        # shards of a staggered run start later; drive them with the same loop
-        run_trainer(t, synth_eval, allow_empty=True)
-        st, pr, lb, go = t.raw_samples()
-        parts.append((st, pr, lb, go + first))
-    st = np.concatenate([p[0] for p in parts])
-    assert st.tobytes() == st_w.tobytes()
-    assert np.concatenate([p[1] for p in parts]).tobytes() == pr_w.tobytes()
-    assert np.concatenate([p[2] for p in parts]).tobytes() == lb_w.tobytes()
-    assert (np.concatenate([p[3] for p in parts]) == go_w).all()
+    single-trainer run game by game. In the 1 300-game run the second shard starts before output
+    624 of the seed stream and ends after output 1 248, so its seeds come from three MT19937
+    blocks, the first of them entered part-way."""
+    for (games, seed, max_searches, spe), shards in (((12, 31, 32, 8), ((0, 5), (5, 7))),
+                                                     ((1300, 17, 4, 4), ((0, 600), (600, 700)))):
+        whole = make_engine((games, seed, max_searches, spe, 1.0, 0.25, False))
+        play_out(whole, synth_eval)
+        st_w, pr_w, lb_w, go_w = whole.raw_samples()
+        parts = []
+        for first, cnt in shards:
+            t = cb.Trainer(cnt, "", seed, max_searches, spe, 1.0, 0.25, 0, 1, False, total_games=games,
+                           first_game=first)
+            # shards of a staggered run start later; drive them with the same loop
+            play_out(t, synth_eval, allow_empty=True)
+            st, pr, lb, go = t.raw_samples()
+            parts.append((st, pr, lb, go + first))
+        st = np.concatenate([p[0] for p in parts])
+        assert st.tobytes() == st_w.tobytes()
+        assert np.concatenate([p[1] for p in parts]).tobytes() == pr_w.tobytes()
+        assert np.concatenate([p[2] for p in parts]).tobytes() == lb_w.tobytes()
+        assert (np.concatenate([p[3] for p in parts]) == go_w).all()
 
 
 def test_write_scores_and_errors(tmp_path):
